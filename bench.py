@@ -3,6 +3,7 @@
 CPU-baseline evidence.  Contract: see DESIGN.md "Measurement".
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg5|cfg4]
+                    [--dump-outputs DIR]
 
 A "step" is one `update_embedding` (forward_fm + BCEWithLogits + sparse backward + fresh-Adam row
 update, the reference's pre-training hot loop main_experiment.py:92-105) over one batch of 8192
@@ -128,13 +129,13 @@ def cpu_port_rate(sizes, k, B, budget_s, seed=0, threads=None):
 
 
 def reference_classes_rate(B=8192, steps=5, threads=None):
-    """The reference's OWN classes (baseline/_ref, copied there unmodified by __graft_entry__.build()) on this box's host
+    """The reference's OWN classes (oracle/_ref, copied there unmodified by __graft_entry__.build()) on this box's host
     cores: DeepFMAdam(use_cuda=False).update_embedding at BASELINE.json configs[3]'s shape (the Criteo-tiny tables of
     main_experiment.py:56-58; the 33 M-row tables of configs[4] would need minutes per step: the reference's Adam step is
     dense over every row).  ndarray inputs (the reference converts them per call)."""
-    ref = os.path.join(ROOT, "baseline", "_ref")
+    ref = os.path.join(ROOT, "oracle", "_ref")
     if not os.path.isdir(os.path.join(ref, "models")):
-        return {"unavailable": "baseline/_ref not populated (run __graft_entry__.build() where /root/reference exists)"}
+        return {"unavailable": "oracle/_ref not populated (run __graft_entry__.build() where the reference checkout exists)"}
     import types
     import torch
     if "matplotlib" not in sys.modules:
@@ -250,7 +251,7 @@ def run_reference(args):
     ones = np.ones((B, len(sizes)), np.float32)
     for w in range(max(1, min(args.warmup, 2))):
         orc.update_embedding(batches[0][0], ones, batches[0][1])
-    K = min(args.steps, 40)
+    K = args.steps
     t0 = time.perf_counter()
     for i in range(K):
         Xi, Y = batches[i % len(batches)]
@@ -276,6 +277,38 @@ def workload_config(args, sizes):
             "update": "fresh-Adam sign step (reference)", "l2": "tables larger than L2; a different batch every step"}
 
 
+DUMP_BUDGET_BYTES = 64 << 20
+DUMP_UPDATED_ROWS, DUMP_SAMPLE_ROWS, DUMP_SEED = 1 << 19, 1 << 18, 20240601
+
+
+def dump_outputs(out_dir, model, batch, loss):
+    """--dump-outputs: what the last timed step computed, as DIR/<name>.npy, so that two builds can be compared output
+    for output.  The step returns its loss and updates the bias and the table rows its batch hits; the whole table is
+    too large to store (2 GB at cfg5), so the trained columns (V, then w1) are written for the rows that step updated
+    (ascending row id, a seeded subset above DUMP_UPDATED_ROWS) and for a fixed, seeded sample of all rows.  The row ids
+    are written beside them (float64, exact)."""
+    import torch
+    k = model.embedding_size
+    rng = np.random.RandomState(DUMP_SEED)
+    updated = np.unique(batch.ids.cpu().numpy())
+    if len(updated) > DUMP_UPDATED_ROWS:
+        updated = np.sort(rng.choice(updated, DUMP_UPDATED_ROWS, replace=False))
+    sample = np.unique(rng.randint(0, model._R, size=DUMP_SAMPLE_ROWS))
+
+    def rows(ids):
+        idx = torch.from_numpy(ids.astype(np.int64)).to(model.device)
+        return model._table.index_select(0, idx)[:, :k + 1].cpu().numpy()
+
+    out = {"loss": loss.reshape(1).cpu().numpy(), "bias": model.bias.detach().reshape(-1).cpu().numpy(),
+           "updated_row_ids": updated.astype(np.float64), "updated_rows": rows(updated),
+           "sample_row_ids": sample.astype(np.float64), "sample_rows": rows(sample)}
+    assert all(a.dtype in (np.float32, np.float64) for a in out.values())
+    assert sum(a.nbytes for a in out.values()) <= DUMP_BUDGET_BYTES
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -285,6 +318,8 @@ def run_ours(args):
     rank = int(os.environ.get("RANK", "0"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
     torch.cuda.set_device(local)
+    if world > 1 and args.dump_outputs:
+        raise SystemExit("--dump-outputs is supported with --gpus 1 only")
     if world > 1:
         dist.init_process_group("nccl", device_id=torch.device("cuda", local))
     sizes = feature_sizes(args.workload)
@@ -328,13 +363,15 @@ def run_ours(args):
     ev0.record(stream)
     th0 = time.perf_counter()
     for i in range(K):
-        step(base + i)
+        last_loss = step(base + i)
     host_ms = (time.perf_counter() - th0) * 1e3 / K     # time the host needs to SUBMIT one step (no sync inside)
     ev1.record(stream)
     torch.cuda.synchronize()
     ms = ev0.elapsed_time(ev1)
     assert lib.fmb_session_graph_count(sess) == graphs0, "a step graph was captured inside the timed region"
     launches = lib.fmb_session_launches(sess) - launches0
+    if args.dump_outputs:   # before the host-path measurements below train the same table further
+        dump_outputs(args.dump_outputs, model, enc[(base + K - 1) % NB], last_loss)
 
     # ---- e2e: HOST buffers through the C-ABI host entry point, every step: H2D of that step's ids/labels
     # from pinned host memory + the step + D2H of its loss.  Two input slots: the copies of step t+1
@@ -545,7 +582,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the cfg4 DeepFMAdam.fit record")
     ap.add_argument("--no-presort", action="store_true", help="sort each batch inside its own step")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed to DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs is supported with --impl ours only")
     if args.impl == "reference":
         run_reference(args)
     else:
