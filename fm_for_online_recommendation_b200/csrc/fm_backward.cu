@@ -692,7 +692,8 @@ FMB_API int fmb_fm_backward_update_rl(const int32_t* sorted_keys, const int32_t*
     FMB_CHECK_ARG(!rl || (rl->entries && rl->seg_count && rl->nseg >= 1 && rl->nseg <= 2048 && rl->seg_cap >= 1),
                   "fmb_fm_backward_update: bad run list");
     FMB_CHECK_ARG(sorted_keys && perm && table && S && gs && ws, "fmb_fm_backward_update: null pointer");
-    FMB_CHECK_ARG(N > 0 && F > 0 && F < 512 && k > 0 && k <= 124, "fmb_fm_backward_update: bad shape");
+    FMB_CHECK_ARG(N > 0 && F > 0 && F < 512 && k > 0 && k <= 124, "fmb_fm_backward_update: bad shape N=%lld F=%d k=%d (need F < 512, k <= 124)",
+                  (long long)N, F, k);
     FMB_CHECK_ARG(mode == 0 || mode == 1, "fmb_fm_backward_update: unknown update mode %d", mode);
     FMB_CHECK_ARG(use_fm2 || gvec, "fmb_fm_backward_update: neither gradient path enabled");
     FMB_CHECK_ARG(n_entries > 0 && n_entries < ((int64_t)1 << 31), "fmb_fm_backward_update: n_entries out of range");
@@ -759,7 +760,8 @@ FMB_API int fmb_fm_backward_runs_list(const int32_t* sorted_keys, int64_t N, flo
     FMB_CHECK_ARG(sorted_keys && table && ws, "fmb_fm_backward_runs: null pointer");
     FMB_CHECK_ARG(!rl || (rl->entries && rl->seg_count && rl->nseg >= 1 && rl->nseg <= 2048 && rl->seg_cap >= 1),
                   "fmb_fm_backward_runs: bad run list");
-    FMB_CHECK_ARG(N > 0 && F > 0 && F < 512 && k > 0 && k <= 124, "fmb_fm_backward_runs: bad shape");
+    FMB_CHECK_ARG(N > 0 && F > 0 && F < 512 && k > 0 && k <= 124, "fmb_fm_backward_runs: bad shape N=%lld F=%d k=%d (need F < 512, k <= 124)",
+                  (long long)N, F, k);
     FMB_CHECK_ARG(mode == 0 || mode == 1 || (mode == 2 && ftrl && ftrl->zn), "fmb_fm_backward_runs: unknown update mode %d", mode);
     if (ws_bytes < fmb_bwd_workspace_bytes(N, k)) { fmb_set_error("fmb_fm_backward_runs: workspace too small"); return FMB_ERR_WS; }
     BwdParams p;

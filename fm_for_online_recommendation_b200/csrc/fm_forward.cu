@@ -141,7 +141,7 @@ FMB_API int fmb_fm_forward(const int32_t* ids, const float* xv, const float* tab
                            int loss_kind, float* delta, float* lossv, cudaStream_t stream) {
     FMB_CHECK_ARG(ids && table && bias, "fmb_fm_forward: null ids/table/bias");
     FMB_CHECK_ARG(B > 0 && F > 0 && k > 0, "fmb_fm_forward: bad shape B=%d F=%d k=%d", B, F, k);
-    FMB_CHECK_ARG(F < 512 && k <= 252, "fmb_fm_forward: need F < 512 and k <= 252");
+    FMB_CHECK_ARG(F < 512 && k <= 252, "fmb_fm_forward: bad shape F=%d k=%d (need F < 512, k <= 252)", F, k);
     FMB_CHECK_ARG(!y || (delta && lossv), "fmb_fm_forward: y given without delta/lossv");
     FwdParams p;
     p.ids = ids; p.xv = xv; p.table = table; p.bias = bias;
@@ -156,7 +156,7 @@ FMB_API int fmb_fm_forward(const int32_t* ids, const float* xv, const float* tab
         return sizeof(float) * ((size_t)sb * F * p.cu * 4 + (size_t)2 * sb * F + (size_t)sb * k);
     };
     while (SB > 1 && bytes(SB) > 48 * 1024) SB >>= 1;
-    FMB_CHECK_ARG(bytes(SB) <= 200 * 1024, "fmb_fm_forward: F*k too large for one sample tile");
+    FMB_CHECK_ARG(bytes(SB) <= 200 * 1024, "fmb_fm_forward: F*k too large for one sample tile (F=%d k=%d)", F, k);
     p.SB = SB;
     static bool attr_set = false;
     if (!attr_set) {

@@ -41,7 +41,7 @@ struct StepParams {
     int cu;                    // 16-byte chunks of a row that hold data: ceil((k+1)/4)
     int ql_log;                // log2 of lanes per (sample, field) in the gather phase (pow2 >= cu)
     int jl_log;                // log2 of lanes per sample in the reduce phase (pow2 >= kp4)
-    uint32_t mF, mcu;          // ceil(2^32 / F), ceil(2^32 / cu): x / F == __umulhi(x, mF) for x < 2^16 * ... (see magic_div)
+    uint32_t mF, mcu;          // fmb_div_magic(F), fmb_div_magic(cu): x / F == fmb_div_by_magic(x, mF) (x < SB*F*cu)
     int loss_kind, mode;
     float lr, astep;
     float* delta;              // [B] out
@@ -187,9 +187,9 @@ __global__ void __launch_bounds__(256, MODE == 2 ? 4 : 8) fm_step_fused_kernel(c
     // precomputed reciprocals (a runtime integer division is ~20 instructions, and there were two per item).
     const int ns = n_single, nm = n_multi;
     for (int it = threadIdx.x; it < ((p.dbg & 1) ? 0 : ns * cu); it += blockDim.x) {
-        const int li = (int)__umulhi((unsigned)it, p.mcu), q = it - li * cu;
+        const int li = fmb_div_by_magic((unsigned)it, p.mcu), q = it - li * cu;
         const int ef = single_s[li];
-        const int s = (int)__umulhi((unsigned)ef, p.mF);
+        const int s = fmb_div_by_magic((unsigned)ef, p.mF);
         const float x = XV ? x_s[ef] : 1.0f, d = d_s[s];
         const float4 S4 = *reinterpret_cast<const float4*>(S_s + s * rp + q * 4);
         const float4 v4 = *reinterpret_cast<const float4*>(rows_s + (size_t)ef * rp + q * 4);
@@ -280,9 +280,9 @@ __global__ void __launch_bounds__(256, MODE == 2 ? 4 : 8) fm_step_fused_kernel(c
     FMB_TS(5);
     // phase 4b: rows hit several times: stage the entry's contribution at its sorted position (run kernel sums them)
     for (int it = threadIdx.x; it < ((p.dbg & 2) ? 0 : nm * cu); it += blockDim.x) {
-        const int li = (int)__umulhi((unsigned)it, p.mcu), q = it - li * cu;
+        const int li = fmb_div_by_magic((unsigned)it, p.mcu), q = it - li * cu;
         const int ef = multi_s[li];
-        const int s = (int)__umulhi((unsigned)ef, p.mF);
+        const int s = fmb_div_by_magic((unsigned)ef, p.mF);
         const float x = XV ? x_s[ef] : 1.0f, d = d_s[s];
         const float4 S4 = *reinterpret_cast<const float4*>(S_s + s * rp + q * 4);
         const float4 v4 = *reinterpret_cast<const float4*>(rows_s + (size_t)ef * rp + q * 4);
@@ -423,7 +423,7 @@ FMB_API int fmb_fm_step_fused_ex(const int32_t* ids, const float* xv, const floa
     p.table = table; p.bias = bias;
     p.B = B; p.F = F; p.k = k; p.rowp = fmb_round_up(k + 1, 16); p.kp4 = fmb_round_up(k, 4);
     p.cu = (k + 1 + 3) / 4; p.ql_log = ilog2_ceil(p.cu); p.jl_log = ilog2_ceil(p.kp4);
-    p.mF = (uint32_t)(0x100000000ull / (unsigned)F) + 1u; p.mcu = (uint32_t)(0x100000000ull / (unsigned)p.cu) + 1u;
+    p.mF = fmb_div_magic((unsigned)F); p.mcu = fmb_div_magic((unsigned)p.cu);
     p.loss_kind = loss_kind; p.mode = mode; p.lr = lr; p.astep = -(lr / 0.1f);
     p.delta = delta; p.lossv = lossv;
     p.G = (float*)ws; p.Npad = (N + 3) / 4 * 4 + 64;
@@ -450,7 +450,8 @@ FMB_API int fmb_fm_step_fused_ex(const int32_t* ids, const float* xv, const floa
         if (cap < 0) { const char* e = getenv("FMB_STEP_SB"); cap = e ? atoi(e) : 0; }
         if (cap > 0 && SB > cap) SB = cap;
     }
-    FMB_CHECK_ARG(bytes(SB) <= 200 * 1024, "fmb_fm_step_fused: F*k too large for one sample tile");
+    FMB_CHECK_ARG(bytes(SB) <= 200 * 1024, "fmb_fm_step_fused: F*k too large for one sample tile (F=%d k=%d: %zu bytes > 200 KB)",
+                  F, k, bytes(SB));
     p.SB = SB;
     const fused_fn_t fn = fused_fn(p.cu, xv != nullptr, mode);
     if (bytes(SB) > 48 * 1024) cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);

@@ -29,6 +29,12 @@ void fmb_set_error(const char* fmt, ...);
 
 static inline int fmb_round_up(int x, int m) { return (x + m - 1) / m * m; }
 
+// x / d by multiplication, for d >= 1 and x * d < 2^31: __umulhi(2x, floor(2^31 / d) + 1).  The error term of the
+// multiplier, x * (d - 2^31 mod d) / (d * 2^31), stays below 1/d.  (The 2^32 form, multiplier ceil(2^32 / d), has no
+// 32-bit multiplier for d = 1.)
+static inline uint32_t fmb_div_magic(unsigned d) { return 0x80000000u / d + 1u; }
+__device__ __forceinline__ int fmb_div_by_magic(unsigned x, uint32_t m) { return (int)__umulhi(x << 1, m); }
+
 namespace fmb {
 
 // ---------------------------------------------------------------------------------------------

@@ -255,7 +255,8 @@ FMB_API int fmb_online_deep_run(int kind, const int32_t* ids, const float* xv, c
                                 cudaStream_t stream) {
     FMB_CHECK_ARG(kind >= 0 && kind <= 4, "fmb_online_deep_run: unknown model kind %d", kind);
     FMB_CHECK_ARG(ids && y && table && bias && preds && conf, "fmb_online_deep_run: null pointer");
-    FMB_CHECK_ARG(N > 0 && F > 0 && F < 512 && k > 0 && k <= 124, "fmb_online_deep_run: bad shape");
+    FMB_CHECK_ARG(N > 0 && F > 0 && F < 512 && k > 0 && k <= 124, "fmb_online_deep_run: bad shape N=%d F=%d k=%d (need F < 512, k <= 124)",
+                  N, F, k);
     FMB_CHECK_ARG(kind == 0 || (mlp && L > 0 && H > 0 && H < 512), "fmb_online_deep_run: tower needs mlp, 0 < H < 512");
     FMB_CHECK_ARG(kind < 3 || (alpha && acc), "fmb_online_deep_run: ONN needs alpha and acc");
     OnlineParams p;
@@ -266,7 +267,8 @@ FMB_API int fmb_online_deep_run(int kind, const int32_t* ids, const float* xv, c
     const int mx = p.H > k ? p.H : k;
     const size_t fl = (size_t)F * p.cu * 4 + 2 * F + 2 * k + (size_t)p.L * p.H + 2 * mx + k + 2 * (p.L > 0 ? p.L : 1) + 16;
     const size_t smb = fl * sizeof(float);
-    FMB_CHECK_ARG(smb <= 200 * 1024, "fmb_online_deep_run: model too large for one CTA's shared memory");
+    FMB_CHECK_ARG(smb <= 200 * 1024, "fmb_online_deep_run: model too large for one CTA's shared memory (F=%d k=%d L=%d H=%d: %zu bytes > 200 KB)",
+                  F, k, p.L, p.H, smb);
     cudaFuncSetAttribute(online_deep_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
     online_deep_kernel<<<1, OT, smb, stream>>>(p);
     FMB_CHECK_LAUNCH("online_deep_kernel");

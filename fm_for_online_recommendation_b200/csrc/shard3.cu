@@ -107,7 +107,7 @@ __global__ void __launch_bounds__(256, 7) shard_step_fused_kernel(Step3Params p)
         const int i = it * 32 + lane;
         bool own = false;
         if (i < npairs) {
-            const int s = (int)__umulhi((unsigned)i, p.mF), f = i - s * F;
+            const int s = fmb_div_by_magic((unsigned)i, p.mF), f = i - s * F;
             own = (sid[f * (SB + 1) + s] & (p.G - 1)) == p.me;
         }
         const unsigned bal = __ballot_sync(0xffffffffu, own);
@@ -138,7 +138,7 @@ __global__ void __launch_bounds__(256, 7) shard_step_fused_kernel(Step3Params p)
         int s = 0, f = 0;
         int32_t gid = 0;
         if (i < npairs) {
-            s = (int)__umulhi((unsigned)i, p.mF); f = i - s * F;
+            s = fmb_div_by_magic((unsigned)i, p.mF); f = i - s * F;
             gid = sid[f * (SB + 1) + s];
             own = (gid & (p.G - 1)) == p.me;
         }
@@ -377,7 +377,7 @@ FMB_API int fmb_shard3_step(const int32_t* idsT_all, float* table_local, const f
         const int need = (F * (p.SB + 1) + p.cu * 4 - 1) / (p.cu * 4);   // the tile's ids must fit where the rows go
         if (p.cap_e < need) p.cap_e = (need + 15) / 16 * 16;
     }
-    p.mF = (uint32_t)(0x100000000ull / (unsigned)F) + 1u; p.mcu = (uint32_t)(0x100000000ull / (unsigned)p.cu) + 1u;
+    p.mF = fmb_div_magic((unsigned)F); p.mcu = fmb_div_magic((unsigned)p.cu);
     p.loss_kind = loss_kind; p.mode = mode; p.lr = lr; p.astep = -(lr / 0.1f);
     p.Gst = (float*)ws; p.Npad = npad3(N);
     for (int r = 0; r < 8; ++r) {
