@@ -46,6 +46,7 @@ _SIGS = {
     "fmb_math_eval": (C.c_int, [C.c_int, vp, vp, C.c_int64, vp]),
     "fmb_update_dense": (C.c_int, [vp, vp, C.c_int64, C.c_float, C.c_int, vp]),
     "fmb_finish_step": (C.c_int, [vp, vp, C.c_int, vp, C.c_float, C.c_int, vp, vp]),
+    "fmb_update_dense_ex": (C.c_int, [vp, vp, C.c_int64, C.c_float, C.c_int, vp, C.c_float, vp]),
     "fmb_sort_workspace_bytes": (C.c_size_t, [C.c_int64]),
     "fmb_sort_segment": (C.c_int, [vp, C.c_int64, C.c_int, vp, C.c_size_t, vp, vp, vp, vp, vp]),
     "fmb_bwd_workspace_bytes": (C.c_size_t, [C.c_int64, C.c_int]),
@@ -80,6 +81,9 @@ _SIGS = {
                                             C.c_int, C.c_int, vp, C.c_int32, C.c_float, C.c_int, vp, C.c_size_t, vp]),
     "fmb_fm_backward_update_rl": (C.c_int, [vp, vp, C.c_int64, C.c_int64, vp, vp, C.c_int, C.c_int, vp, C.c_int, vp,
                                             C.c_int, C.c_int, vp, C.c_int32, C.c_float, C.c_int, vp, vp, C.c_size_t, vp]),
+    "fmb_fm_backward_update_rl_ex": (C.c_int, [vp, vp, C.c_int64, C.c_int64, vp, vp, C.c_int, C.c_int, vp, C.c_int, vp,
+                                               C.c_int, C.c_int, vp, C.c_int32, C.c_float, C.c_int, vp, vp, vp, C.c_size_t,
+                                               vp]),
     "fmb_shard_pw": (C.c_int, [C.c_int]),
     "fmb_shard_cw": (C.c_int, [C.c_int]),
     "fmb_shard_sort_max_cap": (C.c_int, []),
@@ -111,6 +115,8 @@ _SIGS = {
     "fmb_shard_signal": (C.c_int, [vp, vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, vp, vp]),
     "fmb_online_deep_run": (C.c_int, [C.c_int, vp, vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, vp, vp, vp, vp,
                                       vp, C.c_float, C.c_float, C.c_float, C.c_int, vp, vp, vp]),
+    "fmb_online_deep_run_ex": (C.c_int, [C.c_int, vp, vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, vp, vp, vp,
+                                         vp, vp, C.c_float, C.c_float, C.c_float, C.c_int, vp, vp, vp, vp]),
     "fmb_session_create": (C.c_int, [C.POINTER(vp), C.c_int, C.c_int, C.c_int64, vp]),
     "fmb_sort_fields_max_batch": (C.c_int, []),
     "fmb_sort_fields": (C.c_int, [vp, C.c_int, C.c_int, vp, vp, vp, vp]),
@@ -126,6 +132,7 @@ _SIGS = {
     "fmb_session_presort": (C.c_int, [vp, vp, C.c_int, C.c_int]),
     "fmb_session_presort_invalidate": (None, [vp]),
     "fmb_session_set_ftrl": (C.c_int, [vp, vp, vp, C.c_float, C.c_float, C.c_float]),
+    "fmb_session_set_adagrad": (C.c_int, [vp, vp, vp, C.c_float]),
     "fmb_fm_step_fused_ex": (C.c_int, [vp, vp, vp, vp, vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_float, C.c_int, vp,
                                        vp, vp, vp, C.c_size_t, vp]),
     "fmb_fm_backward_runs_ex": (C.c_int, [vp, C.c_int64, vp, C.c_int, C.c_int, C.c_float, C.c_int, vp, vp, C.c_size_t,
@@ -152,6 +159,11 @@ _lib = None
 class RunList(C.Structure):
     """fmb_runlist_t (include/fmb200.h): the runs of >= 2 equal sorted keys, one segment per producer CTA."""
     _fields_ = [("entries", C.c_void_p), ("seg_count", C.c_void_p), ("nseg", C.c_int), ("seg_cap", C.c_int)]
+
+
+class AdagradState(C.Structure):
+    """fmb_adagrad_t (include/fmb200.h): update mode 3's sums of the table, the bias and the tower, and eps."""
+    _fields_ = [("sums", C.c_void_p), ("bias_sum", C.c_void_p), ("mlp_sums", C.c_void_p), ("eps", C.c_float)]
 
 
 def load():

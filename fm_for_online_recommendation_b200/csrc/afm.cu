@@ -232,6 +232,7 @@ FMB_API int fmb_afm_step(const int32_t* ids, const float* xv, const float* y, co
 FMB_API int fmb_afm_dense_update(const float* dense_g, int B, int k, int A, float* W, float* c, float* H, float* P, float lr,
                                  int mode, float* grads_out, cudaStream_t stream) {
     FMB_CHECK_ARG(dense_g && W && c && H && P && B > 0, "fmb_afm_dense_update: bad arguments");
+    FMB_CHECK_ARG(mode != 3, "fmb_afm_dense_update: update mode 3 (Adagrad) is not supported by AFM");
     const int PD = A * k + 2 * A + k;
     afm_dense_update_kernel<<<PD, 32, 0, stream>>>(dense_g, B, PD, W, c, H, P, A, k, lr, mode, grads_out);
     FMB_CHECK_LAUNCH("afm_dense_update_kernel");

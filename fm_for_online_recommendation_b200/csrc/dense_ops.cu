@@ -43,6 +43,17 @@ __global__ void update_dense_kernel(float* __restrict__ p, const float* __restri
     if (i < n) p[i] = fmb::apply_update(p[i], g[i], lr, mode);
 }
 
+// update mode 3 (Adagrad) of dense parameters: sums [n] next to the parameters
+__global__ void update_dense_adagrad_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ sums,
+                                            int64_t n, float lr, float eps) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) {
+        float s = sums[i];
+        p[i] = fmb::adagrad_update(p[i], g[i], s, lr, eps);
+        sums[i] = s;
+    }
+}
+
 // ATen-order sum of x[0:n], parallel where the order allows it.  ATen's cascade (SumKernel.cpp multi_row_sum)
 // adds rows of 32 floats (4 ilp x 8 lanes) in blocks of `level_step` rows: a block's sum is
 // ((0 + r0) + r1) + ... and depends on nothing else, only the way block sums are folded upwards is serial.
@@ -111,7 +122,7 @@ __global__ void __launch_bounds__(FIN_THREADS) finish_step_kernel(const float* _
                                                                   const float* __restrict__ lossv, int B, float* bias,
                                                                   float lr, int mode, float* loss_out,
                                                                   float* scratch /*[2][nblocks*32] or NULL*/,
-                                                                  fmb::FtrlState ftrl) {
+                                                                  fmb::UpdateState st) {
     extern __shared__ __align__(16) float fin_sm[];
     const int half = (threadIdx.x >> 5) >= 16 ? 1 : 0;
     const float* src = half == 0 ? (bias ? delta : nullptr) : ((loss_out && lossv) ? lossv : nullptr);
@@ -130,9 +141,14 @@ __global__ void __launch_bounds__(FIN_THREADS) finish_step_kernel(const float* _
     if (lane == 0) {
         if (half == 0) {
             if (mode == 2) {
+                const fmb::FtrlState& ftrl = st.ftrl;
                 float z = ftrl.bias_zn[0], n = ftrl.bias_zn[1];
                 bias[0] = fmb::ftrl_update(bias[0], total, z, n, lr, ftrl.beta, ftrl.l1, ftrl.l2);
                 ftrl.bias_zn[0] = z; ftrl.bias_zn[1] = n;
+            } else if (mode == 3) {
+                float s = st.ada.bias_sum[0];
+                bias[0] = fmb::adagrad_update(bias[0], total, s, lr, st.ada.eps);
+                st.ada.bias_sum[0] = s;
             } else {
                 bias[0] = fmb::apply_update(bias[0], total, lr, mode);
             }
@@ -180,10 +196,21 @@ FMB_API int fmb_update_dense(float* p, const float* g, int64_t n, float lr, int 
     return FMB_OK;
 }
 
+// _ex: update mode 3 (Adagrad) with the parameters' sums [n] (read and written; NULL in the other modes)
+FMB_API int fmb_update_dense_ex(float* p, const float* g, int64_t n, float lr, int mode, float* sums, float eps,
+                                cudaStream_t stream) {
+    if (mode != 3) return fmb_update_dense(p, g, n, lr, mode, stream);
+    FMB_CHECK_ARG(p && g && n > 0 && sums, "fmb_update_dense: bad arguments (mode 3 needs the Adagrad sums)");
+    update_dense_adagrad_kernel<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(p, g, sums, n, lr, eps);
+    FMB_CHECK_LAUNCH("update_dense_adagrad_kernel");
+    return FMB_OK;
+}
+
 // end of a training step: bias update from sum(delta) (bias nullable) and mean loss (loss_out nullable).
 // B <= 1 M samples (block sums are staged in shared memory up to 256 K samples, in `fmb_finish_scratch` above).
 static float* g_fin_scratch = nullptr;
 struct fmb_ftrl_t { float* zn; float* bias_zn; float beta, l1, l2; };   // include/fmb200.h
+struct fmb_adagrad_t { float* sums; float* bias_sum; float* mlp_sums; float eps; };   // include/fmb200.h (mode 3's state)
 
 FMB_API int fmb_finish_step_ex(const float* delta, const float* lossv, int B, float* bias, float lr, int mode,
                                const fmb_ftrl_t* ftrl, float* loss_out, cudaStream_t stream) {
@@ -204,10 +231,15 @@ FMB_API int fmb_finish_step_ex(const float* delta, const float* lossv, int B, fl
     }
     static bool attr = false;
     if (!attr) { cudaFuncSetAttribute(finish_step_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 132 * 1024); attr = true; }
-    fmb::FtrlState fs = {nullptr, nullptr, 0.f, 0.f, 0.f};
+    fmb::UpdateState fs;
+    fs.ftrl = {nullptr, nullptr, 0.f, 0.f, 0.f};
     if (mode == 2) {
         FMB_CHECK_ARG(ftrl && ftrl->bias_zn, "fmb_finish_step: update mode 2 needs the FTRL state");
-        fs.zn = ftrl->zn; fs.bias_zn = ftrl->bias_zn; fs.beta = ftrl->beta; fs.l1 = ftrl->l1; fs.l2 = ftrl->l2;
+        fs.ftrl.zn = ftrl->zn; fs.ftrl.bias_zn = ftrl->bias_zn; fs.ftrl.beta = ftrl->beta; fs.ftrl.l1 = ftrl->l1; fs.ftrl.l2 = ftrl->l2;
+    } else if (mode == 3) {   // the state slot carries an fmb_adagrad_t in mode 3 (include/fmb200.h)
+        const fmb_adagrad_t* a = reinterpret_cast<const fmb_adagrad_t*>(ftrl);
+        FMB_CHECK_ARG(bias == nullptr || (a && a->bias_sum), "fmb_finish_step: update mode 3 needs the Adagrad state");
+        if (a) { fs.ada.sums = a->sums; fs.ada.bias_sum = a->bias_sum; fs.ada.eps = a->eps; }
     }
     finish_step_kernel<<<1, FIN_THREADS, smem, stream>>>(delta, lossv, B, bias, lr, mode, loss_out, scratch, fs);
     FMB_CHECK_LAUNCH("finish_step_kernel");

@@ -56,7 +56,10 @@ struct BwdParams {
     float astep;          // -(lr/0.1f): Adam step size, computed once on the host (same IEEE division)
     // multi-GPU (csrc/shard2.cu): shard_G > 0 = do not update, store the run's partial gradient into the inbox of the
     // row's owner (key % G) at slot [shard_me][position of the run's first entry]
-    fmb::FtrlState ftrl;   // mode 2 only
+    union {                // the update rule's per-coordinate state (same size as the FTRL state alone)
+        fmb::FtrlState ftrl;   // mode 2 only
+        fmb::AdagradState ada; // mode 3 only
+    };
     int min_run1;          // 1: rows hit once are summed (0 + g) and updated here too (AFM path: nothing updates them earlier)
     float* inbox[8];
     int shard_G, shard_me;
@@ -70,7 +73,22 @@ struct BwdParams {
     int pdl;                       // 1: launched as a programmatic dependent of the kernel that stages G
 };
 
+// update of coordinate c of row `key` from its summed gradient: modes 0 / 1 in registers, mode 3 (Adagrad: ADA, an
+// instantiation of its own so that the others stay as they are) also reads and writes the coordinate's sum
+template <bool ADA>
+__device__ __forceinline__ float row_update(const BwdParams& p, float old, float g, int32_t key, int c) {
+    if (ADA) {
+        float* sp = p.ada.sums + (size_t)key * p.rowp + c;
+        float sv = *sp;
+        const float o = fmb::adagrad_update(old, g, sv, p.lr, p.ada.eps);
+        *sp = sv;
+        return o;
+    }
+    return fmb::apply_update_a(old, g, p.lr, p.astep, p.mode);
+}
+
 // ---------------------------------------------------------------------------------------------
+template <bool ADA>
 __global__ void __launch_bounds__(256) fm_bwd_entry_kernel(BwdParams p) {
     const int q = threadIdx.x & ((1 << p.ql_log) - 1);
     const int64_t i = (int64_t)blockIdx.x * (256 >> p.ql_log) + (threadIdx.x >> p.ql_log);
@@ -114,9 +132,9 @@ __global__ void __launch_bounds__(256) fm_bwd_entry_kernel(BwdParams p) {
             if (j < p.k) {
                 const float gr = two ? __fadd_rn(__fadd_rn(0.f, a[t]), __fadd_rn(0.f, c[t]))
                                      : __fadd_rn(0.f, p.gvec ? c[t] : a[t]);
-                o[t] = fmb::apply_update_a(v[t], gr, p.lr, p.astep, p.mode);
+                o[t] = row_update<ADA>(p, v[t], gr, key, j);
             } else if (j == p.k) {
-                o[t] = fmb::apply_update_a(v[t], __fadd_rn(0.f, a[t]), p.lr, p.astep, p.mode);
+                o[t] = row_update<ADA>(p, v[t], __fadd_rn(0.f, a[t]), key, j);
             } else {
                 o[t] = v[t];
             }
@@ -142,7 +160,7 @@ __global__ void __launch_bounds__(256) fm_bwd_entry_kernel(BwdParams p) {
 // loads, permutation, sample index, delta, feature value) is paid once per entry instead of once per
 // 16-byte chunk, which is what made the lane-per-chunk kernel instruction-bound (75 % issue utilisation,
 // ~450 instructions per lane: profiles/r1g).  Row and S reads are random per entry either way.
-template <int CU>
+template <int CU, bool ADA>
 __global__ void __launch_bounds__(256) fm_bwd_entry1_kernel(BwdParams p) {
     const int64_t i = (int64_t)blockIdx.x * 256 + threadIdx.x;
     if (i >= p.N) return;
@@ -185,9 +203,9 @@ __global__ void __launch_bounds__(256) fm_bwd_entry1_kernel(BwdParams p) {
             // the only entry of its row: sum = 0 + contribution; update from registers
             if (j < p.k) {
                 const float gr = two ? __fadd_rn(__fadd_rn(0.f, a), __fadd_rn(0.f, c)) : __fadd_rn(0.f, p.gvec ? c : a);
-                o[j] = fmb::apply_update_a(v[j], gr, p.lr, p.astep, p.mode);
+                o[j] = row_update<ADA>(p, v[j], gr, key, j);
             } else if (j == p.k) {
-                o[j] = fmb::apply_update_a(v[j], __fadd_rn(0.f, a), p.lr, p.astep, p.mode);
+                o[j] = row_update<ADA>(p, v[j], __fadd_rn(0.f, a), key, j);
             } else {
                 o[j] = v[j];
             }
@@ -254,7 +272,7 @@ __device__ __forceinline__ void tma_g2s_2d(void* smem_dst, const CUtensorMap* tm
 // bid / nblocks: this CTA's index among the CTAs running this body, and their number (the run-list launch runs two bodies:
 // its first CTAs take the long runs, the others the short ones).  segb_off: offset (floats) of the segment-count prefix in
 // dynamic shared memory.  warps_per_block: working warps (the CTA's other warps only help with the prefix).
-template <bool LIST, int RING_SE, int RING_NS, bool LONGM>
+template <bool LIST, int RING_SE, int RING_NS, bool LONGM, bool ADA>
 __device__ __forceinline__ void runs_body(const CUtensorMap& gmap, const BwdParams& p, int warps_per_block, int warp_f, int accs_n,
                                           int ring_comps, unsigned bid, unsigned nblocks, int segb_off) {
     constexpr int RING_SEP = RING_SE + 4;
@@ -514,7 +532,12 @@ __device__ __forceinline__ void runs_body(const CUtensorMap& gmap, const BwdPara
                 }
                 float* addr = p.table + (size_t)key * p.rowp + c;
                 const float old = c < 32 ? accs[accs_n + c] : *addr;
-                if (p.mode == 2) {
+                if (ADA) {
+                    float* sp = p.ada.sums + (size_t)key * p.rowp + c;
+                    float sv = *sp;
+                    *addr = fmb::adagrad_update(old, gsum, sv, p.lr, p.ada.eps);
+                    *sp = sv;
+                } else if (p.mode == 2) {
                     float* zp = p.ftrl.zn + (size_t)key * 2 * p.rowp + c;
                     float z = zp[0], n = zp[p.rowp];
                     *addr = fmb::ftrl_update(old, gsum, z, n, p.lr, p.ftrl.beta, p.ftrl.l1, p.ftrl.l2);
@@ -537,21 +560,23 @@ __device__ __forceinline__ void runs_body(const CUtensorMap& gmap, const BwdPara
     }
 }
 
-// position-major launch (tower fit, AFM, sharded paths)
+// position-major launch (tower fit, AFM, sharded paths).  ADA: update mode 3 (Adagrad)
+template <bool ADA>
 __global__ void __launch_bounds__(256, 2) fm_bwd_runs_kernel(const __grid_constant__ CUtensorMap gmap, BwdParams p, int warps_per_block, int warp_f,
                                                              int accs_n, int ring_comps) {
-    runs_body<false, 64, 4, false>(gmap, p, warps_per_block, warp_f, accs_n, ring_comps, blockIdx.x, gridDim.x, 0);
+    runs_body<false, 64, 4, false, ADA>(gmap, p, warps_per_block, warp_f, accs_n, ring_comps, blockIdx.x, gridDim.x, 0);
 }
 
 // run-list launch: CTAs [0, nlong) take the long runs (>= 128 entries: 128-entry stages, ring from the first entry, wpl
 // working warps), the others the short runs.  The long runs are the step's longest dependent chain, so their CTAs come
 // first in the grid and are placed first; as two launches the second one waited for shared memory behind the first.
 constexpr int LONG_SE = 128, LONG_NS = 4;
+template <bool ADA>
 __global__ void __launch_bounds__(256, 2) fm_bwd_runs_list_kernel(const __grid_constant__ CUtensorMap gmap_s, const __grid_constant__ CUtensorMap gmap_l,
                                                                   BwdParams p, int wps, int warp_f_s, int wpl, int warp_f_l, int accs_n,
                                                                   int ring_comps, unsigned nlong, int segb_off) {
-    if (blockIdx.x < nlong) runs_body<true, LONG_SE, LONG_NS, true>(gmap_l, p, wpl, warp_f_l, accs_n, ring_comps, blockIdx.x, nlong, segb_off);
-    else runs_body<true, 64, 4, false>(gmap_s, p, wps, warp_f_s, accs_n, ring_comps, blockIdx.x - nlong, gridDim.x - nlong, segb_off);
+    if (blockIdx.x < nlong) runs_body<true, LONG_SE, LONG_NS, true, ADA>(gmap_l, p, wpl, warp_f_l, accs_n, ring_comps, blockIdx.x, nlong, segb_off);
+    else runs_body<true, 64, 4, false, ADA>(gmap_s, p, wps, warp_f_s, accs_n, ring_comps, blockIdx.x - nlong, gridDim.x - nlong, segb_off);
 }
 
 static int ilog2_ceil(int x) { int l = 0; while ((1 << l) < x) ++l; return l; }
@@ -605,7 +630,8 @@ static int ring_tensor_map(CUtensorMap* gmap, const BwdParams& p, int nv, int ri
     return FMB_OK;
 }
 
-static int launch_runs(BwdParams& p, bool two, cudaStream_t stream) {
+template <bool ADA>
+static int launch_runs_t(BwdParams& p, bool two, cudaStream_t stream) {
     const int k = p.k;
     const int64_t N = p.N;
     const int nv = k + 1 + (two ? k : 0);
@@ -620,15 +646,15 @@ static int launch_runs(BwdParams& p, bool two, cudaStream_t stream) {
     const unsigned grid = (unsigned)((nwarps + wpb - 1) / wpb);
     static bool attr = false;
     if (!attr) {
-        cudaFuncSetAttribute(fm_bwd_runs_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-        cudaFuncSetAttribute(fm_bwd_runs_list_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+        cudaFuncSetAttribute(fm_bwd_runs_kernel<ADA>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+        cudaFuncSetAttribute(fm_bwd_runs_list_kernel<ADA>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
         attr = true;
     }
     CUtensorMap gmap;
     int rc = ring_tensor_map(&gmap, p, nv, ring_comps, 64);
     if (rc) return rc;
     if (!p.run_list) {
-        fm_bwd_runs_kernel<<<grid, 32 * wpb, sm, stream>>>(gmap, p, wpb, warp_f, accs_n, ring_comps);
+        fm_bwd_runs_kernel<ADA><<<grid, 32 * wpb, sm, stream>>>(gmap, p, wpb, warp_f, accs_n, ring_comps);
         FMB_CHECK_LAUNCH("fm_bwd_runs_kernel");
         return FMB_OK;
     }
@@ -662,15 +688,18 @@ static int launch_runs(BwdParams& p, bool two, cudaStream_t stream) {
         at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
         at[0].val.programmaticStreamSerializationAllowed = 1;
         cfg.attrs = at; cfg.numAttrs = 1;
-        const cudaError_t le = cudaLaunchKernelEx(&cfg, fm_bwd_runs_list_kernel, gmap, gmap_l, p, wpb, warp_f, wpl, warp_f_l, accs_n,
+        const cudaError_t le = cudaLaunchKernelEx(&cfg, fm_bwd_runs_list_kernel<ADA>, gmap, gmap_l, p, wpb, warp_f, wpl, warp_f_l, accs_n,
                                                   ring_comps, nlong, (int)(smd / 4));
         if (le != cudaSuccess) { fmb_set_error("fm_bwd_runs_list_kernel (programmatic launch): %s", cudaGetErrorString(le)); return FMB_ERR_CUDA; }
     } else {
-        fm_bwd_runs_list_kernel<<<nlong + nshort, 32 * wpb, smd + segb, stream>>>(gmap, gmap_l, p, wpb, warp_f, wpl, warp_f_l, accs_n,
+        fm_bwd_runs_list_kernel<ADA><<<nlong + nshort, 32 * wpb, smd + segb, stream>>>(gmap, gmap_l, p, wpb, warp_f, wpl, warp_f_l, accs_n,
                                                                                  ring_comps, nlong, (int)(smd / 4));
     }
     FMB_CHECK_LAUNCH("fm_bwd_runs_list_kernel");
     return FMB_OK;
+}
+static int launch_runs(BwdParams& p, bool two, cudaStream_t stream) {
+    return p.mode == 3 ? launch_runs_t<true>(p, two, stream) : launch_runs_t<false>(p, two, stream);
 }
 
 // A6 sparse backward + update (see file header).
@@ -684,17 +713,20 @@ static int launch_runs(BwdParams& p, bool two, cudaStream_t stream) {
 // _rl: with the run list of the sorted keys (nullable; fmb_shard_sort_fields_rl / fmb_sort_fields_ex) the run kernel starts
 // one warp per run, the long runs first (the owner-side chains of the sharded step are G*B/rows long)
 struct fmb_runlist_t { int32_t* entries; uint32_t* seg_count; int nseg, seg_cap; };   // include/fmb200.h
-FMB_API int fmb_fm_backward_update_rl(const int32_t* sorted_keys, const int32_t* perm, int64_t N, int64_t n_entries,
-                                      const float* xv, float* table, int F, int k, const float* S, int s_pitch,
-                                      const float* gs, int gs_stride, int use_fm2, const float* gvec,
-                                      int32_t key_limit, float lr, int mode, const fmb_runlist_t* rl, void* ws, size_t ws_bytes,
-                                      cudaStream_t stream) {
+struct fmb_adagrad_t { float* sums; float* bias_sum; float* mlp_sums; float eps; };   // include/fmb200.h
+// _rl_ex: update mode 3 (Adagrad) needs `ada` (the table's sums); NULL otherwise
+FMB_API int fmb_fm_backward_update_rl_ex(const int32_t* sorted_keys, const int32_t* perm, int64_t N, int64_t n_entries,
+                                         const float* xv, float* table, int F, int k, const float* S, int s_pitch,
+                                         const float* gs, int gs_stride, int use_fm2, const float* gvec,
+                                         int32_t key_limit, float lr, int mode, const fmb_adagrad_t* ada,
+                                         const fmb_runlist_t* rl, void* ws, size_t ws_bytes, cudaStream_t stream) {
     FMB_CHECK_ARG(!rl || (rl->entries && rl->seg_count && rl->nseg >= 1 && rl->nseg <= 2048 && rl->seg_cap >= 1),
                   "fmb_fm_backward_update: bad run list");
     FMB_CHECK_ARG(sorted_keys && perm && table && S && gs && ws, "fmb_fm_backward_update: null pointer");
     FMB_CHECK_ARG(N > 0 && F > 0 && F < 512 && k > 0 && k <= 124, "fmb_fm_backward_update: bad shape N=%lld F=%d k=%d (need F < 512, k <= 124)",
                   (long long)N, F, k);
-    FMB_CHECK_ARG(mode == 0 || mode == 1, "fmb_fm_backward_update: unknown update mode %d", mode);
+    FMB_CHECK_ARG(mode == 0 || mode == 1 || (mode == 3 && ada && ada->sums),
+                  "fmb_fm_backward_update: unknown update mode %d (mode 3 needs the Adagrad state)", mode);
     FMB_CHECK_ARG(use_fm2 || gvec, "fmb_fm_backward_update: neither gradient path enabled");
     FMB_CHECK_ARG(n_entries > 0 && n_entries < ((int64_t)1 << 31), "fmb_fm_backward_update: n_entries out of range");
     if (ws_bytes < fmb_bwd_workspace_bytes(N, k)) { fmb_set_error("fmb_fm_backward_update: workspace too small"); return FMB_ERR_WS; }
@@ -713,24 +745,47 @@ FMB_API int fmb_fm_backward_update_rl(const int32_t* sorted_keys, const int32_t*
     p.S = S; p.gs = gs; p.use_fm2 = use_fm2; p.gvec = gvec; p.lr = lr; p.mode = mode;
     p.s_pitch = s_pitch; p.gs_stride = gs_stride; p.key_limit = key_limit;
     p.astep = -(lr / 0.1f);
+    if (mode == 3) { p.ada.sums = ada->sums; p.ada.bias_sum = ada->bias_sum; p.ada.eps = ada->eps; }
     p.dbg = g_runs_dbg;
     p.Npad = bwd_npad(N);
     p.G = (float*)ws;
     const bool two = use_fm2 && gvec;
     const unsigned grid1 = (unsigned)((N + 255) / 256);
-    switch (p.cu) {
-        case 1: fm_bwd_entry1_kernel<1><<<grid1, 256, 0, stream>>>(p); break;
-        case 2: fm_bwd_entry1_kernel<2><<<grid1, 256, 0, stream>>>(p); break;
-        case 3: fm_bwd_entry1_kernel<3><<<grid1, 256, 0, stream>>>(p); break;
-        case 4: fm_bwd_entry1_kernel<4><<<grid1, 256, 0, stream>>>(p); break;
-        default: {
-            const int epb = 256 >> p.ql_log;
-            fm_bwd_entry_kernel<<<(unsigned)((N + epb - 1) / epb), 256, 0, stream>>>(p);
+    if (mode == 3) {
+        switch (p.cu) {
+            case 1: fm_bwd_entry1_kernel<1, true><<<grid1, 256, 0, stream>>>(p); break;
+            case 2: fm_bwd_entry1_kernel<2, true><<<grid1, 256, 0, stream>>>(p); break;
+            case 3: fm_bwd_entry1_kernel<3, true><<<grid1, 256, 0, stream>>>(p); break;
+            case 4: fm_bwd_entry1_kernel<4, true><<<grid1, 256, 0, stream>>>(p); break;
+            default: {
+                const int epb = 256 >> p.ql_log;
+                fm_bwd_entry_kernel<true><<<(unsigned)((N + epb - 1) / epb), 256, 0, stream>>>(p);
+            }
+        }
+    } else {
+        switch (p.cu) {
+            case 1: fm_bwd_entry1_kernel<1, false><<<grid1, 256, 0, stream>>>(p); break;
+            case 2: fm_bwd_entry1_kernel<2, false><<<grid1, 256, 0, stream>>>(p); break;
+            case 3: fm_bwd_entry1_kernel<3, false><<<grid1, 256, 0, stream>>>(p); break;
+            case 4: fm_bwd_entry1_kernel<4, false><<<grid1, 256, 0, stream>>>(p); break;
+            default: {
+                const int epb = 256 >> p.ql_log;
+                fm_bwd_entry_kernel<false><<<(unsigned)((N + epb - 1) / epb), 256, 0, stream>>>(p);
+            }
         }
     }
     FMB_CHECK_LAUNCH("fm_bwd_entry_kernel");
     if (rl) { p.run_list = reinterpret_cast<const int4*>(rl->entries); p.run_segc = rl->seg_count; p.run_nseg = rl->nseg; p.run_cap = rl->seg_cap; }
     return launch_runs(p, two, stream);
+}
+
+FMB_API int fmb_fm_backward_update_rl(const int32_t* sorted_keys, const int32_t* perm, int64_t N, int64_t n_entries,
+                                      const float* xv, float* table, int F, int k, const float* S, int s_pitch,
+                                      const float* gs, int gs_stride, int use_fm2, const float* gvec,
+                                      int32_t key_limit, float lr, int mode, const fmb_runlist_t* rl, void* ws, size_t ws_bytes,
+                                      cudaStream_t stream) {
+    return fmb_fm_backward_update_rl_ex(sorted_keys, perm, N, n_entries, xv, table, F, k, S, s_pitch, gs, gs_stride, use_fm2,
+                                        gvec, key_limit, lr, mode, nullptr, rl, ws, ws_bytes, stream);
 }
 
 FMB_API int fmb_fm_backward_update_ex(const int32_t* sorted_keys, const int32_t* perm, int64_t N, int64_t n_entries,
@@ -762,7 +817,9 @@ FMB_API int fmb_fm_backward_runs_list(const int32_t* sorted_keys, int64_t N, flo
                   "fmb_fm_backward_runs: bad run list");
     FMB_CHECK_ARG(N > 0 && F > 0 && F < 512 && k > 0 && k <= 124, "fmb_fm_backward_runs: bad shape N=%lld F=%d k=%d (need F < 512, k <= 124)",
                   (long long)N, F, k);
-    FMB_CHECK_ARG(mode == 0 || mode == 1 || (mode == 2 && ftrl && ftrl->zn), "fmb_fm_backward_runs: unknown update mode %d", mode);
+    FMB_CHECK_ARG(mode == 0 || mode == 1 || (mode == 2 && ftrl && ftrl->zn) ||
+                  (mode == 3 && ftrl && reinterpret_cast<const fmb_adagrad_t*>(ftrl)->sums),
+                  "fmb_fm_backward_runs: unknown update mode %d", mode);
     if (ws_bytes < fmb_bwd_workspace_bytes(N, k)) { fmb_set_error("fmb_fm_backward_runs: workspace too small"); return FMB_ERR_WS; }
     BwdParams p;
     memset(&p, 0, sizeof(p));
@@ -774,6 +831,10 @@ FMB_API int fmb_fm_backward_runs_list(const int32_t* sorted_keys, int64_t N, flo
     p.Npad = bwd_npad(N);
     p.G = (float*)ws;
     if (mode == 2) { p.ftrl.zn = ftrl->zn; p.ftrl.bias_zn = ftrl->bias_zn; p.ftrl.beta = ftrl->beta; p.ftrl.l1 = ftrl->l1; p.ftrl.l2 = ftrl->l2; }
+    if (mode == 3) {   // the state slot carries an fmb_adagrad_t in mode 3 (include/fmb200.h)
+        const fmb_adagrad_t* a = reinterpret_cast<const fmb_adagrad_t*>(ftrl);
+        p.ada.sums = a->sums; p.ada.bias_sum = a->bias_sum; p.ada.eps = a->eps;
+    }
     if (rl) { p.run_list = reinterpret_cast<const int4*>(rl->entries); p.run_segc = rl->seg_count; p.run_nseg = rl->nseg; p.run_cap = rl->seg_cap; }
     p.pdl = rl ? g_runs_pdl : 0;
     g_runs_pdl = 0;
@@ -795,7 +856,8 @@ FMB_API int fmb_fm_backward_runs(const int32_t* sorted_keys, int64_t N, float* t
 FMB_API int fmb_fm_backward_runs_all(const int32_t* sorted_keys, int64_t N, float* table, int F, int k, float lr,
                                      int mode, void* ws, size_t ws_bytes, cudaStream_t stream) {
     FMB_CHECK_ARG(sorted_keys && table && ws, "fmb_fm_backward_runs_all: null pointer");
-    FMB_CHECK_ARG(N > 0 && F > 0 && F < 512 && k > 0 && k <= 124 && (mode == 0 || mode == 1), "fmb_fm_backward_runs_all: bad arguments");
+    FMB_CHECK_ARG(N > 0 && F > 0 && F < 512 && k > 0 && k <= 124, "fmb_fm_backward_runs_all: bad arguments");
+    FMB_CHECK_ARG(mode == 0 || mode == 1, "fmb_fm_backward_runs_all: unknown update mode %d", mode);
     if (ws_bytes < fmb_bwd_workspace_bytes(N, k)) { fmb_set_error("fmb_fm_backward_runs_all: workspace too small"); return FMB_ERR_WS; }
     BwdParams p;
     memset(&p, 0, sizeof(p));

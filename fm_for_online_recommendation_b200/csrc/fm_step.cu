@@ -48,7 +48,10 @@ struct StepParams {
     float* lossv;              // [B] out
     float* G;                  // [k+1][Npad] staged contributions of multi-hit entries
     int64_t Npad;
-    fmb::FtrlState ftrl;       // mode 2 only
+    union {                    // the update rule's per-coordinate state (same size as the FTRL state alone)
+        fmb::FtrlState ftrl;       // mode 2 only
+        fmb::AdagradState ada;     // mode 3 only
+    };
     long long* tdbg;           // debug only: per-CTA phase timestamps [grid][8] (globaltimer ns), else NULL
     int dbg;                   // debug/attribution only (fmb_debug_set_step_flags): 1 = skip phase 4a, 2 = skip phase 4b
 };
@@ -58,7 +61,8 @@ struct StepParams {
 // Template parameters: CU = 16-byte chunks per row when known at compile time (3 for k = 8..11: the row pitch in shared
 // memory is then a constant and the field loop addresses with immediates), 0 = read it from the parameters;
 // XV = the batch carries real feature values (else all ones: no loads, no multiplications by x -- a product with 1.0f
-// is exact, so skipping it changes no bit); MODE = update rule (0 fresh-Adam sign step, 1 SGD, 2 FTRL-Proximal).
+// is exact, so skipping it changes no bit); MODE = update rule (0 fresh-Adam sign step, 1 SGD, 2 FTRL-Proximal,
+// 3 Adagrad).
 // 32 registers (8 CTAs per SM): the 1 024 tiles of an 8 192-sample batch are then resident at once.
 template <int CU, bool XV, int MODE>
 __global__ void __launch_bounds__(256, MODE == 2 ? 4 : 8) fm_step_fused_kernel(const int32_t* __restrict__ ids, const float* __restrict__ xv,
@@ -199,7 +203,8 @@ __global__ void __launch_bounds__(256, MODE == 2 ? 4 : 8) fm_step_fused_kernel(c
             // Saturated samples (the reference's N(0,1) initialisation puts |z| ~ 90 on Criteo-shaped rows) leave their
             // rows exactly where they are; two exact item-level tests spare them the per-coordinate work.
             // (i) delta == 0 (sigmoid rounded to y): every gradient is +0 after the `0 +`, and the Adam step of a zero
-            //     gradient returns p for every p (shortcut, or p + (-0) in the full pipeline); SGD: fma(+0, -lr, p) = p.
+            //     gradient returns p for every p (shortcut, or p + (-0) in the full pipeline); SGD: fma(+0, -lr, p) = p;
+            //     Adagrad: fma(+0, +0, s) = s and p + (-0) / std = p.
             if (d == 0.0f) continue;
             // (ii) |delta| < 1e-30 with |S_j| < 1e4 and 1e-9 < |p| < 1e4: |g| <= 2.0001e-26 is below the window test's
             //     range, and the quarter-ulp bound |a|*0.1*|g|*1.0001e8 <= 2.001e-18 (|a| <= 10) is below
@@ -215,6 +220,32 @@ __global__ void __launch_bounds__(256, MODE == 2 ? 4 : 8) fm_step_fused_kernel(c
                 }
                 if (same) continue;
             }
+        }
+        if (MODE == 3) {
+            // Adagrad: the row's sums sit at the row's offsets of their own table (read + written: 8F(k+1) more bytes per
+            // sample).  Gradient and update per coordinate, so that only one gradient is live at a time (32 registers).
+            float* srow = p.ada.sums + (size_t)ids_s[ef] * p.rowp + q * 4;
+            const float4 s4 = *reinterpret_cast<const float4*>(srow);
+            float sv[4] = {s4.x, s4.y, s4.z, s4.w}, o[4];
+#pragma unroll
+            for (int t = 0; t < 4; ++t) {
+                const int j = q * 4 + t;
+                o[t] = v[t];
+                if (j <= k) {
+                    float a;
+                    if (j < k) {
+                        const float ej = XV ? __fmul_rn(v[t], x) : v[t];
+                        a = __fsub_rn(__fmul_rn(d, Sq[t]), __fmul_rn(d, ej));
+                        if (XV) a = __fmul_rn(a, x);
+                    } else {
+                        a = XV ? __fmul_rn(d, x) : d;
+                    }
+                    o[t] = fmb::adagrad_update(v[t], __fadd_rn(0.f, a), sv[t], p.lr, p.ada.eps);
+                }
+            }
+            *reinterpret_cast<float4*>(p.table + (size_t)ids_s[ef] * p.rowp + q * 4) = make_float4(o[0], o[1], o[2], o[3]);
+            *reinterpret_cast<float4*>(srow) = make_float4(sv[0], sv[1], sv[2], sv[3]);   // padding lanes: as read
+            continue;
         }
         float o[4];
         bool moved = false;
@@ -365,8 +396,9 @@ FMB_API void fmb_debug_set_step_flags(int f) { g_step_dbg = f; }
 // host-side handle of the fused kernel, for graph-node identification in session.cu (arguments 0..3 are ids, xv, y, posflag)
 typedef void (*fused_fn_t)(const int32_t*, const float*, const float*, const uint32_t*, StepParams);
 static fused_fn_t fused_fn(int cu, bool xv, int mode) {
-#define FMB_FUSED_ROW(C, X) {fm_step_fused_kernel<C, X, 0>, fm_step_fused_kernel<C, X, 1>, fm_step_fused_kernel<C, X, 2>}
-    static const fused_fn_t tab[2][2][3] = {{FMB_FUSED_ROW(0, false), FMB_FUSED_ROW(0, true)},
+#define FMB_FUSED_ROW(C, X) {fm_step_fused_kernel<C, X, 0>, fm_step_fused_kernel<C, X, 1>, fm_step_fused_kernel<C, X, 2>, \
+                             fm_step_fused_kernel<C, X, 3>}
+    static const fused_fn_t tab[2][2][4] = {{FMB_FUSED_ROW(0, false), FMB_FUSED_ROW(0, true)},
                                             {FMB_FUSED_ROW(3, false), FMB_FUSED_ROW(3, true)}};
 #undef FMB_FUSED_ROW
     return tab[cu == 3][xv][mode];
@@ -375,7 +407,7 @@ static fused_fn_t fused_fn(int cu, bool xv, int mode) {
 FMB_API int fmb_is_fused_kernel_fn(const void* fn) {
     for (int c = 0; c < 2; ++c)
         for (int x = 0; x < 2; ++x)
-            for (int m = 0; m < 3; ++m)
+            for (int m = 0; m < 4; ++m)
                 if (fn == (const void*)fused_fn(c ? 3 : 0, x != 0, m)) return 1;
     return 0;
 }
@@ -408,6 +440,7 @@ FMB_API int fmb_pos_flags(const int32_t* sorted_keys, const int32_t* perm, int64
 //   bytes, handed to fmb_fm_backward_runs afterwards;  delta/lossv [B]: per-sample gradient and loss (inputs of
 //   fmb_finish_step).  mode as in fmb_fm_backward_update.
 struct fmb_ftrl_t { float* zn; float* bias_zn; float beta, l1, l2; };   // include/fmb200.h
+struct fmb_adagrad_t { float* sums; float* bias_sum; float* mlp_sums; float eps; };   // include/fmb200.h
 
 FMB_API int fmb_fm_step_fused_ex(const int32_t* ids, const float* xv, const float* y, float* table, const float* bias,
                                  const uint32_t* posflag, int B, int F, int k, int loss_kind, float lr, int mode,
@@ -416,7 +449,9 @@ FMB_API int fmb_fm_step_fused_ex(const int32_t* ids, const float* xv, const floa
     FMB_CHECK_ARG(ids && y && table && bias && posflag && delta && lossv && ws, "fmb_fm_step_fused: null pointer");
     FMB_CHECK_ARG(B > 0 && F > 0 && F < 512 && k > 0 && k <= 124, "fmb_fm_step_fused: bad shape B=%d F=%d k=%d", B, F, k);
     FMB_CHECK_ARG(loss_kind == 0 || loss_kind == 1, "fmb_fm_step_fused: unknown loss kind %d", loss_kind);
-    FMB_CHECK_ARG(mode == 0 || mode == 1 || (mode == 2 && ftrl && ftrl->zn), "fmb_fm_step_fused: unknown update mode %d (mode 2 needs the FTRL state)", mode);
+    FMB_CHECK_ARG(mode == 0 || mode == 1 || (mode == 2 && ftrl && ftrl->zn) ||
+                  (mode == 3 && ftrl && reinterpret_cast<const fmb_adagrad_t*>(ftrl)->sums),
+                  "fmb_fm_step_fused: unknown update mode %d (mode 2 needs the FTRL state, mode 3 the Adagrad state)", mode);
     const int64_t N = (int64_t)B * F;
     if (ws_bytes < fmb_bwd_workspace_bytes(N, k)) { fmb_set_error("fmb_fm_step_fused: workspace too small"); return FMB_ERR_WS; }
     StepParams p;
@@ -430,6 +465,7 @@ FMB_API int fmb_fm_step_fused_ex(const int32_t* ids, const float* xv, const floa
     p.dbg = g_step_dbg;
     p.ftrl.zn = nullptr; p.ftrl.bias_zn = nullptr; p.ftrl.beta = p.ftrl.l1 = p.ftrl.l2 = 0.f;
     if (mode == 2) { p.ftrl.zn = ftrl->zn; p.ftrl.bias_zn = ftrl->bias_zn; p.ftrl.beta = ftrl->beta; p.ftrl.l1 = ftrl->l1; p.ftrl.l2 = ftrl->l2; }
+    if (mode == 3) { const fmb_adagrad_t* a = reinterpret_cast<const fmb_adagrad_t*>(ftrl); p.ada.sums = a->sums; p.ada.bias_sum = a->bias_sum; p.ada.eps = a->eps; }
     p.tdbg = g_step_tdbg;
     int SB = 256 >> p.jl_log;
     if (SB < 4) SB = 4;

@@ -211,6 +211,28 @@ __device__ __forceinline__ float ftrl_update(float w, float g, float& z, float& 
     const float den = __fadd_rn(__fdiv_rn(__fadd_rn(beta, snn), alpha), l2);
     return -__fdiv_rn(num, den);
 }
+// mode 3: torch.optim.Adagrad (lr_decay = 0, weight_decay = 0) with a persistent per-coordinate sum s, in the order
+// torch 2.11's CPU _single_tensor_adagrad rounds it (tests/adagrad_oracle.c orc_adagrad_update is the same sequence, pinned on torch):
+//   s' = fma(g, g, s)   (state_sum.addcmul_(grad, grad, value=1))
+//   std = sqrt(s') + eps   (state_sum.sqrt(): MKL vsSqrt = sqrt_mkl, then add_(eps))
+//   p' = p + (-lr * g) / std   (param.addcdiv_(grad, std, value=-lr): the product first, then the quotient)
+// A zero gradient leaves p and s exactly as they are, so updating only the rows a batch hits is the dense optimizer.
+struct AdagradState {
+    float* sums;      // [R][rowp]: row r's sums at row r's offsets of the packed table (NULL = mode 3 unavailable)
+    float* bias_sum;  // [1]
+    float eps;
+};
+// the per-coordinate state of modes 2 and 3 in one kernel argument
+union UpdateState {
+    FtrlState ftrl;
+    AdagradState ada;
+};
+__device__ __forceinline__ float adagrad_update(float p, float g, float& s, float lr, float eps) {
+    const float ss = __fmaf_rn(g, g, s);
+    s = ss;
+    const float sd = __fadd_rn(sqrt_mkl(ss), eps);
+    return __fadd_rn(p, __fdiv_rn(__fmul_rn(-lr, g), sd));
+}
 // same with the Adam step size precomputed
 __device__ __forceinline__ float apply_update_a(float p, float g, float lr, float astep, int mode) {
     return mode == 0 ? adam1_a(p, g, astep) : __fmaf_rn(g, -lr, p);

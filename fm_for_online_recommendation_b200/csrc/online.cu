@@ -28,6 +28,10 @@ struct OnlineParams {
     float* acc;          // [n_mlp] hedge accumulator (ONN)
     float lr, hb, hs;
     int mode;
+    float* ada_sums;     // mode 3 (Adagrad): sums of the table [R][rowp], the bias [1] and the tower [n_mlp]
+    float* ada_bias;
+    float* ada_mlp;
+    float eps;
     uint8_t* preds;      // [N]
     int64_t* conf;       // [4] tp, fp, tn, fn
 };
@@ -36,6 +40,20 @@ __device__ __forceinline__ size_t w_off(int k, int H, int l) {
     return l == 0 ? 0 : (size_t)H * k + H + (size_t)(l - 1) * ((size_t)H * H + H);
 }
 
+// the Adam family's update of one parameter; mode 3 (ADA, an instantiation of its own so that the other modes' kernel
+// stays as it is) also reads and writes its Adagrad sum *s
+template <bool ADA>
+__device__ __forceinline__ float online_update(const OnlineParams& p, float w, float g, float* s) {
+    if (ADA) {
+        float sv = *s;
+        const float o = fmb::adagrad_update(w, g, sv, p.lr, p.eps);
+        *s = sv;
+        return o;
+    }
+    return fmb::apply_update(w, g, p.lr, p.mode);
+}
+
+template <bool ADA>
 __global__ void __launch_bounds__(OT) online_deep_kernel(OnlineParams p) {
     extern __shared__ __align__(16) float sm[];
     const int F = p.F, k = p.k, L = p.L, H = p.H, rp = p.cu * 4;
@@ -158,9 +176,10 @@ __global__ void __launch_bounds__(OT) online_deep_kernel(OnlineParams p) {
                     __syncthreads();
                     for (int q = tid; q < H * nin; q += OT) {  // fresh-Adam step on W_l (gradient = gp[o]*x[i], B = 1)
                         const int o = q / nin, i = q - o * nin;
-                        W[q] = fmb::apply_update(W[q], __fmaf_rn(gp[o], xin[i], 0.f), p.lr, p.mode);
+                        W[q] = online_update<ADA>(p, W[q], __fmaf_rn(gp[o], xin[i], 0.f), p.ada_mlp + w_off(k, H, l) + q);
                     }
-                    for (int o = tid; o < H; o += OT) c[o] = fmb::apply_update(c[o], __fadd_rn(0.f, gp[o]), p.lr, p.mode);
+                    for (int o = tid; o < H; o += OT)
+                        c[o] = online_update<ADA>(p, c[o], __fadd_rn(0.f, gp[o]), p.ada_mlp + w_off(k, H, l) + (size_t)H * nin + o);
                     __syncthreads();
                     if (l > 0) { for (int i = tid; i < H; i += OT) gp[i] = act[(l - 1) * H + i] > 0.f ? gx[i] : 0.f; }
                     else { for (int i = tid; i < k; i += OT) gbi[i] = gx[i]; }
@@ -182,9 +201,9 @@ __global__ void __launch_bounds__(OT) online_deep_kernel(OnlineParams p) {
                 } else {
                     g = __fadd_rn(0.f, __fmul_rn(d, x));
                 }
-                p.table[(size_t)id[f] * p.rowp + j] = fmb::apply_update(v, g, p.lr, p.mode);
+                p.table[(size_t)id[f] * p.rowp + j] = online_update<ADA>(p, v, g, p.ada_sums + (size_t)id[f] * p.rowp + j);
             }
-            if (tid == 0) p.bias[0] = fmb::apply_update(p.bias[0], __fadd_rn(0.f, d), p.lr, p.mode);
+            if (tid == 0) p.bias[0] = online_update<ADA>(p, p.bias[0], __fadd_rn(0.f, d), p.ada_bias);
         } else {
             // hedge backpropagation, batch_size = 1: L backward passes, only the tower and alpha change
             const size_t nm = w_off(k, H, L);
@@ -249,28 +268,48 @@ static int ilog2_ceil(int x) { int l = 0; while ((1 << l) < x) ++l; return l; }
 // NFMOnn; ids [N,F] global row ids, xv [N,F] or NULL, y [N]; mlp/alpha/acc may be NULL for kind 0 (acc:
 // [fmb_mlp_numel] scratch, ONN only).  Outputs: preds [N] (the prediction made BEFORE fitting example i),
 // conf [4] = tp, fp, tn, fn (int64).
-FMB_API int fmb_online_deep_run(int kind, const int32_t* ids, const float* xv, const float* y, int N, int F, int k,
-                                int L, int H, float* table, float* bias, float* mlp, float* alpha, float* acc,
-                                float lr, float hb, float hs, int mode, uint8_t* preds, int64_t* conf,
-                                cudaStream_t stream) {
+// _ex: update mode 3 (Adagrad) of the Adam family (kinds 0-2) reads and writes the sums in `ada` (the table's, the
+// bias's and, with a tower, the tower's); the ONN kinds' hedge step uses no optimizer and ignores the mode.
+struct fmb_adagrad_t { float* sums; float* bias_sum; float* mlp_sums; float eps; };   // include/fmb200.h
+FMB_API int fmb_online_deep_run_ex(int kind, const int32_t* ids, const float* xv, const float* y, int N, int F, int k,
+                                   int L, int H, float* table, float* bias, float* mlp, float* alpha, float* acc,
+                                   float lr, float hb, float hs, int mode, const fmb_adagrad_t* ada, uint8_t* preds,
+                                   int64_t* conf, cudaStream_t stream) {
     FMB_CHECK_ARG(kind >= 0 && kind <= 4, "fmb_online_deep_run: unknown model kind %d", kind);
     FMB_CHECK_ARG(ids && y && table && bias && preds && conf, "fmb_online_deep_run: null pointer");
     FMB_CHECK_ARG(N > 0 && F > 0 && F < 512 && k > 0 && k <= 124, "fmb_online_deep_run: bad shape N=%d F=%d k=%d (need F < 512, k <= 124)",
                   N, F, k);
     FMB_CHECK_ARG(kind == 0 || (mlp && L > 0 && H > 0 && H < 512), "fmb_online_deep_run: tower needs mlp, 0 < H < 512");
     FMB_CHECK_ARG(kind < 3 || (alpha && acc), "fmb_online_deep_run: ONN needs alpha and acc");
+    FMB_CHECK_ARG(mode != 3 || kind >= 3 || (ada && ada->sums && ada->bias_sum && (kind == 0 || ada->mlp_sums)),
+                  "fmb_online_deep_run: update mode 3 needs the Adagrad state (sums of the table, the bias and the tower)");
     OnlineParams p;
     p.kind = kind; p.N = N; p.F = F; p.k = k; p.L = kind == 0 ? 0 : L; p.H = kind == 0 ? 0 : H;
     p.rowp = fmb_round_up(k + 1, 16); p.kp4 = fmb_round_up(k, 4); p.cu = (k + 1 + 3) / 4; p.ql_log = ilog2_ceil(p.cu);
     p.ids = ids; p.xv = xv; p.y = y; p.table = table; p.bias = bias; p.mlp = mlp; p.alpha = alpha; p.acc = acc;
     p.lr = lr; p.hb = hb; p.hs = hs; p.mode = mode; p.preds = preds; p.conf = conf;
+    p.ada_sums = p.ada_bias = p.ada_mlp = nullptr; p.eps = 0.f;
+    if (mode == 3 && ada) { p.ada_sums = ada->sums; p.ada_bias = ada->bias_sum; p.ada_mlp = ada->mlp_sums; p.eps = ada->eps; }
     const int mx = p.H > k ? p.H : k;
     const size_t fl = (size_t)F * p.cu * 4 + 2 * F + 2 * k + (size_t)p.L * p.H + 2 * mx + k + 2 * (p.L > 0 ? p.L : 1) + 16;
     const size_t smb = fl * sizeof(float);
     FMB_CHECK_ARG(smb <= 200 * 1024, "fmb_online_deep_run: model too large for one CTA's shared memory (F=%d k=%d L=%d H=%d: %zu bytes > 200 KB)",
                   F, k, p.L, p.H, smb);
-    cudaFuncSetAttribute(online_deep_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-    online_deep_kernel<<<1, OT, smb, stream>>>(p);
+    if (mode == 3 && kind < 3) {
+        cudaFuncSetAttribute(online_deep_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+        online_deep_kernel<true><<<1, OT, smb, stream>>>(p);
+    } else {
+        cudaFuncSetAttribute(online_deep_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+        online_deep_kernel<false><<<1, OT, smb, stream>>>(p);
+    }
     FMB_CHECK_LAUNCH("online_deep_kernel");
     return FMB_OK;
+}
+
+FMB_API int fmb_online_deep_run(int kind, const int32_t* ids, const float* xv, const float* y, int N, int F, int k,
+                                int L, int H, float* table, float* bias, float* mlp, float* alpha, float* acc,
+                                float lr, float hb, float hs, int mode, uint8_t* preds, int64_t* conf,
+                                cudaStream_t stream) {
+    return fmb_online_deep_run_ex(kind, ids, xv, y, N, F, k, L, H, table, bias, mlp, alpha, acc, lr, hb, hs, mode, nullptr,
+                                  preds, conf, stream);
 }

@@ -26,6 +26,7 @@ int fmb_fm_backward_update(const int32_t*, const int32_t*, int64_t, const float*
                            const float*, int, const float*, float, int, void*, size_t, cudaStream_t);
 int fmb_finish_step(const float*, const float*, int, float*, float, int, float*, cudaStream_t);
 struct fmb_ftrl_t { float* zn; float* bias_zn; float beta, l1, l2; };
+struct fmb_adagrad_t { float* sums; float* bias_sum; float* mlp_sums; float eps; };
 int fmb_fm_backward_runs_list(const int32_t*, int64_t, float*, int, int, float, int, const fmb_ftrl_t*, const fmb_runlist_t*,
                               void*, size_t, cudaStream_t);
 int fmb_finish_step_ex(const float*, const float*, int, float*, float, int, const fmb_ftrl_t*, float*, cudaStream_t);
@@ -130,6 +131,8 @@ struct fmb_session {
     int npsg, presort_warm;
     fmb_ftrl_t ftrl;       // update mode 2 (fmb_session_set_ftrl)
     int ftrl_set;
+    fmb_adagrad_t ada;     // update mode 3 (fmb_session_set_adagrad)
+    int ada_set;
 };
 
 #define CU(call)                                                                              \
@@ -272,6 +275,18 @@ FMB_API int fmb_session_set_ftrl(fmb_session* s, float* zn_dev, float* bias_zn_d
     return FMB_OK;
 }
 
+// update mode 3 (Adagrad): the sums the session's steps read and write.  sums_dev [R][rowp] (row r's sums at row r's
+// offsets of the packed table), bias_sum_dev [1]; initialised by the caller (initial_accumulator_value).  Step graphs
+// captured before this call are dropped.
+FMB_API int fmb_session_set_adagrad(fmb_session* s, float* sums_dev, float* bias_sum_dev, float eps) {
+    FMB_CHECK_ARG(s && sums_dev && bias_sum_dev && eps >= 0.f, "fmb_session_set_adagrad: bad arguments");
+    s->ada.sums = sums_dev; s->ada.bias_sum = bias_sum_dev; s->ada.mlp_sums = nullptr; s->ada.eps = eps;
+    s->ada_set = 1;
+    for (int i = 0; i < s->ngraphs; ++i) { cudaGraphExecDestroy(s->gvar[i].exec); cudaGraphDestroy(s->gvar[i].graph); }
+    s->ngraphs = 0; s->next_evict = 0;
+    return FMB_OK;
+}
+
 FMB_API int64_t fmb_session_launches(const fmb_session* s) { return s ? s->launches : 0; }
 FMB_API int fmb_session_graph_count(const fmb_session* s) { return s ? s->ngraphs : 0; }
 
@@ -341,7 +356,9 @@ static int fm_step_launch(fmb_session* s, const int32_t* ids, const float* xv, c
         rc = sort_launch(s, ids, B, key_bits, cur, s->d_sort_ws, main, nlaunch);
         if (rc) return rc;
     }
-    const fmb_ftrl_t* ft = s->ftrl_set ? &s->ftrl : nullptr;
+    // the state slot of the step's kernels: the FTRL state, or in mode 3 the Adagrad state (include/fmb200.h)
+    const fmb_ftrl_t* ft = mode == 3 ? (s->ada_set ? reinterpret_cast<const fmb_ftrl_t*>(&s->ada) : nullptr)
+                                     : (s->ftrl_set ? &s->ftrl : nullptr);
     rc = fmb_fm_step_fused_ex(ids, xv, y, table, bias, s->d_posflag_buf[cur], B, s->F, s->k, loss_kind, lr, mode, ft,
                               s->d_delta, s->d_lossv, s->d_bwd_ws, s->bwd_ws_bytes, main);
     if (rc) return rc;

@@ -23,9 +23,10 @@ import torch
 import torch.nn as nn
 
 from . import _lib
-from ._lib import FmbError, RunList, check, ptr
+from ._lib import AdagradState, FmbError, RunList, check, ptr
 
 UPDATE_ADAM1, UPDATE_SGD, UPDATE_FTRL = 0, 1, 2   # 2: per-coordinate FTRL-Proximal (enable_ftrl), FM-only steps
+UPDATE_ADAGRAD = 3   # torch.optim.Adagrad with state kept across calls (enable_adagrad): FM steps, tower fit, run_experiment
 LOSS_LOGITS, LOSS_LOGITS_OF_SIG = 0, 1
 _PRESORT_STANDALONE = __import__("os").environ.get("FMB_PRESORT_STANDALONE", "0") == "1"
 _DEEP_GRAPH = __import__("os").environ.get("FMB_DEEP_GRAPH", "1") != "0"   # tower `fit` replayed as one CUDA graph
@@ -72,6 +73,10 @@ def _rebuild(cls, kwargs, state):
     m = cls(**kwargs)
     m._load_packed_state(state)
     return m
+
+
+def _f32(t):
+    return None if t is None else t.detach().cpu()
 
 
 class _DeepBase(nn.Module):
@@ -155,6 +160,9 @@ class _DeepBase(nn.Module):
         self._session_cap = 0
         self._presorted = None   # the EncodedBatch whose sorted form the session holds (kept alive: its ids pointer is the key)
         self._ws = {}
+        self._ada = None
+        if update_mode == UPDATE_ADAGRAD:
+            self.enable_adagrad()
 
     def _bind_embeddings(self):
         k = self.embedding_size
@@ -194,6 +202,9 @@ class _DeepBase(nn.Module):
             st["mlp"] = self._mlp.detach().cpu()
         if self._IS_ONN:
             st["alpha"] = self.alpha.detach().cpu()
+        if self.update_mode == UPDATE_ADAGRAD:
+            st["adagrad"] = {"eps": self._ada_eps, "sums": _f32(self._ada_sums), "bias_sum": _f32(self._ada_bias),
+                             "mlp_sums": _f32(self._ada_mlp)}
         return st
 
     def _load_packed_state(self, st):
@@ -204,6 +215,14 @@ class _DeepBase(nn.Module):
                 self._mlp.copy_(st["mlp"])
             if self._IS_ONN:
                 self.alpha.copy_(st["alpha"])
+        ada = st.get("adagrad")
+        if ada is not None:
+            self.enable_adagrad(eps=ada["eps"])
+            with torch.no_grad():
+                self._ada_sums.copy_(ada["sums"])
+                self._ada_bias.copy_(ada["bias_sum"])
+                if self._ada_mlp is not None:
+                    self._ada_mlp.copy_(ada["mlp_sums"])
 
     def __reduce__(self):  # pickle.dump(model) (main_experiment.py:160-162): one copy of the table, no handles
         return (_rebuild, (type(self), self._ctor_kwargs(), self._export_state()))
@@ -276,6 +295,36 @@ class _DeepBase(nn.Module):
         check(self._lib.fmb_session_set_ftrl(self._session, ptr(self._ftrl_zn), ptr(self._ftrl_bias), *self._ftrl),
               "fmb_session_set_ftrl")
 
+    def enable_adagrad(self, eps=1e-10, initial_accumulator_value=0.0):
+        """Switch update_embedding, fit (FMAdam / DeepFMAdam / NFMAdam) and run_experiment to torch.optim.Adagrad: the
+        same trajectory as ONE `torch.optim.Adagrad(model.parameters(), lr=n, eps=eps,
+        initial_accumulator_value=initial_accumulator_value)` kept across calls in place of the reference's per-call
+        Adam.  Only the rows a batch hits are updated: a zero gradient leaves Adagrad's weight and sum as they are, so this
+        is the dense optimizer exactly.  The sums (one per coordinate of the table, the bias and the tower) start at
+        `initial_accumulator_value`; calling this again resets them.  The ONN classes' hedge fit uses no optimizer and
+        stays as it is."""
+        v = float(np.float32(initial_accumulator_value))
+        if v < 0:
+            raise ValueError("initial_accumulator_value must be >= 0")
+        self.update_mode = UPDATE_ADAGRAD
+        self._ada_eps = float(np.float32(eps))
+        self._ada_sums = torch.full((self._R, self._rowp), v, dtype=torch.float32, device=self.device)
+        self._ada_bias = torch.full((1,), v, dtype=torch.float32, device=self.device)
+        self._ada_mlp = None if self._mlp is None else torch.full_like(self._mlp, v)
+        self._ada = AdagradState(self._ada_sums.data_ptr(), self._ada_bias.data_ptr(),
+                                 None if self._ada_mlp is None else self._ada_mlp.data_ptr(), self._ada_eps)
+        self.__dict__.pop("_fit_graphs", None)   # captured fits hold the previous state's pointers
+        if self._session is not None:
+            self._bind_adagrad()
+
+    def _ada_arg(self):
+        """the fmb_adagrad_t of the C entry points' state slot in mode 3, else NULL"""
+        return C.byref(self._ada) if self.update_mode == UPDATE_ADAGRAD and self._ada is not None else None
+
+    def _bind_adagrad(self):
+        check(self._lib.fmb_session_set_adagrad(self._session, ptr(self._ada_sums), ptr(self._ada_bias), self._ada_eps),
+              "fmb_session_set_adagrad")
+
     def _get_session(self, B):
         if self._session is None or B > self._session_cap:
             if self._session is not None:
@@ -290,6 +339,8 @@ class _DeepBase(nn.Module):
             self._presorted = None
             if self.update_mode == UPDATE_FTRL:
                 self._bind_ftrl()
+            elif self.update_mode == UPDATE_ADAGRAD:
+                self._bind_adagrad()
         return self._session
 
     def _buf(self, name, shape, dtype=torch.float32):
@@ -454,13 +505,15 @@ class _DeepBase(nn.Module):
         N = B * F
         bwsb = lib.fmb_bwd_workspace_bytes(N, k)
         bws = self._buf("bwd_ws", (bwsb,), torch.uint8)
-        check(lib.fmb_fm_backward_update_rl(ptr(sk), ptr(pm), N, N, ptr(e.xv), ptr(self._table), F, k, ptr(o["S"]), self._kp4,
-                                            ptr(delta), 1, 0 if self._IS_NFM else 1, ptr(gbi), 0x7FFFFFFF, self._lr,
-                                            self.update_mode, C.byref(rl) if rl is not None else None, ptr(bws), bwsb, st),
-              "fmb_fm_backward_update")
-        check(lib.fmb_update_dense(ptr(self._mlp), ptr(gmlp), self._mlp.numel(), self._lr, self.update_mode, st),
+        ada = self._ada_arg()   # the _ex forms are the plain ones outside mode 3
+        check(lib.fmb_fm_backward_update_rl_ex(ptr(sk), ptr(pm), N, N, ptr(e.xv), ptr(self._table), F, k, ptr(o["S"]),
+                                               self._kp4, ptr(delta), 1, 0 if self._IS_NFM else 1, ptr(gbi), 0x7FFFFFFF,
+                                               self._lr, self.update_mode, ada, C.byref(rl) if rl is not None else None,
+                                               ptr(bws), bwsb, st), "fmb_fm_backward_update")
+        check(lib.fmb_update_dense_ex(ptr(self._mlp), ptr(gmlp), self._mlp.numel(), self._lr, self.update_mode,
+                                      ptr(self._ada_mlp) if ada else None, self._ada_eps if ada else 0.0, st),
               "fmb_update_dense")
-        check(lib.fmb_finish_step(ptr(delta), None, B, ptr(self.bias), self._lr, self.update_mode, None, st),
+        check(lib.fmb_finish_step_ex(ptr(delta), None, B, ptr(self.bias), self._lr, self.update_mode, ada, None, st),
               "fmb_finish_step")
 
     def _deep_fit_graphed(self, e):
@@ -611,11 +664,11 @@ class _DeepBase(nn.Module):
         preds_dev = torch.empty(data_size, dtype=torch.uint8, device=self.device)
         conf_dev = torch.zeros(4, dtype=torch.int64, device=self.device)
         acc = self._buf("hedge_acc", (self._mlp.numel(),)) if self._IS_ONN else None
-        check(self._lib.fmb_online_deep_run(self._KIND_ID, ptr(enc.ids), ptr(enc.xv), ptr(enc.y), data_size,
-                                            self.field_size, self.embedding_size, self._L, self._H, ptr(self._table),
-                                            ptr(self.bias), ptr(self._mlp), ptr(getattr(self, "alpha", None)),
-                                            ptr(acc), self._lr, self._hb, self._hs, self.update_mode, ptr(preds_dev),
-                                            ptr(conf_dev), _stream()), "fmb_online_deep_run")
+        check(self._lib.fmb_online_deep_run_ex(self._KIND_ID, ptr(enc.ids), ptr(enc.xv), ptr(enc.y), data_size,
+                                               self.field_size, self.embedding_size, self._L, self._H, ptr(self._table),
+                                               ptr(self.bias), ptr(self._mlp), ptr(getattr(self, "alpha", None)),
+                                               ptr(acc), self._lr, self._hb, self._hs, self.update_mode, self._ada_arg(),
+                                               ptr(preds_dev), ptr(conf_dev), _stream()), "fmb_online_deep_run")
         # bookkeeping of fm_adam.py:101-116: the kernel counted tp/fp/tn/fn as it went; the reference returns only the
         # LAST accuracy / roc entry, which are functions of the final counts (one 32-byte read, no per-sample host loop)
         tp, fp, tn, fn = (int(v) for v in conf_dev.cpu())

@@ -41,6 +41,8 @@ typedef struct fmb_session fmb_session;
 #define FMB_UPDATE_ADAM1 0 /* torch.optim.Adam re-created every call => first-step sign update
                               (fm_adam.py:60,68; SURVEY.md A12) -- the reference behaviour */
 #define FMB_UPDATE_SGD 1   /* p -= lr * g (legacy notebooks' torch.optim.SGD; SURVEY.md 8f.4) */
+#define FMB_UPDATE_FTRL 2  /* per-coordinate FTRL-Proximal, FM-only steps (fmb_ftrl_t below) */
+#define FMB_UPDATE_ADAGRAD 3 /* torch.optim.Adagrad with persistent per-coordinate sums (fmb_adagrad_t below) */
 
 /* loss variants (SURVEY.md A6) */
 #define FMB_LOSS_BCE_LOGITS 0         /* F.binary_cross_entropy_with_logits(z, y) */
@@ -131,6 +133,9 @@ int fmb_math_eval(int op, const float* x_dev, float* y_dev, int64_t n, fmb_strea
 int fmb_sum_aten(const float* x_dev, int64_t n, float* out_dev, fmb_stream_t stream);
 /* optimizer.step() on dense parameters (bias, hidden_layers): fm_adam.py:68 */
 int fmb_update_dense(float* p_dev, const float* g_dev, int64_t n, float lr, int mode, fmb_stream_t stream);
+/* _ex: update mode 3 (Adagrad) with the parameters' sums sums_dev [n] (read and written; NULL in the other modes) */
+int fmb_update_dense_ex(float* p_dev, const float* g_dev, int64_t n, float lr, int mode, float* sums_dev, float eps,
+                        fmb_stream_t stream);
 /* bias step from sum(delta) and mean loss; bias_dev / loss_out_dev nullable */
 int fmb_finish_step(const float* delta_dev, const float* lossv_dev, int B, float* bias_dev, float lr, int mode,
                     float* loss_out_dev, fmb_stream_t stream);
@@ -181,6 +186,16 @@ int fmb_sort_fields_ex(const int32_t* ids_dev, int B, int F, const int32_t* fiel
  * zn_dev [R][2][rowp] holds the z and n sub-rows of every packed table row, bias_zn_dev [2] those of the bias.  The _ex
  * entry points are the plain ones plus this state (NULL unless mode == 2); algorithmic bytes grow by 16F(k+1) per sample. */
 typedef struct fmb_ftrl_t { float* zn_dev; float* bias_zn_dev; float beta, l1, l2; } fmb_ftrl_t;
+/* update mode 3: torch.optim.Adagrad(lr = the step's lr, lr_decay = 0, weight_decay = 0, eps,
+ * initial_accumulator_value = the caller's fill of the sums), one optimizer kept across calls.  Per coordinate, in the
+ * order torch's CPU _single_tensor_adagrad rounds it:  s' = fma(g, g, s);  p' = p + (-lr * g) / (sqrt(s') + eps).
+ * A zero gradient leaves p and s as they are, so updating only the rows a batch hits is the dense optimizer.
+ * sums_dev [R][rowp]: row r's sums at row r's offsets of the packed table (padding columns are never written);
+ * bias_sum_dev [1]; mlp_sums_dev [fmb_mlp_numel] (tower fit and fmb_online_deep_run_ex, NULL for FM-only steps).
+ * Entry points with a state slot (fmb_fm_step_fused_ex, fmb_fm_backward_runs_ex / _list, fmb_finish_step_ex) take it
+ * there in mode 3: pass (const fmb_ftrl_t*)&adagrad.  Algorithmic bytes of the FM step grow by 8F(k+1) per sample.
+ * Sharded steps, AFM and fmb_fm_backward_runs_all reject mode 3. */
+typedef struct fmb_adagrad_t { float* sums_dev; float* bias_sum_dev; float* mlp_sums_dev; float eps; } fmb_adagrad_t;
 int fmb_fm_step_fused_ex(const int32_t* ids_dev, const float* xv_dev, const float* y_dev, float* table_dev,
                          const float* bias_dev, const uint32_t* posflag_dev, int B, int F, int k, int loss_kind, float lr,
                          int mode, const fmb_ftrl_t* ftrl, float* delta_dev, float* lossv_dev, void* ws_dev,
@@ -230,6 +245,13 @@ int fmb_fm_backward_update_rl(const int32_t* sorted_keys_dev, const int32_t* per
                               const float* gs_dev, int gs_stride, int use_fm2, const float* gvec_dev, int32_t key_limit,
                               float lr, int mode, const fmb_runlist_t* rl, void* ws_dev, size_t ws_bytes,
                               fmb_stream_t stream);
+
+/* _rl_ex: update mode 3 needs `ada` (its sums_dev; NULL in the other modes) -- the tower fit's backward */
+int fmb_fm_backward_update_rl_ex(const int32_t* sorted_keys_dev, const int32_t* perm_dev, int64_t N, int64_t n_entries,
+                                 const float* xv_dev, float* table_dev, int F, int k, const float* S_dev, int s_pitch,
+                                 const float* gs_dev, int gs_stride, int use_fm2, const float* gvec_dev, int32_t key_limit,
+                                 float lr, int mode, const fmb_adagrad_t* ada, const fmb_runlist_t* rl, void* ws_dev,
+                                 size_t ws_bytes, fmb_stream_t stream);
 
 /* ---- row-sharded multi-GPU step (BASELINE.json configs[4]; no counterpart in the reference, which is
  * single-device: SURVEY.md 8e).  Row r lives on rank r % G at local row r / G.  See csrc/sharded.cu. */
@@ -400,6 +422,12 @@ int fmb_online_deep_run(int kind, const int32_t* ids_dev /*[N,F]*/, const float*
                         int F, int k, int L, int H, float* table_dev, float* bias_dev, float* mlp_dev,
                         float* alpha_dev, float* acc_dev /*[fmb_mlp_numel], ONN*/, float lr, float hb, float hs,
                         int mode, uint8_t* preds_dev, int64_t* conf_dev, fmb_stream_t stream);
+/* _ex: update mode 3 of kinds 0-2 reads and writes the sums of `ada` (table, bias and, with a tower, the tower's); the
+ * ONN kinds' hedge step uses no optimizer and ignores the mode.  fmb_online_deep_run rejects mode 3 for kinds 0-2. */
+int fmb_online_deep_run_ex(int kind, const int32_t* ids_dev, const float* xv_dev, const float* y_dev, int N, int F, int k,
+                           int L, int H, float* table_dev, float* bias_dev, float* mlp_dev, float* alpha_dev,
+                           float* acc_dev, float lr, float hb, float hs, int mode, const fmb_adagrad_t* ada,
+                           uint8_t* preds_dev, int64_t* conf_dev, fmb_stream_t stream);
 
 /* ---- A9-A11: classical fp64 online learners, one persistent launch per stream -------------------
  * fmb_ftrl_fm_run : FM_FTRL.online_learning (models/models_online/FM_FTRL.py:47-92)
@@ -440,6 +468,8 @@ int fmb_session_fm_step_host(fmb_session* s, const int32_t* ids_host, const floa
 int fmb_session_presort(fmb_session* s, const int32_t* ids_dev, int B, int key_bits);
 /* FTRL-Proximal state of the session's steps (update mode 2) */
 int fmb_session_set_ftrl(fmb_session* s, float* zn_dev, float* bias_zn_dev, float beta, float l1, float l2);
+/* Adagrad state of the session's steps (update mode 3): sums_dev [R][rowp], bias_sum_dev [1], filled by the caller */
+int fmb_session_set_adagrad(fmb_session* s, float* sums_dev, float* bias_sum_dev, float eps);
 /* forget a pending pre-sort (the caller cannot vouch that the pre-sorted ids buffer still holds the same batch) */
 void fmb_session_presort_invalidate(fmb_session* s);
 /* fmb_session_fm_step with the sort of the NEXT batch riding along: next_ids_dev (nullable) are the ids the
