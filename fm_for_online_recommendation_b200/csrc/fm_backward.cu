@@ -676,9 +676,7 @@ static int launch_runs_t(BwdParams& p, bool two, cudaStream_t stream) {
     if (per_sm < 1) per_sm = 1;
     if (per_sm * wpb > 32) per_sm = 32 / wpb;
     const unsigned nlong = (unsigned)sms;                                   // one long-run CTA per SM
-    static int short_per_sm = -1;      // experiment knob FMB_RUNS_SHORT_PER_SM (default: one slot less than fit)
-    if (short_per_sm < 0) { const char* e = getenv("FMB_RUNS_SHORT_PER_SM"); short_per_sm = e ? atoi(e) : 0; }
-    unsigned nshort = (unsigned)(sms * (short_per_sm > 0 ? short_per_sm : (per_sm > 1 ? per_sm - 1 : 1)));
+    unsigned nshort = (unsigned)(sms * (per_sm > 1 ? per_sm - 1 : 1));   // one slot less than fit
     if (nshort > grid) nshort = grid;
     if (p.pdl) {
         cudaLaunchConfig_t cfg;
@@ -803,15 +801,11 @@ struct fmb_ftrl_t { float* zn; float* bias_zn; float beta, l1, l2; };   // inclu
 
 // rl (nullable): the runs of >= 2 entries found by the sort one step ahead (fmb_sort_fields_ex / fmb_pos_flags_ex); with it
 // one warp is started per RUN instead of per 32 sorted positions.
-
-static thread_local int g_runs_pdl = 0;   // per calling thread: set and consumed by consecutive calls of one host thread
-// internal (session.cu): the NEXT fmb_fm_backward_runs_list call is launched as a programmatic dependent of the kernel
-// in front of it on its stream (the fused kernel, which executes griddepcontrol.launch_dependents)
-FMB_API void fmb_runs_list_next_is_dependent(int on) { g_runs_pdl = on; }
-
-FMB_API int fmb_fm_backward_runs_list(const int32_t* sorted_keys, int64_t N, float* table, int F, int k, float lr,
-                                      int mode, const fmb_ftrl_t* ftrl, const fmb_runlist_t* rl,
-                                      void* ws, size_t ws_bytes, cudaStream_t stream) {
+// pdl (internal, session.cu): with a run list, launch the kernel as a programmatic dependent of the kernel in front of it
+// on its stream (the fused kernel, which executes griddepcontrol.launch_dependents)
+int fmb_fm_backward_runs_list_launch(const int32_t* sorted_keys, int64_t N, float* table, int F, int k, float lr, int mode,
+                                     const fmb_ftrl_t* ftrl, const fmb_runlist_t* rl, void* ws, size_t ws_bytes, bool pdl,
+                                     cudaStream_t stream) {
     FMB_CHECK_ARG(sorted_keys && table && ws, "fmb_fm_backward_runs: null pointer");
     FMB_CHECK_ARG(!rl || (rl->entries && rl->seg_count && rl->nseg >= 1 && rl->nseg <= 2048 && rl->seg_cap >= 1),
                   "fmb_fm_backward_runs: bad run list");
@@ -836,10 +830,15 @@ FMB_API int fmb_fm_backward_runs_list(const int32_t* sorted_keys, int64_t N, flo
         p.ada.sums = a->sums; p.ada.bias_sum = a->bias_sum; p.ada.eps = a->eps;
     }
     if (rl) { p.run_list = reinterpret_cast<const int4*>(rl->entries); p.run_segc = rl->seg_count; p.run_nseg = rl->nseg; p.run_cap = rl->seg_cap; }
-    p.pdl = rl ? g_runs_pdl : 0;
-    g_runs_pdl = 0;
+    p.pdl = rl && pdl;
     p.dbg = g_runs_dbg;
     return launch_runs(p, false, stream);
+}
+
+FMB_API int fmb_fm_backward_runs_list(const int32_t* sorted_keys, int64_t N, float* table, int F, int k, float lr,
+                                      int mode, const fmb_ftrl_t* ftrl, const fmb_runlist_t* rl,
+                                      void* ws, size_t ws_bytes, cudaStream_t stream) {
+    return fmb_fm_backward_runs_list_launch(sorted_keys, N, table, F, k, lr, mode, ftrl, rl, ws, ws_bytes, false, stream);
 }
 
 FMB_API int fmb_fm_backward_runs_ex(const int32_t* sorted_keys, int64_t N, float* table, int F, int k, float lr,

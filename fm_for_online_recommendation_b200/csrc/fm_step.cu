@@ -411,7 +411,6 @@ FMB_API int fmb_is_fused_kernel_fn(const void* fn) {
                 if (fn == (const void*)fused_fn(c ? 3 : 0, x != 0, m)) return 1;
     return 0;
 }
-FMB_API const void* fmb_pos_flags_kernel_fn(void) { return (const void*)pos_flags_kernel; }
 
 // per-entry sorted position + multi-hit flag from the stable sort's output (fmb_sort_fields / fmb_sort_segment);
 // _ex: also the run list for fmb_fm_backward_runs_list, as ONE segment (rl->nseg == 1, seg_cap >= N/2) whose counters
@@ -481,11 +480,6 @@ FMB_API int fmb_fm_step_fused_ex(const int32_t* ids, const float* xv, const floa
     // 16-sample tiles; the kernel is latency-bound (55 % "no eligible warp" at B = 65 536 with 16-sample tiles,
     // profiles/r2_final3_fused_ncu_summary.txt): measured 158.0 vs 164.1 us per launch and 363 vs 391 us per step there
     while (SB > 8) SB >>= 1;
-    {   // experiment knob: FMB_STEP_SB caps the samples per tile
-        static int cap = -1;
-        if (cap < 0) { const char* e = getenv("FMB_STEP_SB"); cap = e ? atoi(e) : 0; }
-        if (cap > 0 && SB > cap) SB = cap;
-    }
     FMB_CHECK_ARG(bytes(SB) <= 200 * 1024, "fmb_fm_step_fused: F*k too large for one sample tile (F=%d k=%d: %zu bytes > 200 KB)",
                   F, k, bytes(SB));
     p.SB = SB;

@@ -11,8 +11,6 @@
 #include <new>
 
 extern "C" {
-int fmb_fm_forward(const int32_t*, const float*, const float*, const float*, int, int, int, float*, float*, float*,
-                   float*, float*, const float*, int, float*, float*, cudaStream_t);
 size_t fmb_sort_workspace_bytes(int64_t);
 int fmb_sort_segment(const int32_t*, int64_t, int, void*, size_t, int32_t*, int32_t*, int32_t*, int32_t*,
                      cudaStream_t);
@@ -22,27 +20,17 @@ struct fmb_runlist_t { int32_t* entries; uint32_t* seg_count; int nseg, seg_cap;
 void fmb_runlist_shape(int, int, int*, int*);
 int fmb_sort_fields_ex(const int32_t*, int, int, const int32_t*, int32_t*, int32_t*, uint32_t*, const fmb_runlist_t*, int, cudaStream_t);
 int fmb_pos_flags_ex(const int32_t*, const int32_t*, int64_t, uint32_t*, const fmb_runlist_t*, cudaStream_t);
-int fmb_fm_backward_update(const int32_t*, const int32_t*, int64_t, const float*, float*, int, int, const float*,
-                           const float*, int, const float*, float, int, void*, size_t, cudaStream_t);
-int fmb_finish_step(const float*, const float*, int, float*, float, int, float*, cudaStream_t);
 struct fmb_ftrl_t { float* zn; float* bias_zn; float beta, l1, l2; };
 struct fmb_adagrad_t { float* sums; float* bias_sum; float* mlp_sums; float eps; };
-int fmb_fm_backward_runs_list(const int32_t*, int64_t, float*, int, int, float, int, const fmb_ftrl_t*, const fmb_runlist_t*,
-                              void*, size_t, cudaStream_t);
 int fmb_finish_step_ex(const float*, const float*, int, float*, float, int, const fmb_ftrl_t*, float*, cudaStream_t);
 int fmb_fm_step_fused_ex(const int32_t*, const float*, const float*, float*, const float*, const uint32_t*, int, int, int,
                          int, float, int, const fmb_ftrl_t*, float*, float*, void*, size_t, cudaStream_t);
-int fmb_fm_backward_runs_ex(const int32_t*, int64_t, float*, int, int, float, int, const fmb_ftrl_t*, void*, size_t,
-                            cudaStream_t);
-int fmb_pos_flags(const int32_t*, const int32_t*, int64_t, uint32_t*, cudaStream_t);
-int fmb_fm_step_fused(const int32_t*, const float*, const float*, float*, const float*, const uint32_t*, int, int, int,
-                      int, float, int, float*, float*, void*, size_t, cudaStream_t);
-int fmb_fm_backward_runs(const int32_t*, int64_t, float*, int, int, float, int, void*, size_t, cudaStream_t);
 int fmb_is_fused_kernel_fn(const void*);
-void fmb_runs_list_next_is_dependent(int);
 const void* fmb_finish_kernel_fn(void);
 int fmb_sort_fields_kernel_fns(const void**, int*, int*);
 }
+int fmb_fm_backward_runs_list_launch(const int32_t*, int64_t, float*, int, int, float, int, const fmb_ftrl_t*,
+                                     const fmb_runlist_t*, void*, size_t, bool pdl, cudaStream_t);   // fm_backward.cu
 
 // One captured step graph per CONFIGURATION (batch size, loss, update mode, with/without xv, sorted in the step or
 // before it, with/without the sort of the next batch riding along) -- never per batch: the per-batch pointers
@@ -63,13 +51,20 @@ struct StepVariant {
     const void *cur_ids, *cur_xv, *cur_y, *cur_sort_ids, *cur_next_ids, *cur_loss;
 };
 
+// One input slot of the host entry points: device buffers for one batch, the pinned staging area pageable inputs are
+// copied through, and the pinned word the step's mean loss lands in
+struct HostSlot {
+    int32_t* d_ids; float* d_xv; float* d_y;
+    int32_t* h_ids; float* h_xv; float* h_y;
+    float* h_loss;                 // into one pinned block shared by the four slots, 32 bytes apart (owned by slot 0)
+    cudaEvent_t ev_h2d, ev_done;   // this slot's inputs have landed / its step has finished
+    bool used;
+};
+
 struct fmb_session {
     int F, k, rowp, kp4;
     int64_t maxB;
     // device
-    int32_t* d_ids;
-    float* d_xv;
-    float* d_y;
     float* d_S;
     float* d_z;
     float* d_delta;
@@ -97,20 +92,11 @@ struct fmb_session {
     void* d_bwd_ws;
     size_t bwd_ws_bytes;
     int32_t* d_field_off;  // [F+1] global row offset of every field (enables the per-field sort)
-    // pinned host staging
-    int32_t* h_ids;
-    float* h_xv;
-    float* h_y;
-    float* h_loss;
-    // second input slot + copy stream for the pipelined host entry point (slot 0 = the buffers above)
-    int32_t* d_ids2; float* d_xv2; float* d_y2; float* d_loss2;
-    int32_t* h_ids2; float* h_xv2; float* h_y2;
-    // slots 2 and 3 (allocated on first use): with four slots the host runs up to three steps ahead of the GPU
-    int32_t* d_idsx[2]; float* d_xvx[2]; float* d_yx[2];
-    int32_t* h_idsx[2]; float* h_xvx[2]; float* h_yx[2];
+    // input slots of the host entry points (slot 0 allocated with the session: fmb_session_fm_step_host stages through
+    // it; slots 1-3 on first use) and the copy stream of the pipelined one: with four slots the host runs up to three
+    // steps ahead of the GPU
+    HostSlot slot[4];
     cudaStream_t st_copy;
-    cudaEvent_t ev_h2d[4], ev_done[4];
-    int slot_used[4];
     int64_t launches;  // kernels launched through this session (bench.py's gpu_launches)
     // CUDA-graph cache of whole steps, keyed by every argument that is baked into the kernels
     cudaStream_t st0, st1, st2, st3, st4;   // st0/st1: graph capture (main / side branch); st2: pre-sorts; st3: sparse-field
@@ -119,9 +105,6 @@ struct fmb_session {
     int64_t steps_done;
     cudaEvent_t ev_fork, ev_fwd, ev_sort, ev_join;
     int use_graph, use_prio;
-    int host_path;         // set while fmb_session_fm_step_host_async runs its step (one graph per input slot)
-    int use_pdl;           // FMB_PDL=0 switches the programmatic dependent launch of the run kernel off
-    int sort_after;        // FMB_SORT_AFTER=1 (experiment; default 0): the next batch's sort waits for the fused kernel
     int sparse_ok;         // FMB_SORT_SPARSE_OK unless FMB_SPARSE=0: fields with >= 16*B rows skip the sort (radix_sort.cu)
     int ngraphs, next_evict;
     StepVariant gvar[FMB_GRAPH_CACHE];
@@ -143,7 +126,7 @@ struct fmb_session {
 
 FMB_API void fmb_session_destroy(fmb_session* s) {
     if (!s) return;
-    cudaFree(s->d_ids); cudaFree(s->d_xv); cudaFree(s->d_y); cudaFree(s->d_S); cudaFree(s->d_z);
+    cudaFree(s->d_S); cudaFree(s->d_z);
     cudaFree(s->d_delta); cudaFree(s->d_lossv); cudaFree(s->d_loss);
     for (int i = 0; i < 2; ++i) { cudaFree(s->d_skeys_buf[i]); cudaFree(s->d_perm_buf[i]); cudaFree(s->d_posflag_buf[i]); cudaFree(s->d_runlist_buf[i]); cudaFree(s->d_runcount_buf[i]); if (s->ev_buf_free[i]) cudaEventDestroy(s->ev_buf_free[i]); }
     cudaFree(s->d_sort_ws2);
@@ -156,15 +139,14 @@ FMB_API void fmb_session_destroy(fmb_session* s) {
     if (s->ev_join4) cudaEventDestroy(s->ev_join4);
     if (s->ev_presort) cudaEventDestroy(s->ev_presort);
     cudaFree(s->d_sort_ws); cudaFree(s->d_bwd_ws); cudaFree(s->d_field_off);
-    cudaFreeHost(s->h_ids); cudaFreeHost(s->h_xv); cudaFreeHost(s->h_y); cudaFreeHost(s->h_loss);
-    cudaFree(s->d_ids2); cudaFree(s->d_xv2); cudaFree(s->d_y2); cudaFree(s->d_loss2);
-    cudaFreeHost(s->h_ids2); cudaFreeHost(s->h_xv2); cudaFreeHost(s->h_y2);
-    if (s->st_copy) cudaStreamDestroy(s->st_copy);
-    for (int i = 0; i < 4; ++i) { if (s->ev_h2d[i]) cudaEventDestroy(s->ev_h2d[i]); if (s->ev_done[i]) cudaEventDestroy(s->ev_done[i]); }
-    for (int i = 0; i < 2; ++i) {
-        cudaFree(s->d_idsx[i]); cudaFree(s->d_xvx[i]); cudaFree(s->d_yx[i]);
-        cudaFreeHost(s->h_idsx[i]); cudaFreeHost(s->h_xvx[i]); cudaFreeHost(s->h_yx[i]);
+    for (HostSlot& h : s->slot) {
+        cudaFree(h.d_ids); cudaFree(h.d_xv); cudaFree(h.d_y);
+        cudaFreeHost(h.h_ids); cudaFreeHost(h.h_xv); cudaFreeHost(h.h_y);
+        if (h.ev_h2d) cudaEventDestroy(h.ev_h2d);
+        if (h.ev_done) cudaEventDestroy(h.ev_done);
     }
+    cudaFreeHost(s->slot[0].h_loss);
+    if (s->st_copy) cudaStreamDestroy(s->st_copy);
     for (int i = 0; i < s->ngraphs; ++i) { cudaGraphExecDestroy(s->gvar[i].exec); cudaGraphDestroy(s->gvar[i].graph); }
     if (s->st0) cudaStreamDestroy(s->st0);
     if (s->st1) cudaStreamDestroy(s->st1);
@@ -174,6 +156,19 @@ FMB_API void fmb_session_destroy(fmb_session* s) {
     if (s->ev_sort) cudaEventDestroy(s->ev_sort);
     if (s->ev_join) cudaEventDestroy(s->ev_join);
     delete s;
+}
+
+// device buffers, pinned staging and events of one input slot for batches of up to maxB samples (what exists is kept)
+static cudaError_t slot_alloc(const fmb_session* s, HostSlot& h) {
+    const size_t N = (size_t)s->maxB * s->F;
+    cudaError_t e = cudaSuccess;
+    auto dm = [&](void** p, size_t n) { if (e == cudaSuccess && !*p) e = cudaMalloc(p, n); };
+    auto hm = [&](void** p, size_t n) { if (e == cudaSuccess && !*p) e = cudaMallocHost(p, n); };
+    auto ev = [&](cudaEvent_t* p) { if (e == cudaSuccess && !*p) e = cudaEventCreateWithFlags(p, cudaEventDisableTiming); };
+    dm((void**)&h.d_ids, N * 4); dm((void**)&h.d_xv, N * 4); dm((void**)&h.d_y, (size_t)s->maxB * 4);
+    hm((void**)&h.h_ids, N * 4); hm((void**)&h.h_xv, N * 4); hm((void**)&h.h_y, (size_t)s->maxB * 4);
+    ev(&h.ev_h2d); ev(&h.ev_done);
+    return e;
 }
 
 // F fields, embedding size k, up to max_batch samples per step.  field_off_host [F+1] (nullable):
@@ -194,23 +189,19 @@ FMB_API int fmb_session_create(fmb_session** out, int F, int k, int64_t max_batc
     cudaError_t e = cudaSuccess;
     auto dm = [&](void** p, size_t n) { if (e == cudaSuccess) e = cudaMalloc(p, n); };
     auto hm = [&](void** p, size_t n) { if (e == cudaSuccess) e = cudaMallocHost(p, n); };
-    dm((void**)&s->d_ids, N * 4); dm((void**)&s->d_xv, N * 4); dm((void**)&s->d_y, max_batch * 4);
+    // slot 0 first: allocated after the workspaces below it moves where they land, and the cfg5 step then measured
+    // 40.1 instead of 39.4 us (B200, 1 000 W power limit)
+    e = slot_alloc(s, s->slot[0]);
     dm((void**)&s->d_S, max_batch * s->kp4 * 4); dm((void**)&s->d_z, max_batch * 4);
     dm((void**)&s->d_delta, max_batch * 4); dm((void**)&s->d_lossv, max_batch * 4); dm((void**)&s->d_loss, 256);
     for (int i = 0; i < 2; ++i) { dm((void**)&s->d_skeys_buf[i], N * 4); dm((void**)&s->d_perm_buf[i], N * 4); dm((void**)&s->d_posflag_buf[i], N * 4); dm((void**)&s->d_runlist_buf[i], (size_t)s->rl_nseg * s->rl_cap * 16); dm((void**)&s->d_runcount_buf[i], (size_t)s->rl_nseg * 8 + 256); }
     if (!(field_off_host && max_batch <= fmb_sort_fields_max_batch())) dm(&s->d_sort_ws2, s->sort_ws_bytes);
     s->d_skeys = s->d_skeys_buf[0]; s->d_perm = s->d_perm_buf[0];
     dm(&s->d_sort_ws, s->sort_ws_bytes); dm(&s->d_bwd_ws, s->bwd_ws_bytes);
-    hm((void**)&s->h_ids, N * 4); hm((void**)&s->h_xv, N * 4); hm((void**)&s->h_y, max_batch * 4);
-    hm((void**)&s->h_loss, 256);
-    dm((void**)&s->d_ids2, N * 4); dm((void**)&s->d_xv2, N * 4); dm((void**)&s->d_y2, max_batch * 4);
-    dm((void**)&s->d_loss2, 256);
-    hm((void**)&s->h_ids2, N * 4); hm((void**)&s->h_xv2, N * 4); hm((void**)&s->h_y2, max_batch * 4);
+    hm((void**)&s->slot[0].h_loss, 256);
+    if (e == cudaSuccess)
+        for (int i = 1; i < 4; ++i) s->slot[i].h_loss = s->slot[0].h_loss + 8 * i;
     if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&s->st_copy, cudaStreamNonBlocking);
-    for (int i = 0; i < 4; ++i) {
-        if (e == cudaSuccess) e = cudaEventCreateWithFlags(&s->ev_h2d[i], cudaEventDisableTiming);
-        if (e == cudaSuccess) e = cudaEventCreateWithFlags(&s->ev_done[i], cudaEventDisableTiming);
-    }
     if (field_off_host) {
         dm((void**)&s->d_field_off, (size_t)(F + 1) * 4);
         if (e == cudaSuccess) e = cudaMemcpy(s->d_field_off, field_off_host, (size_t)(F + 1) * 4, cudaMemcpyHostToDevice);
@@ -221,18 +212,14 @@ FMB_API int fmb_session_create(fmb_session** out, int F, int k, int64_t max_batc
         // every thread slot of the GPU; launched first they kept the sort's 156 clustered CTAs waiting until the first
         // tiles retired (~20 us: the step took sort + 20 us whatever the fused kernel cost).  With priority the sort's
         // CTAs are placed first (one per SM), the tiles take the remaining seven slots, and both chains start together.
-        // FMB_PRIO=0: no priorities; FMB_PRIO=2: the other way round (for comparison).
-        int least = 0, greatest = 0;
-        const char* pe = getenv("FMB_PRIO");
-        s->use_prio = pe ? atoi(pe) : 1;
-        if (s->use_prio && cudaDeviceGetStreamPriorityRange(&least, &greatest) != cudaSuccess) s->use_prio = 0;
-        if (!s->use_prio) least = greatest = 0;
-        if (s->use_prio == 1) { const int t = least; least = greatest; greatest = t; }   // st0/st1 low, st2 high
-        if (e == cudaSuccess) e = cudaStreamCreateWithPriority(&s->st0, cudaStreamNonBlocking, greatest);
-        if (e == cudaSuccess) e = cudaStreamCreateWithPriority(&s->st1, cudaStreamNonBlocking, greatest);
-        if (e == cudaSuccess) e = cudaStreamCreateWithPriority(&s->st2, cudaStreamNonBlocking, least);
-        if (e == cudaSuccess) e = cudaStreamCreateWithPriority(&s->st3, cudaStreamNonBlocking, least);
-        if (e == cudaSuccess) e = cudaStreamCreateWithPriority(&s->st4, cudaStreamNonBlocking, greatest);
+        int low = 0, high = 0;
+        s->use_prio = cudaDeviceGetStreamPriorityRange(&low, &high) == cudaSuccess;
+        if (!s->use_prio) low = high = 0;
+        if (e == cudaSuccess) e = cudaStreamCreateWithPriority(&s->st0, cudaStreamNonBlocking, low);
+        if (e == cudaSuccess) e = cudaStreamCreateWithPriority(&s->st1, cudaStreamNonBlocking, low);
+        if (e == cudaSuccess) e = cudaStreamCreateWithPriority(&s->st2, cudaStreamNonBlocking, high);
+        if (e == cudaSuccess) e = cudaStreamCreateWithPriority(&s->st3, cudaStreamNonBlocking, high);
+        if (e == cudaSuccess) e = cudaStreamCreateWithPriority(&s->st4, cudaStreamNonBlocking, low);
         if (e == cudaSuccess) e = cudaEventCreateWithFlags(&s->ev_join4, cudaEventDisableTiming);
         if (e == cudaSuccess) e = cudaEventCreateWithFlags(&s->ev_sp_fork, cudaEventDisableTiming);
         if (e == cudaSuccess) e = cudaEventCreateWithFlags(&s->ev_sp_join, cudaEventDisableTiming);
@@ -249,10 +236,6 @@ FMB_API int fmb_session_create(fmb_session** out, int F, int k, int64_t max_batc
         s->use_graph = !(ng && ng[0] == '1');
         const char* sp = getenv("FMB_SPARSE");
         s->sparse_ok = !(sp && sp[0] == '0');
-        const char* pd = getenv("FMB_PDL");
-        s->use_pdl = !(pd && pd[0] == '0');
-        const char* sa = getenv("FMB_SORT_AFTER");
-        s->sort_after = sa && sa[0] == '1';
     }
     if (e != cudaSuccess) {
         fmb_set_error("fmb_session_create: %s", cudaGetErrorString(e));
@@ -346,7 +329,7 @@ static int fm_step_launch(fmb_session* s, const int32_t* ids, const float* xv, c
     *nlaunch = 0;
     cudaEventRecord(s->ev_fork, main);
     cudaStreamWaitEvent(side, s->ev_fork, 0);
-    if (next_ids && !s->sort_after) {
+    if (next_ids) {   // forked at the top: started behind the fused kernel, the sort chain ends after the run kernel (DESIGN.md §3)
         cudaStreamWaitEvent(side2, s->ev_fork, 0);
         rc = sort_launch(s, next_ids, B, key_bits, 1 - cur, s->d_sort_ws2, side2, nlaunch);
         if (rc) return rc;
@@ -364,16 +347,6 @@ static int fm_step_launch(fmb_session* s, const int32_t* ids, const float* xv, c
     if (rc) return rc;
     cudaEventRecord(s->ev_fwd, main);
     cudaStreamWaitEvent(side, s->ev_fwd, 0);
-    if (next_ids && s->sort_after) {
-        // Experiment (FMB_SORT_AFTER=1): the sort of the NEXT batch starts when the fused kernel is done and runs beside
-        // the run kernel and the bias step.  The fused kernel then takes 19 us instead of 26-33 (the sort's CTAs no longer
-        // keep its 1 024 tiles from being resident at once), but the sort chain (~20 us) ends after the run kernel:
-        // 51.8 us per step against 42.7 with the sort started at the top of the graph.
-        cudaStreamWaitEvent(side2, s->ev_fwd, 0);
-        rc = sort_launch(s, next_ids, B, key_bits, 1 - cur, s->d_sort_ws2, side2, nlaunch);
-        if (rc) return rc;
-        cudaEventRecord(s->ev_join2, side2);
-    }
     rc = fmb_finish_step_ex(s->d_delta, s->d_lossv, B, bias, lr, mode, ft, loss_dev ? loss_dev : s->d_loss, side);
     if (rc) return rc;
     cudaEventRecord(s->ev_join, side);
@@ -381,8 +354,8 @@ static int fm_step_launch(fmb_session* s, const int32_t* ids, const float* xv, c
     rl.entries = s->d_runlist_buf[cur]; rl.seg_count = s->d_runcount_buf[cur];
     if (by_field_sort(s, B)) fmb_runlist_shape(B, s->F, &rl.nseg, &rl.seg_cap);
     else { rl.nseg = 1; rl.seg_cap = (int)(N / 2 + 1); }
-    fmb_runs_list_next_is_dependent(s->use_pdl);
-    rc = fmb_fm_backward_runs_list(s->d_skeys_buf[cur], N, table, s->F, s->k, lr, mode, ft, &rl, s->d_bwd_ws, s->bwd_ws_bytes, main);
+    rc = fmb_fm_backward_runs_list_launch(s->d_skeys_buf[cur], N, table, s->F, s->k, lr, mode, ft, &rl, s->d_bwd_ws,
+                                          s->bwd_ws_bytes, /*pdl=*/true, main);
     if (rc) return rc;
     cudaStreamWaitEvent(main, s->ev_join, 0);
     if (next_ids) cudaStreamWaitEvent(main, s->ev_join2, 0);
@@ -461,9 +434,11 @@ static int capture_variant(fmb_session* s, StepVariant* v, const int32_t* ids, c
 //   rides along on a side branch of this step, and the next call -- recognised by its ids pointer -- skips its own.
 // The step replays a CUDA graph captured once per configuration and re-pointed at this call's batch;
 // FMB_NO_GRAPH=1 (and batches too large for the per-field sort) launch the kernels directly.
-FMB_API int fmb_session_fm_step_next(fmb_session* s, const int32_t* ids, const float* xv, const float* y, int B,
-                                     float* table, float* bias, int key_bits, int loss_kind, float lr, int mode,
-                                     const int32_t* next_ids, float* loss_dev, cudaStream_t stream) {
+//   graph_per_input: graphs of one configuration are kept one per set of per-batch pointers, up to four, before the first
+//   one is re-pointed (the host entry point's four input slots then replay their graphs without re-pointing a node).
+static int session_fm_step(fmb_session* s, const int32_t* ids, const float* xv, const float* y, int B, float* table,
+                           float* bias, int key_bits, int loss_kind, float lr, int mode, const int32_t* next_ids,
+                           float* loss_dev, cudaStream_t stream, bool graph_per_input) {
     FMB_CHECK_ARG(s && ids && y && table && bias, "fmb_session_fm_step: null pointer");
     FMB_CHECK_ARG(B > 0 && B <= s->maxB, "fmb_session_fm_step: B=%d exceeds session max_batch", B);
     int nl = 0;
@@ -493,19 +468,20 @@ FMB_API int fmb_session_fm_step_next(fmb_session* s, const int32_t* ids, const f
         memset(&key, 0, sizeof(key));
         key.B = B; key.key_bits = key_bits; key.loss_kind = loss_kind; key.mode = mode; key.has_xv = xv != nullptr;
         key.pre = pre; key.has_next = next_ids != nullptr; key.cur = cur; key.table = table; key.bias = bias; key.lr = lr;
-        StepVariant* v = nullptr;
         const size_t keylen = offsetof(StepVariant, graph);
-        // Several graphs may share a key: one per set of per-batch pointers, up to four (the host entry point's four
-        // input slots replay their graphs without re-pointing a node); beyond that the first one is re-pointed.
+        // a graph of this configuration that already holds this call's pointers; else, unless graph_per_input asks for
+        // one more graph while fewer than four share the key, the first one of the configuration (re-pointed below)
         float* want_loss = loss_dev ? loss_dev : s->d_loss;
-        int same_key = 0;
-        for (int i = 0; i < s->ngraphs; ++i)
-            if (memcmp(&s->gvar[i], &key, keylen) == 0) {
-                ++same_key;
-                if (!v) v = &s->gvar[i];
-                if (s->gvar[i].cur_ids == ids && s->gvar[i].cur_y == y && s->gvar[i].cur_loss == want_loss) { v = &s->gvar[i]; same_key = 99; break; }
-            }
-        if (v && same_key < 4 && s->host_path) v = nullptr;     // host path: capture one more instead of re-pointing
+        StepVariant *same = nullptr, *first = nullptr;
+        int nkey = 0;
+        for (int i = 0; i < s->ngraphs && !same; ++i) {
+            StepVariant* g = &s->gvar[i];
+            if (memcmp(g, &key, keylen) != 0) continue;
+            ++nkey;
+            if (!first) first = g;
+            if (g->cur_ids == ids && g->cur_y == y && g->cur_loss == want_loss) same = g;
+        }
+        StepVariant* v = same ? same : (graph_per_input && nkey < 4) ? nullptr : first;
         if (!v) {
             rc = capture_variant(s, &key, ids, xv, y, table, bias, next_ids);
             if (rc) return rc;
@@ -566,6 +542,12 @@ FMB_API int fmb_session_fm_step_next(fmb_session* s, const int32_t* ids, const f
     }
     s->steps_done += 1;
     return FMB_OK;
+}
+
+FMB_API int fmb_session_fm_step_next(fmb_session* s, const int32_t* ids, const float* xv, const float* y, int B,
+                                     float* table, float* bias, int key_bits, int loss_kind, float lr, int mode,
+                                     const int32_t* next_ids, float* loss_dev, cudaStream_t stream) {
+    return session_fm_step(s, ids, xv, y, B, table, bias, key_bits, loss_kind, lr, mode, next_ids, loss_dev, stream, false);
 }
 
 FMB_API int fmb_session_fm_step(fmb_session* s, const int32_t* ids, const float* xv, const float* y, int B,
@@ -656,50 +638,32 @@ FMB_API int fmb_session_fm_step_host_async(fmb_session* s, int slot, const int32
     FMB_CHECK_ARG(slot >= 0 && slot < 4, "fmb_session_fm_step_host_async: slot must be 0..3");
     FMB_CHECK_ARG(B > 0 && B <= s->maxB, "fmb_session_fm_step_host_async: B=%d exceeds session max_batch", B);
     const size_t N = (size_t)B * s->F;
-    if (slot >= 2 && !s->d_idsx[slot - 2]) {     // slots 2 and 3: buffers on first use
-        const size_t NN = (size_t)s->maxB * s->F;
-        const int j = slot - 2;
-        cudaError_t e = cudaMalloc((void**)&s->d_idsx[j], NN * 4);
-        if (e == cudaSuccess) e = cudaMalloc((void**)&s->d_xvx[j], NN * 4);
-        if (e == cudaSuccess) e = cudaMalloc((void**)&s->d_yx[j], (size_t)s->maxB * 4);
-        if (e == cudaSuccess) e = cudaMallocHost((void**)&s->h_idsx[j], NN * 4);
-        if (e == cudaSuccess) e = cudaMallocHost((void**)&s->h_xvx[j], NN * 4);
-        if (e == cudaSuccess) e = cudaMallocHost((void**)&s->h_yx[j], (size_t)s->maxB * 4);
-        if (e != cudaSuccess) { fmb_set_error("fmb_session_fm_step_host_async: %s", cudaGetErrorString(e)); return FMB_ERR_CUDA; }
-    }
-    int32_t* d_ids = slot >= 2 ? s->d_idsx[slot - 2] : (slot ? s->d_ids2 : s->d_ids);
-    float* d_xv = slot >= 2 ? s->d_xvx[slot - 2] : (slot ? s->d_xv2 : s->d_xv);
-    float* d_y = slot >= 2 ? s->d_yx[slot - 2] : (slot ? s->d_y2 : s->d_y);
-    float* d_loss = slot ? s->d_loss2 : s->d_loss;
-    int32_t* h_ids = slot >= 2 ? s->h_idsx[slot - 2] : (slot ? s->h_ids2 : s->h_ids);
-    float* h_xv = slot >= 2 ? s->h_xvx[slot - 2] : (slot ? s->h_xv2 : s->h_xv);
-    float* h_y = slot >= 2 ? s->h_yx[slot - 2] : (slot ? s->h_y2 : s->h_y);
-    // the previous user of this slot (two steps ago) must be done with the device buffers and the staging area
-    if (s->slot_used[slot]) CU(cudaEventSynchronize(s->ev_done[slot]));
+    HostSlot& h = s->slot[slot];
+    const cudaError_t e = slot_alloc(s, h);   // slots 1-3: buffers on first use
+    if (e != cudaSuccess) { fmb_set_error("fmb_session_fm_step_host_async: %s", cudaGetErrorString(e)); return FMB_ERR_CUDA; }
+    // the previous step on this slot must be done with the device buffers and the staging area
+    if (h.used) CU(cudaEventSynchronize(h.ev_done));
     const void* src_ids = ids_host;
     const void* src_y = y_host;
     const void* src_xv = xv_host;
-    if (!host_ptr_is_pinned(ids_host)) { memcpy(h_ids, ids_host, N * 4); src_ids = h_ids; }
-    if (!host_ptr_is_pinned(y_host)) { memcpy(h_y, y_host, (size_t)B * 4); src_y = h_y; }
-    if (xv_host && !host_ptr_is_pinned(xv_host)) { memcpy(h_xv, xv_host, N * 4); src_xv = h_xv; }
-    CU(cudaMemcpyAsync(d_ids, src_ids, N * 4, cudaMemcpyHostToDevice, s->st_copy));
-    CU(cudaMemcpyAsync(d_y, src_y, (size_t)B * 4, cudaMemcpyHostToDevice, s->st_copy));
-    if (xv_host) CU(cudaMemcpyAsync(d_xv, src_xv, N * 4, cudaMemcpyHostToDevice, s->st_copy));
-    CU(cudaEventRecord(s->ev_h2d[slot], s->st_copy));
-    CU(cudaStreamWaitEvent(stream, s->ev_h2d[slot], 0));
+    if (!host_ptr_is_pinned(ids_host)) { memcpy(h.h_ids, ids_host, N * 4); src_ids = h.h_ids; }
+    if (!host_ptr_is_pinned(y_host)) { memcpy(h.h_y, y_host, (size_t)B * 4); src_y = h.h_y; }
+    if (xv_host && !host_ptr_is_pinned(xv_host)) { memcpy(h.h_xv, xv_host, N * 4); src_xv = h.h_xv; }
+    CU(cudaMemcpyAsync(h.d_ids, src_ids, N * 4, cudaMemcpyHostToDevice, s->st_copy));
+    CU(cudaMemcpyAsync(h.d_y, src_y, (size_t)B * 4, cudaMemcpyHostToDevice, s->st_copy));
+    if (xv_host) CU(cudaMemcpyAsync(h.d_xv, src_xv, N * 4, cudaMemcpyHostToDevice, s->st_copy));
+    CU(cudaEventRecord(h.ev_h2d, s->st_copy));
+    CU(cudaStreamWaitEvent(stream, h.ev_h2d, 0));
     // the sort of this batch starts as soon as its ids have landed: it overlaps the step still in flight
-    int rc = presort_impl(s, d_ids, B, key_bits, s->ev_h2d[slot]);
+    int rc = presort_impl(s, h.d_ids, B, key_bits, h.ev_h2d);
     if (rc) return rc;
     // the bias-step kernel writes the mean loss straight into the pinned result word (4 bytes over PCIe: the D2H of the
     // step, without a copy operation of its own)
-    (void)d_loss;
-    s->host_path = 1;
-    rc = fmb_session_fm_step(s, d_ids, xv_host ? d_xv : nullptr, d_y, B, table, bias, key_bits, loss_kind, lr,
-                                 mode, s->h_loss + 8 * slot, stream);
-    s->host_path = 0;
+    rc = session_fm_step(s, h.d_ids, xv_host ? h.d_xv : nullptr, h.d_y, B, table, bias, key_bits, loss_kind, lr, mode,
+                         nullptr, h.h_loss, stream, /*graph_per_input=*/true);
     if (rc) return rc;
-    CU(cudaEventRecord(s->ev_done[slot], stream));
-    s->slot_used[slot] = 1;
+    CU(cudaEventRecord(h.ev_done, stream));
+    h.used = true;
     return FMB_OK;
 }
 
@@ -708,9 +672,9 @@ FMB_API int fmb_session_host_slots(void) { return 4; }
 
 // waits for the step last submitted on `slot` and returns its mean loss
 FMB_API int fmb_session_wait_loss(fmb_session* s, int slot, float* loss_host) {
-    FMB_CHECK_ARG(s && slot >= 0 && slot < 4 && s->slot_used[slot], "fmb_session_wait_loss: nothing submitted on slot %d", slot);
-    CU(cudaEventSynchronize(s->ev_done[slot]));
-    if (loss_host) *loss_host = s->h_loss[8 * slot];
+    FMB_CHECK_ARG(s && slot >= 0 && slot < 4 && s->slot[slot].used, "fmb_session_wait_loss: nothing submitted on slot %d", slot);
+    CU(cudaEventSynchronize(s->slot[slot].ev_done));
+    if (loss_host) *loss_host = *s->slot[slot].h_loss;
     return FMB_OK;
 }
 
@@ -723,19 +687,20 @@ FMB_API int fmb_session_fm_step_host(fmb_session* s, const int32_t* ids_host, co
     FMB_CHECK_ARG(s && ids_host && y_host && table && bias, "fmb_session_fm_step_host: null pointer");
     FMB_CHECK_ARG(B > 0 && B <= s->maxB, "fmb_session_fm_step_host: B=%d exceeds session max_batch", B);
     const size_t N = (size_t)B * s->F;
-    memcpy(s->h_ids, ids_host, N * 4);
-    memcpy(s->h_y, y_host, (size_t)B * 4);
-    CU(cudaMemcpyAsync(s->d_ids, s->h_ids, N * 4, cudaMemcpyHostToDevice, stream));
-    CU(cudaMemcpyAsync(s->d_y, s->h_y, (size_t)B * 4, cudaMemcpyHostToDevice, stream));
+    HostSlot& h = s->slot[0];
+    memcpy(h.h_ids, ids_host, N * 4);
+    memcpy(h.h_y, y_host, (size_t)B * 4);
+    CU(cudaMemcpyAsync(h.d_ids, h.h_ids, N * 4, cudaMemcpyHostToDevice, stream));
+    CU(cudaMemcpyAsync(h.d_y, h.h_y, (size_t)B * 4, cudaMemcpyHostToDevice, stream));
     if (xv_host) {
-        memcpy(s->h_xv, xv_host, N * 4);
-        CU(cudaMemcpyAsync(s->d_xv, s->h_xv, N * 4, cudaMemcpyHostToDevice, stream));
+        memcpy(h.h_xv, xv_host, N * 4);
+        CU(cudaMemcpyAsync(h.d_xv, h.h_xv, N * 4, cudaMemcpyHostToDevice, stream));
     }
-    int rc = fmb_session_fm_step(s, s->d_ids, xv_host ? s->d_xv : nullptr, s->d_y, B, table, bias, key_bits,
+    int rc = fmb_session_fm_step(s, h.d_ids, xv_host ? h.d_xv : nullptr, h.d_y, B, table, bias, key_bits,
                                  loss_kind, lr, mode, s->d_loss, stream);
     if (rc) return rc;
-    CU(cudaMemcpyAsync(s->h_loss, s->d_loss, 4, cudaMemcpyDeviceToHost, stream));
+    CU(cudaMemcpyAsync(h.h_loss, s->d_loss, 4, cudaMemcpyDeviceToHost, stream));
     CU(cudaStreamSynchronize(stream));
-    if (loss_host) *loss_host = s->h_loss[0];
+    if (loss_host) *loss_host = *h.h_loss;
     return FMB_OK;
 }

@@ -28,8 +28,6 @@ from ._lib import AdagradState, FmbError, RunList, check, ptr
 UPDATE_ADAM1, UPDATE_SGD, UPDATE_FTRL = 0, 1, 2   # 2: per-coordinate FTRL-Proximal (enable_ftrl), FM-only steps
 UPDATE_ADAGRAD = 3   # torch.optim.Adagrad with state kept across calls (enable_adagrad): FM steps, tower fit, run_experiment
 LOSS_LOGITS, LOSS_LOGITS_OF_SIG = 0, 1
-_PRESORT_STANDALONE = __import__("os").environ.get("FMB_PRESORT_STANDALONE", "0") == "1"
-_DEEP_GRAPH = __import__("os").environ.get("FMB_DEEP_GRAPH", "1") != "0"   # tower `fit` replayed as one CUDA graph
 
 
 def _stream():
@@ -428,15 +426,10 @@ class _DeepBase(nn.Module):
             self._lib.fmb_session_presort_invalidate(s)   # a pre-sort is only ever honoured for the very same batch object
         nxt = next_batch if (next_batch is not None and next_batch.B == e.B) else None
         loss = torch.empty((), device=self.device)
-        inside = nxt is not None and not _PRESORT_STANDALONE
         check(self._lib.fmb_session_fm_step_next(s, ptr(e.ids), ptr(e.xv), ptr(e.y), e.B, ptr(self._table),
                                                  ptr(self.bias), self._key_bits, loss_kind, self._lr, self.update_mode,
-                                                 ptr(nxt.ids) if inside else None, ptr(loss), _stream()),
+                                                 ptr(nxt.ids) if nxt is not None else None, ptr(loss), _stream()),
               "fmb_session_fm_step_next")
-        if nxt is not None and not inside:
-            # the next batch's sort as a stand-alone launch on the session's side stream: it may still be running when this
-            # step's graph has finished (the step after waits for it), instead of being joined at the end of this graph
-            check(self._lib.fmb_session_presort(s, ptr(nxt.ids), nxt.B, self._key_bits), "fmb_session_presort")
         self._presorted = nxt
         return loss
 
@@ -520,7 +513,7 @@ class _DeepBase(nn.Module):
         """_deep_fit as ONE CUDA graph per configuration: the step is ~25 kernel launches through ctypes, which the host
         submits more slowly than the GPU runs them at cfg4's shapes.  First call of a configuration: eager (allocations,
         function attributes); second: captured on static input buffers; afterwards: copy the batch in, replay."""
-        if not _DEEP_GRAPH or torch.cuda.is_current_stream_capturing():
+        if torch.cuda.is_current_stream_capturing():
             return self._deep_fit(e)
         key = (e.B, e.xv is not None, self._lr, self.update_mode, int(self._lib.fmb_tensor_cores_enabled()))
         graphs = self.__dict__.setdefault("_fit_graphs", {})
@@ -592,7 +585,7 @@ class _DeepBase(nn.Module):
     def _hedge_fit_graphed(self, e):
         """_hedge_fit as one CUDA graph per configuration when it takes the single-pass route (large towers: ~40 launches
         through ctypes otherwise); same scheme as _deep_fit_graphed."""
-        if not _DEEP_GRAPH or torch.cuda.is_current_stream_capturing() or not self._hedge_single_pass(e.B):
+        if torch.cuda.is_current_stream_capturing() or not self._hedge_single_pass(e.B):
             return self._hedge_fit(e)
         key = ("hedge", e.B, e.xv is not None, self._lr)
         graphs = self.__dict__.setdefault("_fit_graphs", {})

@@ -374,7 +374,7 @@ int fmb_mlp_backward(const float* bi_dev, int ldbi, const float* mlp_dev, const 
                      int ldgbi, void* ws_dev, size_t ws_bytes, fmb_stream_t stream);
 /* Contractions of >= 2^24 multiply-adds (cfg4: B = 8192, H = 400) run on the tcgen05 tensor cores as 3xTF32
  * with fp32 accumulation in tensor memory (csrc/gemm_tc.cu, ~1e-6 relative); smaller ones -- every shape of the
- * reference's scripts -- on the exact SIMT kernel.  fmb_set_tensor_cores(0) (or FMB_TC=0) forces the exact path. */
+ * reference's scripts -- on the exact SIMT kernel.  fmb_set_tensor_cores(0) forces the exact path. */
 void fmb_set_tensor_cores(int on);
 int fmb_tensor_cores_enabled(void);
 int fmb_tensor_core_threshold_log2(void);

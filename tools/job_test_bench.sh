@@ -14,5 +14,3 @@ python bench.py --steps 20 --warmup 5 --no-cpu-baseline --no-extra > gpurun_out/
 show gpurun_out/${tag}_bench.json
 python bench.py --steps 200 --warmup 10 --no-cpu-baseline --no-extra > gpurun_out/${tag}_bench200.json 2> gpurun_out/${tag}_bench200.err || tail -5 gpurun_out/${tag}_bench200.err
 show gpurun_out/${tag}_bench200.json
-FMB_PRIO=0 python bench.py --steps 200 --warmup 10 --no-cpu-baseline --no-extra > gpurun_out/${tag}_bench200_noprio.json 2> /dev/null
-show gpurun_out/${tag}_bench200_noprio.json
