@@ -133,6 +133,11 @@ _SIGS = {
     "fmb_session_presort_invalidate": (None, [vp]),
     "fmb_session_set_ftrl": (C.c_int, [vp, vp, vp, C.c_float, C.c_float, C.c_float]),
     "fmb_session_set_adagrad": (C.c_int, [vp, vp, vp, C.c_float]),
+    "fmb_session_set_sparse_adam": (C.c_int, [vp, vp]),
+    "fmb_adam_scalars": (None, [C.c_float, C.c_double, C.c_double, C.c_int64, vp]),
+    "fmb_sparse_adam_advance": (C.c_int, [vp, C.c_float, C.c_int]),
+    "fmb_sparse_adam_online_steps": (C.c_int, [vp, C.c_float, C.c_int, C.c_int, vp]),
+    "fmb_update_dense_adam": (C.c_int, [vp, vp, C.c_int64, vp, vp]),
     "fmb_fm_step_fused_ex": (C.c_int, [vp, vp, vp, vp, vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_float, C.c_int, vp,
                                        vp, vp, vp, C.c_size_t, vp]),
     "fmb_fm_backward_runs_ex": (C.c_int, [vp, C.c_int64, vp, C.c_int, C.c_int, C.c_float, C.c_int, vp, vp, C.c_size_t,
@@ -164,6 +169,19 @@ class RunList(C.Structure):
 class AdagradState(C.Structure):
     """fmb_adagrad_t (include/fmb200.h): update mode 3's sums of the table, the bias and the tower, and eps."""
     _fields_ = [("sums", C.c_void_p), ("bias_sum", C.c_void_p), ("mlp_sums", C.c_void_p), ("eps", C.c_float)]
+
+
+class AdamStep(C.Structure):
+    _fields_ = [("emb_step", C.c_float), ("bias_step", C.c_float), ("bias_bc2s", C.c_float), ("mlp_step", C.c_float),
+                ("mlp_bc2s", C.c_float)]
+
+
+class SparseAdamState(C.Structure):
+    """fmb_sparse_adam_t (include/fmb200.h): update mode 4's moments, hyperparameters, step counters and the scalars of
+    the step being run."""
+    _fields_ = [("mv", C.c_void_p), ("bias_mv", C.c_void_p), ("mlp_mv", C.c_void_p), ("beta1", C.c_double),
+                ("beta2", C.c_double), ("eps", C.c_float), ("step", C.c_int64), ("mlp_step", C.c_int64),
+                ("cur", AdamStep), ("steps_dev", C.c_void_p)]
 
 
 def load():

@@ -54,6 +54,16 @@ __global__ void update_dense_adagrad_kernel(float* __restrict__ p, const float* 
     }
 }
 
+// update mode 4's dense Adam of the tower: m [n] at mv, v [n] at mv + n
+__global__ void update_dense_adam_kernel(float* __restrict__ p, const float* __restrict__ g, int64_t n, fmb::AdamState st) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) {
+        float m = st.mv[i], v = st.mv[n + i];
+        p[i] = fmb::adam_update(p[i], g[i], m, v, st);
+        st.mv[i] = m; st.mv[n + i] = v;
+    }
+}
+
 // ATen-order sum of x[0:n], parallel where the order allows it.  ATen's cascade (SumKernel.cpp multi_row_sum)
 // adds rows of 32 floats (4 ilp x 8 lanes) in blocks of `level_step` rows: a block's sum is
 // ((0 + r0) + r1) + ... and depends on nothing else, only the way block sums are folded upwards is serial.
@@ -117,7 +127,9 @@ __device__ float aten_sum_cta(const float* __restrict__ x, int64_t n, float* bs 
     return total;
 }
 
-// warps 0..15: bias -= step(sum(delta));  warps 16..31: loss_out = sum(lossv) / B
+// warps 0..15: bias -= step(sum(delta));  warps 16..31: loss_out = sum(lossv) / B.  SA: update mode 4 (Adam on st.adam, an
+// instantiation of its own so that the other modes' kernel stays as it is)
+template <bool SA>
 __global__ void __launch_bounds__(FIN_THREADS) finish_step_kernel(const float* __restrict__ delta,
                                                                   const float* __restrict__ lossv, int B, float* bias,
                                                                   float lr, int mode, float* loss_out,
@@ -140,7 +152,11 @@ __global__ void __launch_bounds__(FIN_THREADS) finish_step_kernel(const float* _
     }
     if (lane == 0) {
         if (half == 0) {
-            if (mode == 2) {
+            if (SA) {
+                float m = st.adam.mv[0], v = st.adam.mv[1];
+                bias[0] = fmb::adam_update(bias[0], total, m, v, st.adam);
+                st.adam.mv[0] = m; st.adam.mv[1] = v;
+            } else if (mode == 2) {
                 const fmb::FtrlState& ftrl = st.ftrl;
                 float z = ftrl.bias_zn[0], n = ftrl.bias_zn[1];
                 bias[0] = fmb::ftrl_update(bias[0], total, z, n, lr, ftrl.beta, ftrl.l1, ftrl.l2);
@@ -206,6 +222,15 @@ FMB_API int fmb_update_dense_ex(float* p, const float* g, int64_t n, float lr, i
     return FMB_OK;
 }
 
+// update mode 4: torch.optim.Adam on the tower's n parameters with the moments a->mlp_mv [2][n] and the scalars of
+// a->cur (fmb_sparse_adam_advance with tower = 1)
+FMB_API int fmb_update_dense_adam(float* p, const float* g, int64_t n, const fmb_sparse_adam_t* a, cudaStream_t stream) {
+    FMB_CHECK_ARG(p && g && n > 0 && a && a->mlp_mv, "fmb_update_dense_adam: bad arguments (needs the tower's moments)");
+    update_dense_adam_kernel<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(p, g, n, fmb_sa_dense(a, true));
+    FMB_CHECK_LAUNCH("update_dense_adam_kernel");
+    return FMB_OK;
+}
+
 // end of a training step: bias update from sum(delta) (bias nullable) and mean loss (loss_out nullable).
 // B <= 1 M samples (block sums are staged in shared memory up to 256 K samples, in `fmb_finish_scratch` above).
 static float* g_fin_scratch = nullptr;
@@ -230,7 +255,11 @@ FMB_API int fmb_finish_step_ex(const float* delta, const float* lossv, int B, fl
         scratch = g_fin_scratch;
     }
     static bool attr = false;
-    if (!attr) { cudaFuncSetAttribute(finish_step_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 132 * 1024); attr = true; }
+    if (!attr) {
+        cudaFuncSetAttribute(finish_step_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 132 * 1024);
+        cudaFuncSetAttribute(finish_step_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 132 * 1024);
+        attr = true;
+    }
     fmb::UpdateState fs;
     fs.ftrl = {nullptr, nullptr, 0.f, 0.f, 0.f};
     if (mode == 2) {
@@ -240,14 +269,21 @@ FMB_API int fmb_finish_step_ex(const float* delta, const float* lossv, int B, fl
         const fmb_adagrad_t* a = reinterpret_cast<const fmb_adagrad_t*>(ftrl);
         FMB_CHECK_ARG(bias == nullptr || (a && a->bias_sum), "fmb_finish_step: update mode 3 needs the Adagrad state");
         if (a) { fs.ada.sums = a->sums; fs.ada.bias_sum = a->bias_sum; fs.ada.eps = a->eps; }
+    } else if (mode == 4) {   // the state slot carries an fmb_sparse_adam_t advanced to this step (include/fmb200.h)
+        const fmb_sparse_adam_t* a = reinterpret_cast<const fmb_sparse_adam_t*>(ftrl);
+        FMB_CHECK_ARG(bias == nullptr || (a && a->bias_mv), "fmb_finish_step: update mode 4 needs the SparseAdam state");
+        if (a) fs.adam = fmb_sa_dense(a, false);
     }
-    finish_step_kernel<<<1, FIN_THREADS, smem, stream>>>(delta, lossv, B, bias, lr, mode, loss_out, scratch, fs);
+    if (mode == 4) finish_step_kernel<true><<<1, FIN_THREADS, smem, stream>>>(delta, lossv, B, bias, lr, mode, loss_out, scratch, fs);
+    else finish_step_kernel<false><<<1, FIN_THREADS, smem, stream>>>(delta, lossv, B, bias, lr, mode, loss_out, scratch, fs);
     FMB_CHECK_LAUNCH("finish_step_kernel");
     return FMB_OK;
 }
 
 // host-side handle of the kernel, for graph-node identification in session.cu (argument 6 of 9 = loss_out)
-FMB_API const void* fmb_finish_kernel_fn(void) { return (const void*)finish_step_kernel; }
+FMB_API const void* fmb_finish_kernel_fn(void) { return (const void*)finish_step_kernel<false>; }
+// the mode-4 instantiation (argument 8 = the bias's Adam state, re-pointed at every step's scalars by session.cu)
+const void* fmb_finish_sa_kernel_fn() { return (const void*)finish_step_kernel<true>; }
 
 FMB_API int fmb_finish_step(const float* delta, const float* lossv, int B, float* bias, float lr, int mode,
                             float* loss_out, cudaStream_t stream) {

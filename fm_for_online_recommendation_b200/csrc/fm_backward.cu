@@ -59,6 +59,7 @@ struct BwdParams {
     union {                // the update rule's per-coordinate state (same size as the FTRL state alone)
         fmb::FtrlState ftrl;   // mode 2 only
         fmb::AdagradState ada; // mode 3 only
+        fmb::SparseAdamState sa;   // mode 4 only
     };
     int min_run1;          // 1: rows hit once are summed (0 + g) and updated here too (AFM path: nothing updates them earlier)
     float* inbox[8];
@@ -73,22 +74,34 @@ struct BwdParams {
     int pdl;                       // 1: launched as a programmatic dependent of the kernel that stages G
 };
 
-// update of coordinate c of row `key` from its summed gradient: modes 0 / 1 in registers, mode 3 (Adagrad: ADA, an
-// instantiation of its own so that the others stay as they are) also reads and writes the coordinate's sum
-template <bool ADA>
+// The kernels below are instantiated once per kind of per-coordinate state (SK), so that adding a stateful rule leaves
+// the others' code as it is: SK_NONE (modes 0 / 1 in registers, mode 2 through p.ftrl), SK_ADA (mode 3: Adagrad's sum),
+// SK_SA (mode 4: SparseAdam's m and v, [R][2][rowp] like FTRL's z and n).
+enum { SK_NONE = 0, SK_ADA = 1, SK_SA = 2 };
+static int state_kind(int mode) { return mode == 3 ? SK_ADA : mode == 4 ? SK_SA : SK_NONE; }
+
+// update of coordinate c of row `key` from its summed gradient (modes 0, 1, 3, 4)
+template <int SK>
 __device__ __forceinline__ float row_update(const BwdParams& p, float old, float g, int32_t key, int c) {
-    if (ADA) {
+    if (SK == SK_ADA) {
         float* sp = p.ada.sums + (size_t)key * p.rowp + c;
         float sv = *sp;
         const float o = fmb::adagrad_update(old, g, sv, p.lr, p.ada.eps);
         *sp = sv;
         return o;
     }
+    if (SK == SK_SA) {
+        float* mp = p.sa.mv + (size_t)key * 2 * p.rowp + c;
+        float m = mp[0], v = mp[p.rowp];
+        const float o = fmb::sparse_adam_update(old, g, m, v, p.sa);
+        mp[0] = m; mp[p.rowp] = v;
+        return o;
+    }
     return fmb::apply_update_a(old, g, p.lr, p.astep, p.mode);
 }
 
 // ---------------------------------------------------------------------------------------------
-template <bool ADA>
+template <int SK>
 __global__ void __launch_bounds__(256) fm_bwd_entry_kernel(BwdParams p) {
     const int q = threadIdx.x & ((1 << p.ql_log) - 1);
     const int64_t i = (int64_t)blockIdx.x * (256 >> p.ql_log) + (threadIdx.x >> p.ql_log);
@@ -132,9 +145,9 @@ __global__ void __launch_bounds__(256) fm_bwd_entry_kernel(BwdParams p) {
             if (j < p.k) {
                 const float gr = two ? __fadd_rn(__fadd_rn(0.f, a[t]), __fadd_rn(0.f, c[t]))
                                      : __fadd_rn(0.f, p.gvec ? c[t] : a[t]);
-                o[t] = row_update<ADA>(p, v[t], gr, key, j);
+                o[t] = row_update<SK>(p, v[t], gr, key, j);
             } else if (j == p.k) {
-                o[t] = row_update<ADA>(p, v[t], __fadd_rn(0.f, a[t]), key, j);
+                o[t] = row_update<SK>(p, v[t], __fadd_rn(0.f, a[t]), key, j);
             } else {
                 o[t] = v[t];
             }
@@ -160,7 +173,7 @@ __global__ void __launch_bounds__(256) fm_bwd_entry_kernel(BwdParams p) {
 // loads, permutation, sample index, delta, feature value) is paid once per entry instead of once per
 // 16-byte chunk, which is what made the lane-per-chunk kernel instruction-bound (75 % issue utilisation,
 // ~450 instructions per lane: profiles/r1g).  Row and S reads are random per entry either way.
-template <int CU, bool ADA>
+template <int CU, int SK>
 __global__ void __launch_bounds__(256) fm_bwd_entry1_kernel(BwdParams p) {
     const int64_t i = (int64_t)blockIdx.x * 256 + threadIdx.x;
     if (i >= p.N) return;
@@ -203,9 +216,9 @@ __global__ void __launch_bounds__(256) fm_bwd_entry1_kernel(BwdParams p) {
             // the only entry of its row: sum = 0 + contribution; update from registers
             if (j < p.k) {
                 const float gr = two ? __fadd_rn(__fadd_rn(0.f, a), __fadd_rn(0.f, c)) : __fadd_rn(0.f, p.gvec ? c : a);
-                o[j] = row_update<ADA>(p, v[j], gr, key, j);
+                o[j] = row_update<SK>(p, v[j], gr, key, j);
             } else if (j == p.k) {
-                o[j] = row_update<ADA>(p, v[j], __fadd_rn(0.f, a), key, j);
+                o[j] = row_update<SK>(p, v[j], __fadd_rn(0.f, a), key, j);
             } else {
                 o[j] = v[j];
             }
@@ -272,7 +285,7 @@ __device__ __forceinline__ void tma_g2s_2d(void* smem_dst, const CUtensorMap* tm
 // bid / nblocks: this CTA's index among the CTAs running this body, and their number (the run-list launch runs two bodies:
 // its first CTAs take the long runs, the others the short ones).  segb_off: offset (floats) of the segment-count prefix in
 // dynamic shared memory.  warps_per_block: working warps (the CTA's other warps only help with the prefix).
-template <bool LIST, int RING_SE, int RING_NS, bool LONGM, bool ADA>
+template <bool LIST, int RING_SE, int RING_NS, bool LONGM, int SK>
 __device__ __forceinline__ void runs_body(const CUtensorMap& gmap, const BwdParams& p, int warps_per_block, int warp_f, int accs_n,
                                           int ring_comps, unsigned bid, unsigned nblocks, int segb_off) {
     constexpr int RING_SEP = RING_SE + 4;
@@ -532,11 +545,8 @@ __device__ __forceinline__ void runs_body(const CUtensorMap& gmap, const BwdPara
                 }
                 float* addr = p.table + (size_t)key * p.rowp + c;
                 const float old = c < 32 ? accs[accs_n + c] : *addr;
-                if (ADA) {
-                    float* sp = p.ada.sums + (size_t)key * p.rowp + c;
-                    float sv = *sp;
-                    *addr = fmb::adagrad_update(old, gsum, sv, p.lr, p.ada.eps);
-                    *sp = sv;
+                if (SK != SK_NONE) {
+                    *addr = row_update<SK>(p, old, gsum, key, c);
                 } else if (p.mode == 2) {
                     float* zp = p.ftrl.zn + (size_t)key * 2 * p.rowp + c;
                     float z = zp[0], n = zp[p.rowp];
@@ -560,23 +570,23 @@ __device__ __forceinline__ void runs_body(const CUtensorMap& gmap, const BwdPara
     }
 }
 
-// position-major launch (tower fit, AFM, sharded paths).  ADA: update mode 3 (Adagrad)
-template <bool ADA>
+// position-major launch (tower fit, AFM, sharded paths)
+template <int SK>
 __global__ void __launch_bounds__(256, 2) fm_bwd_runs_kernel(const __grid_constant__ CUtensorMap gmap, BwdParams p, int warps_per_block, int warp_f,
                                                              int accs_n, int ring_comps) {
-    runs_body<false, 64, 4, false, ADA>(gmap, p, warps_per_block, warp_f, accs_n, ring_comps, blockIdx.x, gridDim.x, 0);
+    runs_body<false, 64, 4, false, SK>(gmap, p, warps_per_block, warp_f, accs_n, ring_comps, blockIdx.x, gridDim.x, 0);
 }
 
 // run-list launch: CTAs [0, nlong) take the long runs (>= 128 entries: 128-entry stages, ring from the first entry, wpl
 // working warps), the others the short runs.  The long runs are the step's longest dependent chain, so their CTAs come
 // first in the grid and are placed first; as two launches the second one waited for shared memory behind the first.
 constexpr int LONG_SE = 128, LONG_NS = 4;
-template <bool ADA>
+template <int SK>
 __global__ void __launch_bounds__(256, 2) fm_bwd_runs_list_kernel(const __grid_constant__ CUtensorMap gmap_s, const __grid_constant__ CUtensorMap gmap_l,
                                                                   BwdParams p, int wps, int warp_f_s, int wpl, int warp_f_l, int accs_n,
                                                                   int ring_comps, unsigned nlong, int segb_off) {
-    if (blockIdx.x < nlong) runs_body<true, LONG_SE, LONG_NS, true, ADA>(gmap_l, p, wpl, warp_f_l, accs_n, ring_comps, blockIdx.x, nlong, segb_off);
-    else runs_body<true, 64, 4, false, ADA>(gmap_s, p, wps, warp_f_s, accs_n, ring_comps, blockIdx.x - nlong, gridDim.x - nlong, segb_off);
+    if (blockIdx.x < nlong) runs_body<true, LONG_SE, LONG_NS, true, SK>(gmap_l, p, wpl, warp_f_l, accs_n, ring_comps, blockIdx.x, nlong, segb_off);
+    else runs_body<true, 64, 4, false, SK>(gmap_s, p, wps, warp_f_s, accs_n, ring_comps, blockIdx.x - nlong, gridDim.x - nlong, segb_off);
 }
 
 static int ilog2_ceil(int x) { int l = 0; while ((1 << l) < x) ++l; return l; }
@@ -630,7 +640,7 @@ static int ring_tensor_map(CUtensorMap* gmap, const BwdParams& p, int nv, int ri
     return FMB_OK;
 }
 
-template <bool ADA>
+template <int SK>
 static int launch_runs_t(BwdParams& p, bool two, cudaStream_t stream) {
     const int k = p.k;
     const int64_t N = p.N;
@@ -646,15 +656,15 @@ static int launch_runs_t(BwdParams& p, bool two, cudaStream_t stream) {
     const unsigned grid = (unsigned)((nwarps + wpb - 1) / wpb);
     static bool attr = false;
     if (!attr) {
-        cudaFuncSetAttribute(fm_bwd_runs_kernel<ADA>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-        cudaFuncSetAttribute(fm_bwd_runs_list_kernel<ADA>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+        cudaFuncSetAttribute(fm_bwd_runs_kernel<SK>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+        cudaFuncSetAttribute(fm_bwd_runs_list_kernel<SK>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
         attr = true;
     }
     CUtensorMap gmap;
     int rc = ring_tensor_map(&gmap, p, nv, ring_comps, 64);
     if (rc) return rc;
     if (!p.run_list) {
-        fm_bwd_runs_kernel<ADA><<<grid, 32 * wpb, sm, stream>>>(gmap, p, wpb, warp_f, accs_n, ring_comps);
+        fm_bwd_runs_kernel<SK><<<grid, 32 * wpb, sm, stream>>>(gmap, p, wpb, warp_f, accs_n, ring_comps);
         FMB_CHECK_LAUNCH("fm_bwd_runs_kernel");
         return FMB_OK;
     }
@@ -686,18 +696,48 @@ static int launch_runs_t(BwdParams& p, bool two, cudaStream_t stream) {
         at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
         at[0].val.programmaticStreamSerializationAllowed = 1;
         cfg.attrs = at; cfg.numAttrs = 1;
-        const cudaError_t le = cudaLaunchKernelEx(&cfg, fm_bwd_runs_list_kernel<ADA>, gmap, gmap_l, p, wpb, warp_f, wpl, warp_f_l, accs_n,
+        const cudaError_t le = cudaLaunchKernelEx(&cfg, fm_bwd_runs_list_kernel<SK>, gmap, gmap_l, p, wpb, warp_f, wpl, warp_f_l, accs_n,
                                                   ring_comps, nlong, (int)(smd / 4));
         if (le != cudaSuccess) { fmb_set_error("fm_bwd_runs_list_kernel (programmatic launch): %s", cudaGetErrorString(le)); return FMB_ERR_CUDA; }
     } else {
-        fm_bwd_runs_list_kernel<ADA><<<nlong + nshort, 32 * wpb, smd + segb, stream>>>(gmap, gmap_l, p, wpb, warp_f, wpl, warp_f_l, accs_n,
+        fm_bwd_runs_list_kernel<SK><<<nlong + nshort, 32 * wpb, smd + segb, stream>>>(gmap, gmap_l, p, wpb, warp_f, wpl, warp_f_l, accs_n,
                                                                                  ring_comps, nlong, (int)(smd / 4));
     }
     FMB_CHECK_LAUNCH("fm_bwd_runs_list_kernel");
     return FMB_OK;
 }
 static int launch_runs(BwdParams& p, bool two, cudaStream_t stream) {
-    return p.mode == 3 ? launch_runs_t<true>(p, two, stream) : launch_runs_t<false>(p, two, stream);
+    switch (state_kind(p.mode)) {
+        case SK_ADA: return launch_runs_t<SK_ADA>(p, two, stream);
+        case SK_SA: return launch_runs_t<SK_SA>(p, two, stream);
+        default: return launch_runs_t<SK_NONE>(p, two, stream);
+    }
+}
+
+// the mode-4 run-list kernel (graph-node identification in session.cu), and a copy of its captured BwdParams argument
+// `src` re-pointed at the SparseAdam step size of `a->cur` (argument 2 of the node)
+const void* fmb_runs_list_sa_kernel_fn() { return (const void*)fm_bwd_runs_list_kernel<SK_SA>; }
+void fmb_runs_params_sa(const void* src, void* dst, const fmb_sparse_adam_t* a) {
+    static_assert(sizeof(BwdParams) <= 512, "session.cu patches BwdParams through a 512-byte buffer");
+    BwdParams p = *static_cast<const BwdParams*>(src);
+    p.sa.step = a->cur.emb_step;
+    *static_cast<BwdParams*>(dst) = p;
+}
+
+// the entry kernels of fmb_fm_backward_update_rl_ex for state kind SK
+template <int SK>
+static void launch_entries(const BwdParams& p, cudaStream_t stream) {
+    const unsigned grid1 = (unsigned)((p.N + 255) / 256);
+    switch (p.cu) {
+        case 1: fm_bwd_entry1_kernel<1, SK><<<grid1, 256, 0, stream>>>(p); break;
+        case 2: fm_bwd_entry1_kernel<2, SK><<<grid1, 256, 0, stream>>>(p); break;
+        case 3: fm_bwd_entry1_kernel<3, SK><<<grid1, 256, 0, stream>>>(p); break;
+        case 4: fm_bwd_entry1_kernel<4, SK><<<grid1, 256, 0, stream>>>(p); break;
+        default: {
+            const int epb = 256 >> p.ql_log;
+            fm_bwd_entry_kernel<SK><<<(unsigned)((p.N + epb - 1) / epb), 256, 0, stream>>>(p);
+        }
+    }
 }
 
 // A6 sparse backward + update (see file header).
@@ -712,7 +752,8 @@ static int launch_runs(BwdParams& p, bool two, cudaStream_t stream) {
 // one warp per run, the long runs first (the owner-side chains of the sharded step are G*B/rows long)
 struct fmb_runlist_t { int32_t* entries; uint32_t* seg_count; int nseg, seg_cap; };   // include/fmb200.h
 struct fmb_adagrad_t { float* sums; float* bias_sum; float* mlp_sums; float eps; };   // include/fmb200.h
-// _rl_ex: update mode 3 (Adagrad) needs `ada` (the table's sums); NULL otherwise
+// _rl_ex: update mode 3 (Adagrad) needs `ada` (the table's sums), mode 4 (SparseAdam) an fmb_sparse_adam_t in the same
+// slot, advanced to this step; NULL otherwise
 FMB_API int fmb_fm_backward_update_rl_ex(const int32_t* sorted_keys, const int32_t* perm, int64_t N, int64_t n_entries,
                                          const float* xv, float* table, int F, int k, const float* S, int s_pitch,
                                          const float* gs, int gs_stride, int use_fm2, const float* gvec,
@@ -723,8 +764,10 @@ FMB_API int fmb_fm_backward_update_rl_ex(const int32_t* sorted_keys, const int32
     FMB_CHECK_ARG(sorted_keys && perm && table && S && gs && ws, "fmb_fm_backward_update: null pointer");
     FMB_CHECK_ARG(N > 0 && F > 0 && F < 512 && k > 0 && k <= 124, "fmb_fm_backward_update: bad shape N=%lld F=%d k=%d (need F < 512, k <= 124)",
                   (long long)N, F, k);
-    FMB_CHECK_ARG(mode == 0 || mode == 1 || (mode == 3 && ada && ada->sums),
-                  "fmb_fm_backward_update: unknown update mode %d (mode 3 needs the Adagrad state)", mode);
+    FMB_CHECK_ARG(mode == 0 || mode == 1 || (mode == 3 && ada && ada->sums) ||
+                  (mode == 4 && ada && reinterpret_cast<const fmb_sparse_adam_t*>(ada)->mv),
+                  "fmb_fm_backward_update: unknown update mode %d (mode 3 needs the Adagrad state, mode 4 the SparseAdam state)",
+                  mode);
     FMB_CHECK_ARG(use_fm2 || gvec, "fmb_fm_backward_update: neither gradient path enabled");
     FMB_CHECK_ARG(n_entries > 0 && n_entries < ((int64_t)1 << 31), "fmb_fm_backward_update: n_entries out of range");
     if (ws_bytes < fmb_bwd_workspace_bytes(N, k)) { fmb_set_error("fmb_fm_backward_update: workspace too small"); return FMB_ERR_WS; }
@@ -744,33 +787,15 @@ FMB_API int fmb_fm_backward_update_rl_ex(const int32_t* sorted_keys, const int32
     p.s_pitch = s_pitch; p.gs_stride = gs_stride; p.key_limit = key_limit;
     p.astep = -(lr / 0.1f);
     if (mode == 3) { p.ada.sums = ada->sums; p.ada.bias_sum = ada->bias_sum; p.ada.eps = ada->eps; }
+    if (mode == 4) p.sa = fmb_sa_tables(reinterpret_cast<const fmb_sparse_adam_t*>(ada));
     p.dbg = g_runs_dbg;
     p.Npad = bwd_npad(N);
     p.G = (float*)ws;
     const bool two = use_fm2 && gvec;
-    const unsigned grid1 = (unsigned)((N + 255) / 256);
-    if (mode == 3) {
-        switch (p.cu) {
-            case 1: fm_bwd_entry1_kernel<1, true><<<grid1, 256, 0, stream>>>(p); break;
-            case 2: fm_bwd_entry1_kernel<2, true><<<grid1, 256, 0, stream>>>(p); break;
-            case 3: fm_bwd_entry1_kernel<3, true><<<grid1, 256, 0, stream>>>(p); break;
-            case 4: fm_bwd_entry1_kernel<4, true><<<grid1, 256, 0, stream>>>(p); break;
-            default: {
-                const int epb = 256 >> p.ql_log;
-                fm_bwd_entry_kernel<true><<<(unsigned)((N + epb - 1) / epb), 256, 0, stream>>>(p);
-            }
-        }
-    } else {
-        switch (p.cu) {
-            case 1: fm_bwd_entry1_kernel<1, false><<<grid1, 256, 0, stream>>>(p); break;
-            case 2: fm_bwd_entry1_kernel<2, false><<<grid1, 256, 0, stream>>>(p); break;
-            case 3: fm_bwd_entry1_kernel<3, false><<<grid1, 256, 0, stream>>>(p); break;
-            case 4: fm_bwd_entry1_kernel<4, false><<<grid1, 256, 0, stream>>>(p); break;
-            default: {
-                const int epb = 256 >> p.ql_log;
-                fm_bwd_entry_kernel<false><<<(unsigned)((N + epb - 1) / epb), 256, 0, stream>>>(p);
-            }
-        }
+    switch (state_kind(mode)) {
+        case SK_ADA: launch_entries<SK_ADA>(p, stream); break;
+        case SK_SA: launch_entries<SK_SA>(p, stream); break;
+        default: launch_entries<SK_NONE>(p, stream);
     }
     FMB_CHECK_LAUNCH("fm_bwd_entry_kernel");
     if (rl) { p.run_list = reinterpret_cast<const int4*>(rl->entries); p.run_segc = rl->seg_count; p.run_nseg = rl->nseg; p.run_cap = rl->seg_cap; }
@@ -812,7 +837,8 @@ int fmb_fm_backward_runs_list_launch(const int32_t* sorted_keys, int64_t N, floa
     FMB_CHECK_ARG(N > 0 && F > 0 && F < 512 && k > 0 && k <= 124, "fmb_fm_backward_runs: bad shape N=%lld F=%d k=%d (need F < 512, k <= 124)",
                   (long long)N, F, k);
     FMB_CHECK_ARG(mode == 0 || mode == 1 || (mode == 2 && ftrl && ftrl->zn) ||
-                  (mode == 3 && ftrl && reinterpret_cast<const fmb_adagrad_t*>(ftrl)->sums),
+                  (mode == 3 && ftrl && reinterpret_cast<const fmb_adagrad_t*>(ftrl)->sums) ||
+                  (mode == 4 && ftrl && reinterpret_cast<const fmb_sparse_adam_t*>(ftrl)->mv),
                   "fmb_fm_backward_runs: unknown update mode %d", mode);
     if (ws_bytes < fmb_bwd_workspace_bytes(N, k)) { fmb_set_error("fmb_fm_backward_runs: workspace too small"); return FMB_ERR_WS; }
     BwdParams p;
@@ -829,6 +855,7 @@ int fmb_fm_backward_runs_list_launch(const int32_t* sorted_keys, int64_t N, floa
         const fmb_adagrad_t* a = reinterpret_cast<const fmb_adagrad_t*>(ftrl);
         p.ada.sums = a->sums; p.ada.bias_sum = a->bias_sum; p.ada.eps = a->eps;
     }
+    if (mode == 4) p.sa = fmb_sa_tables(reinterpret_cast<const fmb_sparse_adam_t*>(ftrl));   // the slot carries an fmb_sparse_adam_t
     if (rl) { p.run_list = reinterpret_cast<const int4*>(rl->entries); p.run_segc = rl->seg_count; p.run_nseg = rl->nseg; p.run_cap = rl->seg_cap; }
     p.pdl = rl && pdl;
     p.dbg = g_runs_dbg;
@@ -856,6 +883,7 @@ FMB_API int fmb_fm_backward_runs_all(const int32_t* sorted_keys, int64_t N, floa
                                      int mode, void* ws, size_t ws_bytes, cudaStream_t stream) {
     FMB_CHECK_ARG(sorted_keys && table && ws, "fmb_fm_backward_runs_all: null pointer");
     FMB_CHECK_ARG(N > 0 && F > 0 && F < 512 && k > 0 && k <= 124, "fmb_fm_backward_runs_all: bad arguments");
+    FMB_CHECK_ARG(mode != 4, "fmb_fm_backward_runs_all: update mode 4 (SparseAdam) is not supported");
     FMB_CHECK_ARG(mode == 0 || mode == 1, "fmb_fm_backward_runs_all: unknown update mode %d", mode);
     if (ws_bytes < fmb_bwd_workspace_bytes(N, k)) { fmb_set_error("fmb_fm_backward_runs_all: workspace too small"); return FMB_ERR_WS; }
     BwdParams p;

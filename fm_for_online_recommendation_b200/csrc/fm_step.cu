@@ -51,6 +51,7 @@ struct StepParams {
     union {                    // the update rule's per-coordinate state (same size as the FTRL state alone)
         fmb::FtrlState ftrl;       // mode 2 only
         fmb::AdagradState ada;     // mode 3 only
+        fmb::SparseAdamState sa;   // mode 4 only
     };
     long long* tdbg;           // debug only: per-CTA phase timestamps [grid][8] (globaltimer ns), else NULL
     int dbg;                   // debug/attribution only (fmb_debug_set_step_flags): 1 = skip phase 4a, 2 = skip phase 4b
@@ -62,10 +63,10 @@ struct StepParams {
 // memory is then a constant and the field loop addresses with immediates), 0 = read it from the parameters;
 // XV = the batch carries real feature values (else all ones: no loads, no multiplications by x -- a product with 1.0f
 // is exact, so skipping it changes no bit); MODE = update rule (0 fresh-Adam sign step, 1 SGD, 2 FTRL-Proximal,
-// 3 Adagrad).
+// 3 Adagrad, 4 SparseAdam).
 // 32 registers (8 CTAs per SM): the 1 024 tiles of an 8 192-sample batch are then resident at once.
 template <int CU, bool XV, int MODE>
-__global__ void __launch_bounds__(256, MODE == 2 ? 4 : 8) fm_step_fused_kernel(const int32_t* __restrict__ ids, const float* __restrict__ xv,
+__global__ void __launch_bounds__(256, MODE == 2 || MODE == 4 ? 4 : 8) fm_step_fused_kernel(const int32_t* __restrict__ ids, const float* __restrict__ xv,
                                                             const float* __restrict__ y, const uint32_t* __restrict__ posflag,
                                                             StepParams p) {
     extern __shared__ __align__(16) float smem[];
@@ -199,7 +200,7 @@ __global__ void __launch_bounds__(256, MODE == 2 ? 4 : 8) fm_step_fused_kernel(c
         const float4 v4 = *reinterpret_cast<const float4*>(rows_s + (size_t)ef * rp + q * 4);
         const float Sq[4] = {S4.x, S4.y, S4.z, S4.w};
         const float v[4] = {v4.x, v4.y, v4.z, v4.w};
-        if (MODE != 2) {
+        if (MODE != 2 && MODE != 4) {   // SparseAdam steps every row hit, a zero gradient too (m and v decay)
             // Saturated samples (the reference's N(0,1) initialisation puts |z| ~ 90 on Criteo-shaped rows) leave their
             // rows exactly where they are; two exact item-level tests spare them the per-coordinate work.
             // (i) delta == 0 (sigmoid rounded to y): every gradient is +0 after the `0 +`, and the Adam step of a zero
@@ -245,6 +246,33 @@ __global__ void __launch_bounds__(256, MODE == 2 ? 4 : 8) fm_step_fused_kernel(c
             }
             *reinterpret_cast<float4*>(p.table + (size_t)ids_s[ef] * p.rowp + q * 4) = make_float4(o[0], o[1], o[2], o[3]);
             *reinterpret_cast<float4*>(srow) = make_float4(sv[0], sv[1], sv[2], sv[3]);   // padding lanes: as read
+            continue;
+        }
+        if (MODE == 4) {
+            // SparseAdam: the row's m and v sub-rows, in FTRL's [R][2][rowp] layout (read + written: 16F(k+1) more bytes
+            // per sample).  Gradient and update per coordinate, as in mode 3.
+            float* mrow = p.sa.mv + (size_t)ids_s[ef] * 2 * p.rowp + q * 4;
+            const float4 m4 = *reinterpret_cast<const float4*>(mrow), w4 = *reinterpret_cast<const float4*>(mrow + p.rowp);
+            float mv[4] = {m4.x, m4.y, m4.z, m4.w}, vv[4] = {w4.x, w4.y, w4.z, w4.w}, o[4];
+#pragma unroll
+            for (int t = 0; t < 4; ++t) {
+                const int j = q * 4 + t;
+                o[t] = v[t];
+                if (j <= k) {
+                    float a;
+                    if (j < k) {
+                        const float ej = XV ? __fmul_rn(v[t], x) : v[t];
+                        a = __fsub_rn(__fmul_rn(d, Sq[t]), __fmul_rn(d, ej));
+                        if (XV) a = __fmul_rn(a, x);
+                    } else {
+                        a = XV ? __fmul_rn(d, x) : d;
+                    }
+                    o[t] = fmb::sparse_adam_update(v[t], __fadd_rn(0.f, a), mv[t], vv[t], p.sa);
+                }
+            }
+            *reinterpret_cast<float4*>(p.table + (size_t)ids_s[ef] * p.rowp + q * 4) = make_float4(o[0], o[1], o[2], o[3]);
+            *reinterpret_cast<float4*>(mrow) = make_float4(mv[0], mv[1], mv[2], mv[3]);   // padding lanes: as read
+            *reinterpret_cast<float4*>(mrow + p.rowp) = make_float4(vv[0], vv[1], vv[2], vv[3]);
             continue;
         }
         float o[4];
@@ -397,8 +425,8 @@ FMB_API void fmb_debug_set_step_flags(int f) { g_step_dbg = f; }
 typedef void (*fused_fn_t)(const int32_t*, const float*, const float*, const uint32_t*, StepParams);
 static fused_fn_t fused_fn(int cu, bool xv, int mode) {
 #define FMB_FUSED_ROW(C, X) {fm_step_fused_kernel<C, X, 0>, fm_step_fused_kernel<C, X, 1>, fm_step_fused_kernel<C, X, 2>, \
-                             fm_step_fused_kernel<C, X, 3>}
-    static const fused_fn_t tab[2][2][4] = {{FMB_FUSED_ROW(0, false), FMB_FUSED_ROW(0, true)},
+                             fm_step_fused_kernel<C, X, 3>, fm_step_fused_kernel<C, X, 4>}
+    static const fused_fn_t tab[2][2][5] = {{FMB_FUSED_ROW(0, false), FMB_FUSED_ROW(0, true)},
                                             {FMB_FUSED_ROW(3, false), FMB_FUSED_ROW(3, true)}};
 #undef FMB_FUSED_ROW
     return tab[cu == 3][xv][mode];
@@ -407,9 +435,17 @@ static fused_fn_t fused_fn(int cu, bool xv, int mode) {
 FMB_API int fmb_is_fused_kernel_fn(const void* fn) {
     for (int c = 0; c < 2; ++c)
         for (int x = 0; x < 2; ++x)
-            for (int m = 0; m < 4; ++m)
+            for (int m = 0; m < 5; ++m)
                 if (fn == (const void*)fused_fn(c ? 3 : 0, x != 0, m)) return 1;
     return 0;
+}
+// a mode-4 step graph's fused-kernel node re-pointed at this step's scalar (session.cu): `dst` receives a copy of the
+// captured StepParams argument `src` with the SparseAdam step size of `a->cur`
+void fmb_fused_params_sa(const void* src, void* dst, const fmb_sparse_adam_t* a) {
+    static_assert(sizeof(StepParams) <= 512, "session.cu patches StepParams through a 512-byte buffer");
+    StepParams p = *static_cast<const StepParams*>(src);
+    p.sa.step = a->cur.emb_step;
+    *static_cast<StepParams*>(dst) = p;
 }
 
 // per-entry sorted position + multi-hit flag from the stable sort's output (fmb_sort_fields / fmb_sort_segment);
@@ -449,8 +485,10 @@ FMB_API int fmb_fm_step_fused_ex(const int32_t* ids, const float* xv, const floa
     FMB_CHECK_ARG(B > 0 && F > 0 && F < 512 && k > 0 && k <= 124, "fmb_fm_step_fused: bad shape B=%d F=%d k=%d", B, F, k);
     FMB_CHECK_ARG(loss_kind == 0 || loss_kind == 1, "fmb_fm_step_fused: unknown loss kind %d", loss_kind);
     FMB_CHECK_ARG(mode == 0 || mode == 1 || (mode == 2 && ftrl && ftrl->zn) ||
-                  (mode == 3 && ftrl && reinterpret_cast<const fmb_adagrad_t*>(ftrl)->sums),
-                  "fmb_fm_step_fused: unknown update mode %d (mode 2 needs the FTRL state, mode 3 the Adagrad state)", mode);
+                  (mode == 3 && ftrl && reinterpret_cast<const fmb_adagrad_t*>(ftrl)->sums) ||
+                  (mode == 4 && ftrl && reinterpret_cast<const fmb_sparse_adam_t*>(ftrl)->mv),
+                  "fmb_fm_step_fused: unknown update mode %d (mode 2 needs the FTRL state, mode 3 the Adagrad state, mode 4 "
+                  "the SparseAdam state)", mode);
     const int64_t N = (int64_t)B * F;
     if (ws_bytes < fmb_bwd_workspace_bytes(N, k)) { fmb_set_error("fmb_fm_step_fused: workspace too small"); return FMB_ERR_WS; }
     StepParams p;
@@ -465,6 +503,7 @@ FMB_API int fmb_fm_step_fused_ex(const int32_t* ids, const float* xv, const floa
     p.ftrl.zn = nullptr; p.ftrl.bias_zn = nullptr; p.ftrl.beta = p.ftrl.l1 = p.ftrl.l2 = 0.f;
     if (mode == 2) { p.ftrl.zn = ftrl->zn; p.ftrl.bias_zn = ftrl->bias_zn; p.ftrl.beta = ftrl->beta; p.ftrl.l1 = ftrl->l1; p.ftrl.l2 = ftrl->l2; }
     if (mode == 3) { const fmb_adagrad_t* a = reinterpret_cast<const fmb_adagrad_t*>(ftrl); p.ada.sums = a->sums; p.ada.bias_sum = a->bias_sum; p.ada.eps = a->eps; }
+    if (mode == 4) p.sa = fmb_sa_tables(reinterpret_cast<const fmb_sparse_adam_t*>(ftrl));
     p.tdbg = g_step_tdbg;
     int SB = 256 >> p.jl_log;
     if (SB < 4) SB = 4;

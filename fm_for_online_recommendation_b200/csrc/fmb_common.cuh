@@ -222,16 +222,55 @@ struct AdagradState {
     float* bias_sum;  // [1]
     float eps;
 };
-// the per-coordinate state of modes 2 and 3 in one kernel argument
+// mode 4: torch.optim.SparseAdam on the tables and torch.optim.Adam on the bias and the tower, moments kept across calls.
+// The per-step scalars (bias corrections, step sizes) are computed on the host in double as CPython does and rounded to
+// float as ATen rounds a Python scalar (fmb_sparse_adam_advance, common.cu); the kernels never evaluate pow.
+// The tables' state (24 bytes: fits the union beside the FTRL state)
+struct SparseAdamState {
+    float* mv;        // [R][2][rowp]: m sub-row, v sub-row of every packed table row (padding never written)
+    float b1c, b2c;   // (float)(1 - beta1), (float)(1 - beta2)
+    float eps;
+    float step;       // this step's (float)(-lr * sqrt(1 - beta2^t) / (1 - beta1^t))
+};
+// dense Adam of one parameter group (the bias, the tower): 32 bytes, the size of the FTRL state
+struct AdamState {
+    float* mv;        // m [n], then v [n]
+    float b1c, b2f, b2c, eps;   // (float)(1 - beta1), (float)beta2, (float)(1 - beta2), eps
+    float step;       // this step's (float)(-lr / (1 - beta1^t))
+    float bc2s;       // (float)((1 - beta2^t) ** 0.5)
+};
+// the per-coordinate state of modes 2, 3 and (bias) 4 in one kernel argument
 union UpdateState {
     FtrlState ftrl;
     AdagradState ada;
+    AdamState adam;
 };
 __device__ __forceinline__ float adagrad_update(float p, float g, float& s, float lr, float eps) {
     const float ss = __fmaf_rn(g, g, s);
     s = ss;
     const float sd = __fadd_rn(sqrt_mkl(ss), eps);
     return __fadd_rn(p, __fdiv_rn(__fmul_rn(-lr, g), sd));
+}
+// torch 2.11's CPU sparse_adam (optim/_functional.py) on one coordinate of a row the batch hits -- also when g == 0:
+// the moments decay and p moves by m' (tests/sparse_adam_oracle.c orc_sparse_adam_update is the same sequence):
+//   u1 = (g - m) * (1-b1);  m' = m + u1;  u2 = (g*g - v) * (1-b2);  v' = v + u2
+//   p' = p + step * ((u1 + m) / (sqrt(u2 + v) + eps))     (u1 + m == m', u2 + v == v': the adds commute)
+__device__ __forceinline__ float sparse_adam_update(float p, float g, float& m, float& v, const SparseAdamState& s) {
+    const float u1 = __fmul_rn(__fsub_rn(g, m), s.b1c);
+    const float u2 = __fmul_rn(__fsub_rn(__fmul_rn(g, g), v), s.b2c);
+    m = __fadd_rn(m, u1);
+    v = __fadd_rn(v, u2);
+    return __fadd_rn(p, __fmul_rn(s.step, __fdiv_rn(m, __fadd_rn(sqrt_mkl(v), s.eps))));
+}
+// torch 2.11's CPU _single_tensor_adam (tests/sparse_adam_oracle.c orc_adam_update):
+//   exp_avg.lerp_(g, 1-b1)                     m' = fma(1-b1, g - m, m)   (ATen's lerp for a weight < 0.5)
+//   exp_avg_sq.mul_(b2).addcmul_(g, g, 1-b2)   v' = fma((1-b2) * g, g, v * b2)
+//   denom = sqrt(v') / bc2s + eps;  param.addcdiv_(m', denom, value=step)   p' = p + (step * m') / denom
+__device__ __forceinline__ float adam_update(float p, float g, float& m, float& v, const AdamState& s) {
+    m = __fmaf_rn(s.b1c, __fsub_rn(g, m), m);
+    v = __fmaf_rn(__fmul_rn(s.b2c, g), g, __fmul_rn(v, s.b2f));
+    const float d = __fadd_rn(__fdiv_rn(sqrt_mkl(v), s.bc2s), s.eps);
+    return __fadd_rn(p, __fdiv_rn(__fmul_rn(s.step, m), d));
 }
 // same with the Adam step size precomputed
 __device__ __forceinline__ float apply_update_a(float p, float g, float lr, float astep, int mode) {
@@ -355,3 +394,25 @@ __device__ __forceinline__ float aten_row_sum_warp(const float* __restrict__ x, 
 }
 
 }  // namespace fmb
+
+// update mode 4's state and step counters (include/fmb200.h fmb_sparse_adam_t); the per-step scalars in `cur` are those
+// of the step being run, filled by fmb_sparse_adam_advance (common.cu)
+struct fmb_adam_step_t { float emb_step, bias_step, bias_bc2s, mlp_step, mlp_bc2s; };
+struct fmb_sparse_adam_t {
+    float* mv;        // [R][2][rowp]
+    float* bias_mv;   // [2]
+    float* mlp_mv;    // [2][n_mlp] or NULL
+    double beta1, beta2;
+    float eps;
+    int64_t step, mlp_step;
+    fmb_adam_step_t cur;
+    const float* steps_dev;   // fmb_online_deep_run_ex: [4 + 5N] (fmb_sparse_adam_online_steps), else unused
+};
+static inline fmb::SparseAdamState fmb_sa_tables(const fmb_sparse_adam_t* a) {
+    return {a->mv, (float)(1.0 - a->beta1), (float)(1.0 - a->beta2), a->eps, a->cur.emb_step};
+}
+// the bias's (tower = false) or the tower's dense Adam state; `n` = parameters of the group (the v half follows m)
+static inline fmb::AdamState fmb_sa_dense(const fmb_sparse_adam_t* a, bool tower) {
+    return {tower ? a->mlp_mv : a->bias_mv, (float)(1.0 - a->beta1), (float)a->beta2, (float)(1.0 - a->beta2), a->eps,
+            tower ? a->cur.mlp_step : a->cur.bias_step, tower ? a->cur.mlp_bc2s : a->cur.bias_bc2s};
+}

@@ -28,10 +28,13 @@ struct OnlineParams {
     float* acc;          // [n_mlp] hedge accumulator (ONN)
     float lr, hb, hs;
     int mode;
-    float* ada_sums;     // mode 3 (Adagrad): sums of the table [R][rowp], the bias [1] and the tower [n_mlp]
-    float* ada_bias;
+    float* ada_sums;     // mode 3 (Adagrad): sums of the table [R][rowp], the bias [1] and the tower [n_mlp];
+    float* ada_bias;     // mode 4 (SparseAdam): m and v of the table [R][2][rowp], the bias [2] and the tower [2][n_mlp]
     float* ada_mlp;
-    float eps;
+    union {
+        float eps;                // mode 3
+        const float* sa_steps;    // mode 4: [4 + 5N] = (1-b1, b2, 1-b2, eps), then the five scalars of every example
+    };
     uint8_t* preds;      // [N]
     int64_t* conf;       // [4] tp, fp, tn, fn
 };
@@ -40,20 +43,37 @@ __device__ __forceinline__ size_t w_off(int k, int H, int l) {
     return l == 0 ? 0 : (size_t)H * k + H + (size_t)(l - 1) * ((size_t)H * H + H);
 }
 
-// the Adam family's update of one parameter; mode 3 (ADA, an instantiation of its own so that the other modes' kernel
-// stays as it is) also reads and writes its Adagrad sum *s
-template <bool ADA>
-__device__ __forceinline__ float online_update(const OnlineParams& p, float w, float g, float* s) {
-    if (ADA) {
+// The Adam family's update of one parameter of group grp (0 table, 1 bias, 2 tower) at example n.  The kernel is
+// instantiated once per kind of state SK, so that the other modes' kernel stays as it is: 0 none, 1 Adagrad (mode 3:
+// the sum *s), 2 SparseAdam on the table and Adam on the bias and the tower (mode 4: m at s[0], v one sub-row / one
+// group further; the step's scalars from the host-filled table p.sa_steps).
+template <int SK>
+__device__ __forceinline__ float online_update(const OnlineParams& p, float w, float g, float* s, int grp, int n) {
+    if (SK == 1) {
         float sv = *s;
         const float o = fmb::adagrad_update(w, g, sv, p.lr, p.eps);
         *s = sv;
         return o;
     }
+    if (SK == 2) {
+        const float* c = p.sa_steps;
+        const float* st = c + 4 + (size_t)5 * n;
+        const size_t vo = grp == 0 ? (size_t)p.rowp : grp == 1 ? 1 : w_off(p.k, p.H, p.L);
+        float m = s[0], v = s[vo], o;
+        if (grp == 0) {
+            const fmb::SparseAdamState a = {nullptr, c[0], c[2], c[3], st[0]};
+            o = fmb::sparse_adam_update(w, g, m, v, a);
+        } else {
+            const fmb::AdamState a = {nullptr, c[0], c[1], c[2], c[3], st[grp == 1 ? 1 : 3], st[grp == 1 ? 2 : 4]};
+            o = fmb::adam_update(w, g, m, v, a);
+        }
+        s[0] = m; s[vo] = v;
+        return o;
+    }
     return fmb::apply_update(w, g, p.lr, p.mode);
 }
 
-template <bool ADA>
+template <int SK>
 __global__ void __launch_bounds__(OT) online_deep_kernel(OnlineParams p) {
     extern __shared__ __align__(16) float sm[];
     const int F = p.F, k = p.k, L = p.L, H = p.H, rp = p.cu * 4;
@@ -176,10 +196,10 @@ __global__ void __launch_bounds__(OT) online_deep_kernel(OnlineParams p) {
                     __syncthreads();
                     for (int q = tid; q < H * nin; q += OT) {  // fresh-Adam step on W_l (gradient = gp[o]*x[i], B = 1)
                         const int o = q / nin, i = q - o * nin;
-                        W[q] = online_update<ADA>(p, W[q], __fmaf_rn(gp[o], xin[i], 0.f), p.ada_mlp + w_off(k, H, l) + q);
+                        W[q] = online_update<SK>(p, W[q], __fmaf_rn(gp[o], xin[i], 0.f), p.ada_mlp + w_off(k, H, l) + q, 2, n);
                     }
                     for (int o = tid; o < H; o += OT)
-                        c[o] = online_update<ADA>(p, c[o], __fadd_rn(0.f, gp[o]), p.ada_mlp + w_off(k, H, l) + (size_t)H * nin + o);
+                        c[o] = online_update<SK>(p, c[o], __fadd_rn(0.f, gp[o]), p.ada_mlp + w_off(k, H, l) + (size_t)H * nin + o, 2, n);
                     __syncthreads();
                     if (l > 0) { for (int i = tid; i < H; i += OT) gp[i] = act[(l - 1) * H + i] > 0.f ? gx[i] : 0.f; }
                     else { for (int i = tid; i < k; i += OT) gbi[i] = gx[i]; }
@@ -201,9 +221,9 @@ __global__ void __launch_bounds__(OT) online_deep_kernel(OnlineParams p) {
                 } else {
                     g = __fadd_rn(0.f, __fmul_rn(d, x));
                 }
-                p.table[(size_t)id[f] * p.rowp + j] = online_update<ADA>(p, v, g, p.ada_sums + (size_t)id[f] * p.rowp + j);
+                p.table[(size_t)id[f] * p.rowp + j] = online_update<SK>(p, v, g, p.ada_sums + (size_t)id[f] * (SK == 2 ? 2 : 1) * p.rowp + j, 0, n);
             }
-            if (tid == 0) p.bias[0] = online_update<ADA>(p, p.bias[0], __fadd_rn(0.f, d), p.ada_bias);
+            if (tid == 0) p.bias[0] = online_update<SK>(p, p.bias[0], __fadd_rn(0.f, d), p.ada_bias, 1, n);
         } else {
             // hedge backpropagation, batch_size = 1: L backward passes, only the tower and alpha change
             const size_t nm = w_off(k, H, L);
@@ -269,7 +289,9 @@ static int ilog2_ceil(int x) { int l = 0; while ((1 << l) < x) ++l; return l; }
 // [fmb_mlp_numel] scratch, ONN only).  Outputs: preds [N] (the prediction made BEFORE fitting example i),
 // conf [4] = tp, fp, tn, fn (int64).
 // _ex: update mode 3 (Adagrad) of the Adam family (kinds 0-2) reads and writes the sums in `ada` (the table's, the
-// bias's and, with a tower, the tower's); the ONN kinds' hedge step uses no optimizer and ignores the mode.
+// bias's and, with a tower, the tower's); mode 4 (SparseAdam) takes an fmb_sparse_adam_t in the same slot whose steps_dev
+// holds the scalars of the N examples' steps (fmb_sparse_adam_online_steps).  The ONN kinds' hedge step uses no optimizer
+// and ignores the mode.
 struct fmb_adagrad_t { float* sums; float* bias_sum; float* mlp_sums; float eps; };   // include/fmb200.h
 FMB_API int fmb_online_deep_run_ex(int kind, const int32_t* ids, const float* xv, const float* y, int N, int F, int k,
                                    int L, int H, float* table, float* bias, float* mlp, float* alpha, float* acc,
@@ -283,6 +305,10 @@ FMB_API int fmb_online_deep_run_ex(int kind, const int32_t* ids, const float* xv
     FMB_CHECK_ARG(kind < 3 || (alpha && acc), "fmb_online_deep_run: ONN needs alpha and acc");
     FMB_CHECK_ARG(mode != 3 || kind >= 3 || (ada && ada->sums && ada->bias_sum && (kind == 0 || ada->mlp_sums)),
                   "fmb_online_deep_run: update mode 3 needs the Adagrad state (sums of the table, the bias and the tower)");
+    const fmb_sparse_adam_t* sa = mode == 4 && kind < 3 ? reinterpret_cast<const fmb_sparse_adam_t*>(ada) : nullptr;
+    FMB_CHECK_ARG(mode != 4 || kind >= 3 || (sa && sa->mv && sa->bias_mv && sa->steps_dev && (kind == 0 || sa->mlp_mv)),
+                  "fmb_online_deep_run: update mode 4 needs the SparseAdam state (moments of the table, the bias and the "
+                  "tower, and the examples' step scalars)");
     OnlineParams p;
     p.kind = kind; p.N = N; p.F = F; p.k = k; p.L = kind == 0 ? 0 : L; p.H = kind == 0 ? 0 : H;
     p.rowp = fmb_round_up(k + 1, 16); p.kp4 = fmb_round_up(k, 4); p.cu = (k + 1 + 3) / 4; p.ql_log = ilog2_ceil(p.cu);
@@ -290,17 +316,21 @@ FMB_API int fmb_online_deep_run_ex(int kind, const int32_t* ids, const float* xv
     p.lr = lr; p.hb = hb; p.hs = hs; p.mode = mode; p.preds = preds; p.conf = conf;
     p.ada_sums = p.ada_bias = p.ada_mlp = nullptr; p.eps = 0.f;
     if (mode == 3 && ada) { p.ada_sums = ada->sums; p.ada_bias = ada->bias_sum; p.ada_mlp = ada->mlp_sums; p.eps = ada->eps; }
+    if (sa) { p.ada_sums = sa->mv; p.ada_bias = sa->bias_mv; p.ada_mlp = sa->mlp_mv; p.sa_steps = sa->steps_dev; }
     const int mx = p.H > k ? p.H : k;
     const size_t fl = (size_t)F * p.cu * 4 + 2 * F + 2 * k + (size_t)p.L * p.H + 2 * mx + k + 2 * (p.L > 0 ? p.L : 1) + 16;
     const size_t smb = fl * sizeof(float);
     FMB_CHECK_ARG(smb <= 200 * 1024, "fmb_online_deep_run: model too large for one CTA's shared memory (F=%d k=%d L=%d H=%d: %zu bytes > 200 KB)",
                   F, k, p.L, p.H, smb);
     if (mode == 3 && kind < 3) {
-        cudaFuncSetAttribute(online_deep_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-        online_deep_kernel<true><<<1, OT, smb, stream>>>(p);
+        cudaFuncSetAttribute(online_deep_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+        online_deep_kernel<1><<<1, OT, smb, stream>>>(p);
+    } else if (sa) {
+        cudaFuncSetAttribute(online_deep_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+        online_deep_kernel<2><<<1, OT, smb, stream>>>(p);
     } else {
-        cudaFuncSetAttribute(online_deep_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-        online_deep_kernel<false><<<1, OT, smb, stream>>>(p);
+        cudaFuncSetAttribute(online_deep_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+        online_deep_kernel<0><<<1, OT, smb, stream>>>(p);
     }
     FMB_CHECK_LAUNCH("online_deep_kernel");
     return FMB_OK;

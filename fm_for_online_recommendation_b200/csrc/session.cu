@@ -28,9 +28,16 @@ int fmb_fm_step_fused_ex(const int32_t*, const float*, const float*, float*, con
 int fmb_is_fused_kernel_fn(const void*);
 const void* fmb_finish_kernel_fn(void);
 int fmb_sort_fields_kernel_fns(const void**, int*, int*);
+int fmb_sparse_adam_advance(fmb_sparse_adam_t*, float, int);
 }
 int fmb_fm_backward_runs_list_launch(const int32_t*, int64_t, float*, int, int, float, int, const fmb_ftrl_t*,
                                      const fmb_runlist_t*, void*, size_t, bool pdl, cudaStream_t);   // fm_backward.cu
+// update mode 4: the kernels whose by-value arguments carry a step's scalars, and copies of those arguments with the
+// scalars of fmb_sparse_adam_t::cur (fm_step.cu, fm_backward.cu, dense_ops.cu)
+void fmb_fused_params_sa(const void* src, void* dst, const fmb_sparse_adam_t* a);
+void fmb_runs_params_sa(const void* src, void* dst, const fmb_sparse_adam_t* a);
+const void* fmb_runs_list_sa_kernel_fn();
+const void* fmb_finish_sa_kernel_fn();
 
 // One captured step graph per CONFIGURATION (batch size, loss, update mode, with/without xv, sorted in the step or
 // before it, with/without the sort of the next batch riding along) -- never per batch: the per-batch pointers
@@ -44,6 +51,7 @@ struct StepVariant {
     cudaGraph_t graph;        // kept alive: its nodes own the argument storage the patches start from
     cudaGraphExec_t exec;
     cudaGraphNode_t n_fused, n_finish, n_sort_cur[2], n_sort_next[2];   // a per-field sort is up to two kernels (radix + sparse fields)
+    cudaGraphNode_t n_runs;   // the run-list kernel (re-pointed at every step's scalars in mode 4)
     int np_sort_cur[2], np_sort_next[2];
     int nlaunch;
     // per-batch pointers the nodes currently hold: a node is only re-pointed when its pointers change (a host loop over
@@ -116,6 +124,7 @@ struct fmb_session {
     int ftrl_set;
     fmb_adagrad_t ada;     // update mode 3 (fmb_session_set_adagrad)
     int ada_set;
+    fmb_sparse_adam_t* sa; // update mode 4 (fmb_session_set_sparse_adam): the caller's state, advanced by every step
 };
 
 #define CU(call)                                                                              \
@@ -270,6 +279,19 @@ FMB_API int fmb_session_set_adagrad(fmb_session* s, float* sums_dev, float* bias
     return FMB_OK;
 }
 
+// update mode 4 (SparseAdam on the tables, Adam on the bias): the caller's state, which must outlive the session or the
+// next call of this function.  Every mode-4 step of the session advances it (fmb_sparse_adam_advance, tower = 0) when it
+// is submitted and takes that step's scalars by value, so host pipelines that submit several steps ahead stay exact.  The
+// step graphs stay one per configuration: the scalars reach them through the per-launch kernel-node updates.  Step graphs
+// captured before this call are dropped.
+FMB_API int fmb_session_set_sparse_adam(fmb_session* s, fmb_sparse_adam_t* a) {
+    FMB_CHECK_ARG(s && a && a->mv && a->bias_mv && a->eps >= 0.f, "fmb_session_set_sparse_adam: bad arguments");
+    s->sa = a;
+    for (int i = 0; i < s->ngraphs; ++i) { cudaGraphExecDestroy(s->gvar[i].exec); cudaGraphDestroy(s->gvar[i].graph); }
+    s->ngraphs = 0; s->next_evict = 0;
+    return FMB_OK;
+}
+
 FMB_API int64_t fmb_session_launches(const fmb_session* s) { return s ? s->launches : 0; }
 FMB_API int fmb_session_graph_count(const fmb_session* s) { return s ? s->ngraphs : 0; }
 
@@ -339,8 +361,10 @@ static int fm_step_launch(fmb_session* s, const int32_t* ids, const float* xv, c
         rc = sort_launch(s, ids, B, key_bits, cur, s->d_sort_ws, main, nlaunch);
         if (rc) return rc;
     }
-    // the state slot of the step's kernels: the FTRL state, or in mode 3 the Adagrad state (include/fmb200.h)
+    // the state slot of the step's kernels: the FTRL state, in mode 3 the Adagrad state, in mode 4 the SparseAdam state
+    // (include/fmb200.h)
     const fmb_ftrl_t* ft = mode == 3 ? (s->ada_set ? reinterpret_cast<const fmb_ftrl_t*>(&s->ada) : nullptr)
+                         : mode == 4 ? reinterpret_cast<const fmb_ftrl_t*>(s->sa)
                                      : (s->ftrl_set ? &s->ftrl : nullptr);
     rc = fmb_fm_step_fused_ex(ids, xv, y, table, bias, s->d_posflag_buf[cur], B, s->F, s->k, loss_kind, lr, mode, ft,
                               s->d_delta, s->d_lossv, s->d_bwd_ws, s->bwd_ws_bytes, main);
@@ -364,16 +388,28 @@ static int fm_step_launch(fmb_session* s, const int32_t* ids, const float* xv, c
 }
 
 // re-point one kernel node of an instantiated step graph at new per-batch pointers: argument i of the node is
-// replaced by *repl[i] wherever repl[i] != NULL; the other arguments keep the values captured in `graph`.
-static int patch_node(cudaGraphExec_t exec, cudaGraphNode_t node, int nparams, const void* const* repl) {
+// replaced by *repl[i] wherever repl[i] != NULL; the other arguments keep the values captured in `graph`.  sa_edit
+// (nullable, update mode 4): argument sa_arg becomes sa_edit's copy of the captured one with the scalars of s->sa->cur.
+typedef void (*sa_edit_fn)(const void* src, void* dst, const fmb_sparse_adam_t* a);
+static int patch_node(cudaGraphExec_t exec, cudaGraphNode_t node, int nparams, const void* const* repl,
+                      sa_edit_fn sa_edit = nullptr, int sa_arg = 0, const fmb_sparse_adam_t* sa = nullptr) {
     cudaKernelNodeParams kp;
     CU(cudaGraphKernelNodeGetParams(node, &kp));
     void* args[16];
+    alignas(16) unsigned char edited[512];
     for (int i = 0; i < nparams; ++i) args[i] = repl[i] ? const_cast<void*>(repl[i]) : kp.kernelParams[i];
+    if (sa_edit) { sa_edit(kp.kernelParams[sa_arg], edited, sa); args[sa_arg] = edited; }
     kp.kernelParams = args;
     kp.extra = nullptr;
     CU(cudaGraphExecKernelNodeSetParams(exec, node, &kp));
     return FMB_OK;
+}
+
+// the bias step's state argument (fmb::UpdateState) with the bias's Adam scalars of this step
+static void finish_params_sa(const void* src, void* dst, const fmb_sparse_adam_t* a) {
+    fmb::UpdateState u = *static_cast<const fmb::UpdateState*>(src);
+    u.adam.step = a->cur.bias_step; u.adam.bc2s = a->cur.bias_bc2s;
+    *static_cast<fmb::UpdateState*>(dst) = u;
 }
 
 static int capture_variant(fmb_session* s, StepVariant* v, const int32_t* ids, const float* xv, const float* y,
@@ -393,7 +429,7 @@ static int capture_variant(fmb_session* s, StepVariant* v, const int32_t* ids, c
     const void* sort_fns[8];
     int sort_np[8], sort_ska[8];
     const int nsort = fmb_sort_fields_kernel_fns(sort_fns, sort_np, sort_ska);
-    v->n_fused = v->n_finish = nullptr;
+    v->n_fused = v->n_finish = v->n_runs = nullptr;
     for (int j = 0; j < 2; ++j) v->n_sort_cur[j] = v->n_sort_next[j] = nullptr;
     for (size_t i = 0; i < nn; ++i) {
         cudaGraphNodeType ty;
@@ -402,7 +438,8 @@ static int capture_variant(fmb_session* s, StepVariant* v, const int32_t* ids, c
         cudaKernelNodeParams kp;
         CU(cudaGraphKernelNodeGetParams(nodes[i], &kp));
         if (fmb_is_fused_kernel_fn(kp.func)) { v->n_fused = nodes[i]; continue; }
-        if (kp.func == fmb_finish_kernel_fn()) { v->n_finish = nodes[i]; continue; }
+        if (kp.func == fmb_finish_kernel_fn() || kp.func == fmb_finish_sa_kernel_fn()) { v->n_finish = nodes[i]; continue; }
+        if (kp.func == fmb_runs_list_sa_kernel_fn()) { v->n_runs = nodes[i]; continue; }
         for (int t = 0; t < nsort; ++t)
             if (kp.func == sort_fns[t]) {
                 const int32_t* out = *static_cast<int32_t**>(kp.kernelParams[sort_ska[t]]);   // sorted_keys argument
@@ -413,7 +450,8 @@ static int capture_variant(fmb_session* s, StepVariant* v, const int32_t* ids, c
                 dst[j] = nodes[i]; dnp[j] = sort_np[t];
             }
     }
-    if (!v->n_fused || !v->n_finish || (!v->pre && !v->n_sort_cur[0]) || (v->has_next && !v->n_sort_next[0])) {
+    if (!v->n_fused || !v->n_finish || (!v->pre && !v->n_sort_cur[0]) || (v->has_next && !v->n_sort_next[0]) ||
+        (v->mode == 4 && !v->n_runs)) {
         cudaGraphDestroy(graph);
         fmb_set_error("step graph: kernel nodes not found");
         return FMB_ERR_CUDA;
@@ -441,6 +479,8 @@ static int session_fm_step(fmb_session* s, const int32_t* ids, const float* xv, 
                            float* loss_dev, cudaStream_t stream, bool graph_per_input) {
     FMB_CHECK_ARG(s && ids && y && table && bias, "fmb_session_fm_step: null pointer");
     FMB_CHECK_ARG(B > 0 && B <= s->maxB, "fmb_session_fm_step: B=%d exceeds session max_batch", B);
+    FMB_CHECK_ARG(mode != 4 || s->sa, "fmb_session_fm_step: update mode 4 (SparseAdam) needs fmb_session_set_sparse_adam");
+    if (mode == 4) fmb_sparse_adam_advance(s->sa, lr, 0);   // this step's scalars, taken by value below
     int nl = 0;
     // sorted form of this batch: already produced by a previous call (next_ids / fmb_session_presort), or sorted here
     const bool pre = s->presort_ids == ids && s->presort_B == B && !s->presort_stale;
@@ -494,12 +534,18 @@ static int session_fm_step(fmb_session* s, const int32_t* ids, const float* xv, 
             s->gvar[slot] = key;
             v = &s->gvar[slot];
         }
-        if (v->cur_ids != ids || v->cur_xv != xv || v->cur_y != y) {
+        const bool sa = mode == 4;   // mode 4: the fused, run-list and bias-step nodes take this step's scalars
+        if (sa || v->cur_ids != ids || v->cur_xv != xv || v->cur_y != y) {
             const void* repl[16] = {nullptr};
             repl[0] = &ids; repl[1] = &xv; repl[2] = &y;
-            rc = patch_node(v->exec, v->n_fused, 5, repl);
+            rc = sa ? patch_node(v->exec, v->n_fused, 5, repl, fmb_fused_params_sa, 4, s->sa) : patch_node(v->exec, v->n_fused, 5, repl);
             if (rc) return rc;
             v->cur_ids = ids; v->cur_xv = xv; v->cur_y = y;
+        }
+        if (sa) {
+            const void* repl[16] = {nullptr};
+            rc = patch_node(v->exec, v->n_runs, 11, repl, fmb_runs_params_sa, 2, s->sa);
+            if (rc) return rc;
         }
         if (!pre && v->cur_sort_ids != ids) {
             const void* repl[16] = {nullptr};
@@ -522,10 +568,10 @@ static int session_fm_step(fmb_session* s, const int32_t* ids, const float* xv, 
         {   // the bias-step kernel writes the mean loss straight to the caller's scalar (a 4-byte copy behind every graph
             // launch was a stream operation of its own: ~4 us of bubble per step)
             float* lo = loss_dev ? loss_dev : s->d_loss;
-            if (v->cur_loss != lo) {
+            if (sa || v->cur_loss != lo) {
                 const void* repl[16] = {nullptr};
                 repl[6] = &lo;
-                rc = patch_node(v->exec, v->n_finish, 9, repl);
+                rc = sa ? patch_node(v->exec, v->n_finish, 9, repl, finish_params_sa, 8, s->sa) : patch_node(v->exec, v->n_finish, 9, repl);
                 if (rc) return rc;
                 v->cur_loss = lo;
             }

@@ -455,6 +455,7 @@ FMB_API int fmb_shard2_owner_apply(const int32_t* keys_all, const float* inbox, 
                                    const uint32_t* wait_flags, const uint32_t* wait_epoch_words, int wait_channel,
                                    int* error, cudaStream_t stream) {
     FMB_CHECK_ARG(inbox && cnt && list && nlist && (parity == 0 || parity == 1), "fmb_shard2_owner_apply: null pointer");
+    FMB_CHECK_ARG(mode != 4, "fmb_shard2_owner_apply: update mode 4 (SparseAdam) is not supported by the sharded step");
     FMB_CHECK_ARG(mode == 0 || mode == 1, "fmb_shard2_owner_apply: unknown update mode %d", mode);
     OwnerParams p;
     if (int rc = fill_owner(p, keys_all, inbox, table, cnt, nullptr, hot, hot_base, field_off, G, me, B, F, k, lr, mode)) return rc;

@@ -348,6 +348,7 @@ FMB_API int fmb_shard3_step(const int32_t* idsT_all, float* table_local, const f
                   ctx_local && tflags_local && epoch_dev && error_dev, "fmb_shard3_step: null pointer");
     const int T = fmb_shard3_tiles(G, B, F, k);
     FMB_CHECK_ARG(T > 0 && me >= 0 && me < G && cap > 0, "fmb_shard3_step: unsupported shape G=%d B=%d F=%d k=%d", G, B, F, k);
+    FMB_CHECK_ARG(mode != 4, "fmb_shard3_step: update mode 4 (SparseAdam) is not supported by the sharded step");
     FMB_CHECK_ARG(mode == 0 || mode == 1, "fmb_shard3_step: unknown update mode %d", mode);
     const int64_t N = (int64_t)F * cap;
     if (ws_bytes < fmb_bwd_workspace_bytes(N, k)) { fmb_set_error("fmb_shard3_step: workspace too small"); return FMB_ERR_WS; }

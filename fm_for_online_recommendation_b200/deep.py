@@ -23,10 +23,12 @@ import torch
 import torch.nn as nn
 
 from . import _lib
-from ._lib import AdagradState, FmbError, RunList, check, ptr
+from ._lib import AdagradState, FmbError, RunList, SparseAdamState, check, ptr
 
 UPDATE_ADAM1, UPDATE_SGD, UPDATE_FTRL = 0, 1, 2   # 2: per-coordinate FTRL-Proximal (enable_ftrl), FM-only steps
 UPDATE_ADAGRAD = 3   # torch.optim.Adagrad with state kept across calls (enable_adagrad): FM steps, tower fit, run_experiment
+UPDATE_SPARSE_ADAM = 4   # torch.optim.SparseAdam on the tables + torch.optim.Adam on the bias and the tower, state kept
+                         # across calls (enable_sparse_adam): FM steps, tower fit, run_experiment
 LOSS_LOGITS, LOSS_LOGITS_OF_SIG = 0, 1
 
 
@@ -159,8 +161,11 @@ class _DeepBase(nn.Module):
         self._presorted = None   # the EncodedBatch whose sorted form the session holds (kept alive: its ids pointer is the key)
         self._ws = {}
         self._ada = None
+        self._sa = None
         if update_mode == UPDATE_ADAGRAD:
             self.enable_adagrad()
+        elif update_mode == UPDATE_SPARSE_ADAM:
+            self.enable_sparse_adam()
 
     def _bind_embeddings(self):
         k = self.embedding_size
@@ -203,6 +208,10 @@ class _DeepBase(nn.Module):
         if self.update_mode == UPDATE_ADAGRAD:
             st["adagrad"] = {"eps": self._ada_eps, "sums": _f32(self._ada_sums), "bias_sum": _f32(self._ada_bias),
                              "mlp_sums": _f32(self._ada_mlp)}
+        if self.update_mode == UPDATE_SPARSE_ADAM:
+            a = self._sa
+            st["sparse_adam"] = {"betas": (a.beta1, a.beta2), "eps": a.eps, "step": a.step, "mlp_step": a.mlp_step,
+                                 "mv": _f32(self._sa_mv), "bias_mv": _f32(self._sa_bias), "mlp_mv": _f32(self._sa_mlp)}
         return st
 
     def _load_packed_state(self, st):
@@ -221,6 +230,15 @@ class _DeepBase(nn.Module):
                 self._ada_bias.copy_(ada["bias_sum"])
                 if self._ada_mlp is not None:
                     self._ada_mlp.copy_(ada["mlp_sums"])
+        sa = st.get("sparse_adam")
+        if sa is not None:
+            self.enable_sparse_adam(betas=sa["betas"], eps=sa["eps"])
+            self._sa.step, self._sa.mlp_step = sa["step"], sa["mlp_step"]
+            with torch.no_grad():
+                self._sa_mv.copy_(sa["mv"])
+                self._sa_bias.copy_(sa["bias_mv"])
+                if self._sa_mlp is not None:
+                    self._sa_mlp.copy_(sa["mlp_mv"])
 
     def __reduce__(self):  # pickle.dump(model) (main_experiment.py:160-162): one copy of the table, no handles
         return (_rebuild, (type(self), self._ctor_kwargs(), self._export_state()))
@@ -315,9 +333,39 @@ class _DeepBase(nn.Module):
         if self._session is not None:
             self._bind_adagrad()
 
+    def enable_sparse_adam(self, betas=(0.9, 0.999), eps=1e-8):
+        """Switch update_embedding, fit (FMAdam / DeepFMAdam / NFMAdam) and run_experiment to Adam with its moments kept
+        across calls: the same trajectory as ONE `torch.optim.SparseAdam(<embedding tables>, lr=n, betas, eps)` stepped on
+        the sparse gradient of the rows each batch hits (nn.Embedding(sparse=True)'s, summed in sample order) and ONE
+        `torch.optim.Adam([bias] + <tower>, lr=n, betas, eps)`.  Every row a batch hits steps, also when its gradient is
+        zero; the other rows keep their weights and moments.  The tables and the bias count every step, the tower only
+        the steps that give it a gradient (fit, run_experiment), as torch does.  Calling this again resets the moments and
+        both counters.  The ONN classes' hedge fit uses no optimizer and stays as it is."""
+        b1, b2 = (float(b) for b in betas)
+        if not (0.0 <= b1 < 1.0 and 0.0 <= b2 < 1.0) or eps < 0:
+            raise ValueError("need 0 <= beta1, beta2 < 1 and eps >= 0")
+        self.update_mode = UPDATE_SPARSE_ADAM
+        self._sa_mv = torch.zeros((self._R, 2, self._rowp), dtype=torch.float32, device=self.device)
+        self._sa_bias = torch.zeros((2,), dtype=torch.float32, device=self.device)
+        self._sa_mlp = None if self._mlp is None else torch.zeros((2, self._mlp.numel()), dtype=torch.float32,
+                                                                  device=self.device)
+        self._sa = SparseAdamState(self._sa_mv.data_ptr(), self._sa_bias.data_ptr(),
+                                   None if self._sa_mlp is None else self._sa_mlp.data_ptr(), b1, b2, float(np.float32(eps)),
+                                   0, 0)
+        self.__dict__.pop("_fit_graphs", None)
+        if self._session is not None:
+            self._bind_sparse_adam()
+
+    def _bind_sparse_adam(self):
+        check(self._lib.fmb_session_set_sparse_adam(self._session, C.byref(self._sa)), "fmb_session_set_sparse_adam")
+
     def _ada_arg(self):
-        """the fmb_adagrad_t of the C entry points' state slot in mode 3, else NULL"""
-        return C.byref(self._ada) if self.update_mode == UPDATE_ADAGRAD and self._ada is not None else None
+        """the state slot of the C entry points: fmb_adagrad_t in mode 3, fmb_sparse_adam_t in mode 4, else NULL"""
+        if self.update_mode == UPDATE_ADAGRAD and self._ada is not None:
+            return C.byref(self._ada)
+        if self.update_mode == UPDATE_SPARSE_ADAM and self._sa is not None:
+            return C.byref(self._sa)
+        return None
 
     def _bind_adagrad(self):
         check(self._lib.fmb_session_set_adagrad(self._session, ptr(self._ada_sums), ptr(self._ada_bias), self._ada_eps),
@@ -339,6 +387,8 @@ class _DeepBase(nn.Module):
                 self._bind_ftrl()
             elif self.update_mode == UPDATE_ADAGRAD:
                 self._bind_adagrad()
+            elif self.update_mode == UPDATE_SPARSE_ADAM:
+                self._bind_sparse_adam()
         return self._session
 
     def _buf(self, name, shape, dtype=torch.float32):
@@ -498,14 +548,20 @@ class _DeepBase(nn.Module):
         N = B * F
         bwsb = lib.fmb_bwd_workspace_bytes(N, k)
         bws = self._buf("bwd_ws", (bwsb,), torch.uint8)
-        ada = self._ada_arg()   # the _ex forms are the plain ones outside mode 3
+        ada = self._ada_arg()   # the _ex forms are the plain ones outside modes 3 and 4
+        sa = self.update_mode == UPDATE_SPARSE_ADAM
+        if sa:
+            check(lib.fmb_sparse_adam_advance(ada, self._lr, 1), "fmb_sparse_adam_advance")
         check(lib.fmb_fm_backward_update_rl_ex(ptr(sk), ptr(pm), N, N, ptr(e.xv), ptr(self._table), F, k, ptr(o["S"]),
                                                self._kp4, ptr(delta), 1, 0 if self._IS_NFM else 1, ptr(gbi), 0x7FFFFFFF,
                                                self._lr, self.update_mode, ada, C.byref(rl) if rl is not None else None,
                                                ptr(bws), bwsb, st), "fmb_fm_backward_update")
-        check(lib.fmb_update_dense_ex(ptr(self._mlp), ptr(gmlp), self._mlp.numel(), self._lr, self.update_mode,
-                                      ptr(self._ada_mlp) if ada else None, self._ada_eps if ada else 0.0, st),
-              "fmb_update_dense")
+        if sa:
+            check(lib.fmb_update_dense_adam(ptr(self._mlp), ptr(gmlp), self._mlp.numel(), ada, st), "fmb_update_dense_adam")
+        else:
+            check(lib.fmb_update_dense_ex(ptr(self._mlp), ptr(gmlp), self._mlp.numel(), self._lr, self.update_mode,
+                                          ptr(self._ada_mlp) if ada else None, self._ada_eps if ada else 0.0, st),
+                  "fmb_update_dense")
         check(lib.fmb_finish_step_ex(ptr(delta), None, B, ptr(self.bias), self._lr, self.update_mode, ada, None, st),
               "fmb_finish_step")
 
@@ -513,7 +569,8 @@ class _DeepBase(nn.Module):
         """_deep_fit as ONE CUDA graph per configuration: the step is ~25 kernel launches through ctypes, which the host
         submits more slowly than the GPU runs them at cfg4's shapes.  First call of a configuration: eager (allocations,
         function attributes); second: captured on static input buffers; afterwards: copy the batch in, replay."""
-        if torch.cuda.is_current_stream_capturing():
+        # mode 4: every step has scalars of its own (taken by value at launch), so it is not replayed from a graph
+        if torch.cuda.is_current_stream_capturing() or self.update_mode == UPDATE_SPARSE_ADAM:
             return self._deep_fit(e)
         key = (e.B, e.xv is not None, self._lr, self.update_mode, int(self._lib.fmb_tensor_cores_enabled()))
         graphs = self.__dict__.setdefault("_fit_graphs", {})
@@ -657,6 +714,13 @@ class _DeepBase(nn.Module):
         preds_dev = torch.empty(data_size, dtype=torch.uint8, device=self.device)
         conf_dev = torch.zeros(4, dtype=torch.int64, device=self.device)
         acc = self._buf("hedge_acc", (self._mlp.numel(),)) if self._IS_ONN else None
+        if self.update_mode == UPDATE_SPARSE_ADAM and not self._IS_ONN:
+            # the scalars of the data_size single-example steps, filled on the host (one row per example)
+            tab = torch.empty(4 + 5 * data_size, dtype=torch.float32)
+            check(self._lib.fmb_sparse_adam_online_steps(C.byref(self._sa), self._lr, int(self._HAS_MLP), data_size,
+                                                         tab.data_ptr()), "fmb_sparse_adam_online_steps")
+            steps_dev = tab.to(self.device)
+            self._sa.steps_dev = steps_dev.data_ptr()
         check(self._lib.fmb_online_deep_run_ex(self._KIND_ID, ptr(enc.ids), ptr(enc.xv), ptr(enc.y), data_size,
                                                self.field_size, self.embedding_size, self._L, self._H, ptr(self._table),
                                                ptr(self.bias), ptr(self._mlp), ptr(getattr(self, "alpha", None)),

@@ -43,6 +43,8 @@ typedef struct fmb_session fmb_session;
 #define FMB_UPDATE_SGD 1   /* p -= lr * g (legacy notebooks' torch.optim.SGD; SURVEY.md 8f.4) */
 #define FMB_UPDATE_FTRL 2  /* per-coordinate FTRL-Proximal, FM-only steps (fmb_ftrl_t below) */
 #define FMB_UPDATE_ADAGRAD 3 /* torch.optim.Adagrad with persistent per-coordinate sums (fmb_adagrad_t below) */
+#define FMB_UPDATE_SPARSE_ADAM 4 /* torch.optim.SparseAdam on the tables, torch.optim.Adam on the bias and the tower,
+                                    moments kept across calls (fmb_sparse_adam_t below) */
 
 /* loss variants (SURVEY.md A6) */
 #define FMB_LOSS_BCE_LOGITS 0         /* F.binary_cross_entropy_with_logits(z, y) */
@@ -196,6 +198,37 @@ typedef struct fmb_ftrl_t { float* zn_dev; float* bias_zn_dev; float beta, l1, l
  * there in mode 3: pass (const fmb_ftrl_t*)&adagrad.  Algorithmic bytes of the FM step grow by 8F(k+1) per sample.
  * Sharded steps, AFM and fmb_fm_backward_runs_all reject mode 3. */
 typedef struct fmb_adagrad_t { float* sums_dev; float* bias_sum_dev; float* mlp_sums_dev; float eps; } fmb_adagrad_t;
+/* update mode 4: torch.optim.SparseAdam(betas, eps, lr = the step's lr) on the embedding tables -- only the rows a batch
+ * hits update their moments and weights, a zero gradient of such a row included -- and torch.optim.Adam(betas, eps) on the
+ * bias and the tower, both kept across calls.  Per coordinate, as torch 2.11's CPU kernels round it:
+ *   SparseAdam: u1 = (g - m)*(1-b1); m' = m + u1; u2 = (g*g - v)*(1-b2); v' = v + u2;  p' = p + s_e * (m' / (sqrt(v') + eps))
+ *   Adam:       m' = fma(1-b1, g - m, m); v' = fma((1-b2)*g, g, v*b2);  p' = p + (s_d * m') / (sqrt(v') / c2 + eps)
+ * with the step's float scalars s_e = -lr*sqrt(1-b2^t)/(1-b1^t), s_d = -lr/(1-b1^t), c2 = (1-b2^t)^0.5, computed in double
+ * on the host and rounded to float (fmb_adam_scalars).  The tables and the bias count every step (`step`); the tower counts
+ * only the steps that give it a gradient (`mlp_step`: tower fit, run_experiment), as torch skips a parameter whose .grad
+ * is None.  mv_dev [R][2][rowp]: m and v sub-rows of every packed table row (FTRL's layout; padding never written);
+ * bias_mv_dev [2]; mlp_mv_dev [2][fmb_mlp_numel] (m, then v) or NULL.  Zero-fill the moments and counters to start.
+ * The entry points with a state slot take it there (pass (const fmb_ftrl_t*)&sa), advanced to the step being run by
+ * fmb_sparse_adam_advance; a session step advances it itself (fmb_session_set_sparse_adam).  Algorithmic bytes of the FM
+ * step grow by 16F(k+1) per sample.  Sharded steps, AFM and fmb_fm_backward_runs_all reject mode 4. */
+typedef struct fmb_adam_step_t { float emb_step, bias_step, bias_bc2s, mlp_step, mlp_bc2s; } fmb_adam_step_t;
+typedef struct fmb_sparse_adam_t {
+    float* mv_dev; float* bias_mv_dev; float* mlp_mv_dev;
+    double beta1, beta2;
+    float eps;
+    int64_t step, mlp_step;     /* steps taken so far */
+    fmb_adam_step_t cur;        /* the scalars of the step being run */
+    const float* steps_dev;     /* fmb_online_deep_run_ex: the examples' scalars (fmb_sparse_adam_online_steps) */
+} fmb_sparse_adam_t;
+/* out[0] = s_e, out[1] = s_d, out[2] = c2 of step t (float), from lr and the betas in double as CPython computes them */
+void fmb_adam_scalars(float lr, double beta1, double beta2, int64_t t, float* out);
+/* ++step (and ++mlp_step when tower != 0); fills cur */
+int fmb_sparse_adam_advance(fmb_sparse_adam_t* sa, float lr, int tower);
+/* the scalars of N single-example steps of fmb_online_deep_run_ex into out_host [4 + 5N] ((1-b1, b2, 1-b2, eps), then one
+ * fmb_adam_step_t per example), advancing the counters by N; copy it to the device and point steps_dev at it */
+int fmb_sparse_adam_online_steps(fmb_sparse_adam_t* sa, float lr, int tower, int N, float* out_host);
+/* mode 4's Adam step of the tower's n parameters (mlp_mv_dev and cur.mlp_*) */
+int fmb_update_dense_adam(float* p_dev, const float* g_dev, int64_t n, const fmb_sparse_adam_t* sa, fmb_stream_t stream);
 int fmb_fm_step_fused_ex(const int32_t* ids_dev, const float* xv_dev, const float* y_dev, float* table_dev,
                          const float* bias_dev, const uint32_t* posflag_dev, int B, int F, int k, int loss_kind, float lr,
                          int mode, const fmb_ftrl_t* ftrl, float* delta_dev, float* lossv_dev, void* ws_dev,
@@ -246,7 +279,8 @@ int fmb_fm_backward_update_rl(const int32_t* sorted_keys_dev, const int32_t* per
                               float lr, int mode, const fmb_runlist_t* rl, void* ws_dev, size_t ws_bytes,
                               fmb_stream_t stream);
 
-/* _rl_ex: update mode 3 needs `ada` (its sums_dev; NULL in the other modes) -- the tower fit's backward */
+/* _rl_ex: update mode 3 needs `ada` (its sums_dev), mode 4 an fmb_sparse_adam_t in the same slot (cast), advanced to the
+ * step; NULL in the other modes -- the tower fit's backward */
 int fmb_fm_backward_update_rl_ex(const int32_t* sorted_keys_dev, const int32_t* perm_dev, int64_t N, int64_t n_entries,
                                  const float* xv_dev, float* table_dev, int F, int k, const float* S_dev, int s_pitch,
                                  const float* gs_dev, int gs_stride, int use_fm2, const float* gvec_dev, int32_t key_limit,
@@ -423,7 +457,8 @@ int fmb_online_deep_run(int kind, const int32_t* ids_dev /*[N,F]*/, const float*
                         float* alpha_dev, float* acc_dev /*[fmb_mlp_numel], ONN*/, float lr, float hb, float hs,
                         int mode, uint8_t* preds_dev, int64_t* conf_dev, fmb_stream_t stream);
 /* _ex: update mode 3 of kinds 0-2 reads and writes the sums of `ada` (table, bias and, with a tower, the tower's); the
- * ONN kinds' hedge step uses no optimizer and ignores the mode.  fmb_online_deep_run rejects mode 3 for kinds 0-2. */
+ * ONN kinds' hedge step uses no optimizer and ignores the mode.  fmb_online_deep_run rejects mode 3 for kinds 0-2.  Mode 4
+ * takes an fmb_sparse_adam_t in the same slot (cast) whose steps_dev holds the N examples' scalars. */
 int fmb_online_deep_run_ex(int kind, const int32_t* ids_dev, const float* xv_dev, const float* y_dev, int N, int F, int k,
                            int L, int H, float* table_dev, float* bias_dev, float* mlp_dev, float* alpha_dev,
                            float* acc_dev, float lr, float hb, float hs, int mode, const fmb_adagrad_t* ada,
@@ -470,6 +505,9 @@ int fmb_session_presort(fmb_session* s, const int32_t* ids_dev, int B, int key_b
 int fmb_session_set_ftrl(fmb_session* s, float* zn_dev, float* bias_zn_dev, float beta, float l1, float l2);
 /* Adagrad state of the session's steps (update mode 3): sums_dev [R][rowp], bias_sum_dev [1], filled by the caller */
 int fmb_session_set_adagrad(fmb_session* s, float* sums_dev, float* bias_sum_dev, float eps);
+/* SparseAdam state of the session's steps (update mode 4): the caller's struct, kept by pointer; every mode-4 step
+ * advances it (tower = 0) when submitted and takes that step's scalars by value */
+int fmb_session_set_sparse_adam(fmb_session* s, fmb_sparse_adam_t* sa);
 /* forget a pending pre-sort (the caller cannot vouch that the pre-sorted ids buffer still holds the same batch) */
 void fmb_session_presort_invalidate(fmb_session* s);
 /* fmb_session_fm_step with the sort of the NEXT batch riding along: next_ids_dev (nullable) are the ids the
