@@ -388,7 +388,7 @@ constexpr size_t tc_smem_bytes() { return (size_t)2 * (2 * KCH * (TBM * 16 + 16)
 }  // namespace
 
 static int* g_tc_error = nullptr;
-static float* g_tc_ws = nullptr;
+static float* g_tc_ws = nullptr;   // split-K workspace; a grown one replaces it but none is freed (fmb_gemm_tc_launch)
 static size_t g_tc_ws_bytes = 0;
 static int g_tc_sms = 0;
 
@@ -425,11 +425,14 @@ int fmb_gemm_tc_launch(const float* A, int64_t sam, int64_t sak, const float* B,
     if (splits > 1) {
         const size_t need = ((size_t)splits * M * N + (size_t)splits * M) * sizeof(float);
         if (need > g_tc_ws_bytes) {
-            cudaStreamSynchronize(stream);   // earlier launches may still read the old buffer
-            if (g_tc_ws) cudaFree(g_tc_ws);
-            g_tc_ws = nullptr; g_tc_ws_bytes = 0;
-            if (cudaMalloc(&g_tc_ws, need) != cudaSuccess) { fmb_set_error("gemm_tc: cannot allocate %zu workspace bytes", need); return FMB_ERR_CUDA; }
-            g_tc_ws_bytes = need;
+            // the superseded buffer stays allocated for the life of the process: launches still in flight and CUDA
+            // graphs captured earlier (deep.py's fit graphs) hold its address.  Each new buffer is at least twice the
+            // last, so the kept ones total less than the current one.
+            const size_t bytes = need > 2 * g_tc_ws_bytes ? need : 2 * g_tc_ws_bytes;
+            float* grown = nullptr;
+            if (cudaMalloc(&grown, bytes) != cudaSuccess) { fmb_set_error("gemm_tc: cannot allocate %zu workspace bytes", bytes); return FMB_ERR_CUDA; }
+            g_tc_ws = grown;
+            g_tc_ws_bytes = bytes;
         }
         p.ws = g_tc_ws;
         p.wsc = g_tc_ws + (size_t)splits * M * N;

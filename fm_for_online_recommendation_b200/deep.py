@@ -395,6 +395,13 @@ class _DeepBase(nn.Module):
         t = self._ws.get(name)
         n = int(np.prod(shape))
         if t is None or t.numel() < n or t.dtype != dtype:
+            if t is not None:
+                # the fit graphs captured so far point into the buffer this one replaces, which goes back to torch's
+                # allocator: drop them, the next calls capture again.  A capture re-runs a configuration whose eager
+                # call already sized every buffer, so it never gets here.
+                if torch.cuda.is_current_stream_capturing():
+                    raise RuntimeError(f"workspace '{name}' would grow inside a CUDA graph capture")
+                self.__dict__.pop("_fit_graphs", None)
             t = torch.empty(max(n, 1), dtype=dtype, device=self.device)
             self._ws[name] = t
         return t[:n].view(*shape)
@@ -573,11 +580,10 @@ class _DeepBase(nn.Module):
         if torch.cuda.is_current_stream_capturing() or self.update_mode == UPDATE_SPARSE_ADAM:
             return self._deep_fit(e)
         key = (e.B, e.xv is not None, self._lr, self.update_mode, int(self._lib.fmb_tensor_cores_enabled()))
-        graphs = self.__dict__.setdefault("_fit_graphs", {})
-        ent = graphs.get(key)
+        ent = self.__dict__.get("_fit_graphs", {}).get(key)
         if ent is None:
-            self._deep_fit(e)
-            graphs[key] = "warm"
+            self._deep_fit(e)   # may grow a workspace, which drops every graph captured so far (_buf)
+            self.__dict__.setdefault("_fit_graphs", {})[key] = "warm"
             return
         if ent == "warm":
             se = EncodedBatch(torch.empty_like(e.ids), None if e.xv is None else torch.empty_like(e.xv), torch.empty_like(e.y))
@@ -585,7 +591,7 @@ class _DeepBase(nn.Module):
             torch.cuda.synchronize()
             with torch.cuda.graph(g):
                 self._deep_fit(se)
-            ent = graphs[key] = (g, se)
+            ent = self._fit_graphs[key] = (g, se)
         g, se = ent
         se.ids.copy_(e.ids, non_blocking=True)
         if se.xv is not None:
@@ -645,11 +651,10 @@ class _DeepBase(nn.Module):
         if torch.cuda.is_current_stream_capturing() or not self._hedge_single_pass(e.B):
             return self._hedge_fit(e)
         key = ("hedge", e.B, e.xv is not None, self._lr)
-        graphs = self.__dict__.setdefault("_fit_graphs", {})
-        ent = graphs.get(key)
+        ent = self.__dict__.get("_fit_graphs", {}).get(key)
         if ent is None:
-            self._hedge_fit(e)
-            graphs[key] = "warm"
+            self._hedge_fit(e)   # may grow a workspace, which drops every graph captured so far (_buf)
+            self.__dict__.setdefault("_fit_graphs", {})[key] = "warm"
             return
         if ent == "warm":
             se = EncodedBatch(torch.empty_like(e.ids), None if e.xv is None else torch.empty_like(e.xv), torch.empty_like(e.y))
@@ -657,7 +662,7 @@ class _DeepBase(nn.Module):
             torch.cuda.synchronize()
             with torch.cuda.graph(g):
                 self._hedge_fit(se)
-            ent = graphs[key] = (g, se)
+            ent = self._fit_graphs[key] = (g, se)
         g, se = ent
         se.ids.copy_(e.ids, non_blocking=True)
         if se.xv is not None:
