@@ -111,6 +111,8 @@ _SIGS = {
     "fmb_shard_sort_fields_pf": (C.c_int, [vp, C.c_int, C.c_int, C.c_int, C.c_int, vp, C.c_int, vp, vp, vp, vp, vp, vp, vp]),
     "fmb_shard3_step": (C.c_int, [vp, vp, vp, vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_float,
                                   C.c_int, vp, C.c_size_t, vp, vp, vp, vp, vp, vp, vp, vp, vp]),
+    "fmb_shard3_step_ex": (C.c_int, [vp, vp, vp, vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
+                                     C.c_float, C.c_int, vp, vp, C.c_size_t, vp, vp, vp, vp, vp, vp, vp, vp, vp]),
     "fmb_shard3_bump": (C.c_int, [vp, vp]),
     "fmb_shard_signal": (C.c_int, [vp, vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, vp, vp]),
     "fmb_online_deep_run": (C.c_int, [C.c_int, vp, vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, vp, vp, vp, vp,

@@ -49,6 +49,16 @@ struct Step3Params {
     int* error;                  // 16 + phase on a time-out, 32 on a tile's entry-capacity overflow
     long long* tdbg;             // debug only: per-tile phase timestamps [T][8] (globaltimer ns), else NULL
 };
+// update modes 3 and 4: the same parameters followed by the rule's state (the table's sums, or its moments and the step's
+// scalars by value).  A type of its own, so that the mode 0/1 kernels keep their parameter block as it is.
+struct Step3StateParams : Step3Params {
+    union {
+        fmb::AdagradState ada;       // SK == 3: sums [R_local + 1][rowp], at the local table's offsets
+        fmb::SparseAdamState sa;     // SK == 4: m and v sub-rows [R_local + 1][2][rowp]
+    };
+};
+template <int SK> struct Step3Args { using type = Step3StateParams; };
+template <> struct Step3Args<0> { using type = Step3Params; };
 
 __device__ __forceinline__ void cp_async16(void* smem, const void* gmem) {
     unsigned s = (unsigned)__cvta_generic_to_shared(smem);
@@ -67,8 +77,9 @@ __device__ __forceinline__ bool wait_flag(const uint32_t* f, uint32_t e) {
     return false;
 }
 
-template <int CU>
-__global__ void __launch_bounds__(256, 7) shard_step_fused_kernel(Step3Params p) {
+// SK: state kind of the update rule -- 0 none (modes 0 and 1: p.mode picks), 3 Adagrad, 4 SparseAdam
+template <int CU, int SK>
+__global__ void __launch_bounds__(256, 7) shard_step_fused_kernel(const typename Step3Args<SK>::type p) {
     extern __shared__ __align__(16) float smem[];
     const int F = p.F, k = p.k, SB = p.SB, kp4 = p.kp4, PW = p.PW, CW = p.CW, cap = p.cap_e;
     constexpr int rp = CU * 4;
@@ -269,12 +280,54 @@ __global__ void __launch_bounds__(256, 7) shard_step_fused_kernel(Step3Params p)
         const int idx = list_s[li];
         const int s = ent_s[idx] >> 8;
         const float d = ctx_s[s * CW + kp4];
-        if (d == 0.0f) continue;       // exact: every gradient is +0 and both update rules return p (fm_step.cu, phase 4a)
+        // exact: every gradient is +0, and the fresh-Adam, SGD and Adagrad rules return p (and s) as they are (fm_step.cu,
+        // phase 4a).  SparseAdam steps every row hit, a zero gradient too (m and v decay, p moves by m').
+        if (SK != 4 && d == 0.0f) continue;
         const float4 v4 = *reinterpret_cast<const float4*>(rows_s + (size_t)idx * rp + q * 4);
         float4 S4 = make_float4(0.f, 0.f, 0.f, 0.f);
         if (q * 4 < kp4) S4 = *reinterpret_cast<const float4*>(ctx_s + s * CW + q * 4);
         const float Sq[4] = {S4.x, S4.y, S4.z, S4.w};
         const float v[4] = {v4.x, v4.y, v4.z, v4.w};
+        if constexpr (SK == 3) {
+            // Adagrad: the row's sums, read here at the local table's offsets (8(k+1) more bytes per entry).  Written back
+            // whether p moved or not: the sums move whenever g != 0.  Padding lanes are written as read.
+            float* trow = p.table + (size_t)lrow_s[idx] * p.rowp + q * 4;
+            float* srow = p.ada.sums + (size_t)lrow_s[idx] * p.rowp + q * 4;
+            const float4 s4 = *reinterpret_cast<const float4*>(srow);
+            float sv[4] = {s4.x, s4.y, s4.z, s4.w}, o[4];
+#pragma unroll
+            for (int u = 0; u < 4; ++u) {
+                const int jj = q * 4 + u;
+                o[u] = v[u];
+                if (jj <= k) {
+                    const float a = jj < k ? __fsub_rn(__fmul_rn(d, Sq[u]), __fmul_rn(d, v[u])) : d;
+                    o[u] = fmb::adagrad_update(v[u], __fadd_rn(0.f, a), sv[u], p.lr, p.ada.eps);
+                }
+            }
+            *reinterpret_cast<float4*>(trow) = make_float4(o[0], o[1], o[2], o[3]);
+            *reinterpret_cast<float4*>(srow) = make_float4(sv[0], sv[1], sv[2], sv[3]);
+            continue;
+        }
+        if constexpr (SK == 4) {
+            // SparseAdam: the row's m and v sub-rows in the [R_local + 1][2][rowp] layout (16(k+1) more bytes per entry)
+            float* trow = p.table + (size_t)lrow_s[idx] * p.rowp + q * 4;
+            float* mrow = p.sa.mv + (size_t)lrow_s[idx] * 2 * p.rowp + q * 4;
+            const float4 m4 = *reinterpret_cast<const float4*>(mrow), w4 = *reinterpret_cast<const float4*>(mrow + p.rowp);
+            float mv[4] = {m4.x, m4.y, m4.z, m4.w}, vv[4] = {w4.x, w4.y, w4.z, w4.w}, o[4];
+#pragma unroll
+            for (int u = 0; u < 4; ++u) {
+                const int jj = q * 4 + u;
+                o[u] = v[u];
+                if (jj <= k) {
+                    const float a = jj < k ? __fsub_rn(__fmul_rn(d, Sq[u]), __fmul_rn(d, v[u])) : d;
+                    o[u] = fmb::sparse_adam_update(v[u], __fadd_rn(0.f, a), mv[u], vv[u], p.sa);
+                }
+            }
+            *reinterpret_cast<float4*>(trow) = make_float4(o[0], o[1], o[2], o[3]);
+            *reinterpret_cast<float4*>(mrow) = make_float4(mv[0], mv[1], mv[2], mv[3]);
+            *reinterpret_cast<float4*>(mrow + p.rowp) = make_float4(vv[0], vv[1], vv[2], vv[3]);
+            continue;
+        }
         float o4[4];
         bool moved = false;
 #pragma unroll
@@ -314,6 +367,19 @@ __global__ void __launch_bounds__(256, 7) shard_step_fused_kernel(Step3Params p)
 __global__ void shard3_bump_kernel(uint32_t* epoch) { *epoch += 1u; }
 
 static long long* g_s3_tdbg = nullptr;
+
+template <int SK, typename P>
+static void launch_step3(const P& p, size_t smem, cudaStream_t stream) {
+    void (*fn)(P) = nullptr;
+    switch (p.cu) {
+        case 1: fn = shard_step_fused_kernel<1, SK>; break;
+        case 2: fn = shard_step_fused_kernel<2, SK>; break;
+        case 3: fn = shard_step_fused_kernel<3, SK>; break;
+        default: fn = shard_step_fused_kernel<4, SK>; break;
+    }
+    if (smem > 48 * 1024) cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+    fn<<<p.T, 256, smem, stream>>>(p);
+}
 static int ilog2_exact3(int x) { int l = 0; while ((1 << l) < x) ++l; return (1 << l) == x ? l : -1; }
 static int ilog2_ceil3(int x) { int l = 0; while ((1 << l) < x) ++l; return l; }
 static int64_t npad3(int64_t N) { return (N + 3) / 4 * 4 + 64; }   // == bwd_npad (fm_backward.cu)
@@ -321,6 +387,7 @@ static int64_t npad3(int64_t N) { return (N + 3) / 4 * 4 + 64; }   // == bwd_npa
 }  // namespace
 
 extern "C" size_t fmb_bwd_workspace_bytes(int64_t, int);
+struct fmb_adagrad_t { float* sums; float* bias_sum; float* mlp_sums; float eps; };   // include/fmb200.h
 // debug hook (not in the public header): per-tile phase timestamps of the fused sharded step
 FMB_API void fmb_debug_set_shard3_timestamps(long long* dev) { g_s3_tdbg = dev; }
 
@@ -339,17 +406,25 @@ FMB_API int fmb_shard3_tiles(int G, int B, int F, int k) {
 //   (handed to fmb_fm_backward_runs_list afterwards).  recv / ctx / tflags: HOST arrays of G device pointers (entry r = where
 //   this device maps rank r's buffer); *_local = my own copies; epoch_dev: uint32 step counter in ordinary device memory
 //   (fmb_shard3_bump increments it behind the step); error_dev: see Step3Params.
-FMB_API int fmb_shard3_step(const int32_t* idsT_all, float* table_local, const float* bias, const float* y,
-                            const uint32_t* posflag, int G, int me, int B, int F, int k, int cap, int loss_kind, float lr,
-                            int mode, void* ws, size_t ws_bytes, void* const* recv_peers, void* const* ctx_peers,
-                            void* const* tflag_peers, const float* recv_local, const float* ctx_local,
-                            const uint32_t* tflags_local, const uint32_t* epoch_dev, int* error_dev, cudaStream_t stream) {
+//   state: NULL in modes 0 and 1; mode 3 an fmb_adagrad_t whose sums_dev is this rank's [R_local + 1][rowp] shard, mode 4
+//   an fmb_sparse_adam_t whose mv_dev is its [R_local + 1][2][rowp] shard, advanced to this step (fmb_sparse_adam_advance).
+//   The rows hit several times and the bias are stepped behind this kernel by fmb_fm_backward_runs_list and
+//   fmb_finish_step_ex with the same state.
+FMB_API int fmb_shard3_step_ex(const int32_t* idsT_all, float* table_local, const float* bias, const float* y,
+                               const uint32_t* posflag, int G, int me, int B, int F, int k, int cap, int loss_kind, float lr,
+                               int mode, const void* state, void* ws, size_t ws_bytes, void* const* recv_peers,
+                               void* const* ctx_peers, void* const* tflag_peers, const float* recv_local,
+                               const float* ctx_local, const uint32_t* tflags_local, const uint32_t* epoch_dev, int* error_dev,
+                               cudaStream_t stream) {
     FMB_CHECK_ARG(idsT_all && table_local && bias && y && posflag && ws && recv_peers && ctx_peers && tflag_peers && recv_local &&
                   ctx_local && tflags_local && epoch_dev && error_dev, "fmb_shard3_step: null pointer");
     const int T = fmb_shard3_tiles(G, B, F, k);
     FMB_CHECK_ARG(T > 0 && me >= 0 && me < G && cap > 0, "fmb_shard3_step: unsupported shape G=%d B=%d F=%d k=%d", G, B, F, k);
-    FMB_CHECK_ARG(mode != 4, "fmb_shard3_step: update mode 4 (SparseAdam) is not supported by the sharded step");
-    FMB_CHECK_ARG(mode == 0 || mode == 1, "fmb_shard3_step: unknown update mode %d", mode);
+    FMB_CHECK_ARG(mode != 3 || (state && static_cast<const fmb_adagrad_t*>(state)->sums),
+                  "fmb_shard3_step: update mode 3 (Adagrad) needs the Adagrad state");
+    FMB_CHECK_ARG(mode != 4 || (state && static_cast<const fmb_sparse_adam_t*>(state)->mv),
+                  "fmb_shard3_step: update mode 4 (SparseAdam) needs the SparseAdam state");
+    FMB_CHECK_ARG(mode >= 0 && mode <= 4 && mode != 2, "fmb_shard3_step: unknown update mode %d", mode);
     const int64_t N = (int64_t)F * cap;
     if (ws_bytes < fmb_bwd_workspace_bytes(N, k)) { fmb_set_error("fmb_shard3_step: workspace too small"); return FMB_ERR_WS; }
     Step3Params p;
@@ -390,17 +465,33 @@ FMB_API int fmb_shard3_step(const int32_t* idsT_all, float* table_local, const f
     p.tdbg = g_s3_tdbg;
     const size_t smem = smem_of(p.cap_e);
     FMB_CHECK_ARG(smem <= 200 * 1024, "fmb_shard3_step: tile too large for shared memory");
-    void (*fn)(Step3Params) = nullptr;
-    switch (p.cu) {
-        case 1: fn = shard_step_fused_kernel<1>; break;
-        case 2: fn = shard_step_fused_kernel<2>; break;
-        case 3: fn = shard_step_fused_kernel<3>; break;
-        default: fn = shard_step_fused_kernel<4>; break;
+    if (mode == 3 || mode == 4) {
+        Step3StateParams ps;
+        memset(&ps, 0, sizeof(ps));
+        static_cast<Step3Params&>(ps) = p;
+        if (mode == 3) {
+            const fmb_adagrad_t* a = static_cast<const fmb_adagrad_t*>(state);
+            ps.ada.sums = a->sums; ps.ada.bias_sum = a->bias_sum; ps.ada.eps = a->eps;
+            launch_step3<3>(ps, smem, stream);
+        } else {
+            ps.sa = fmb_sa_tables(static_cast<const fmb_sparse_adam_t*>(state));
+            launch_step3<4>(ps, smem, stream);
+        }
+    } else {
+        launch_step3<0>(p, smem, stream);
     }
-    if (smem > 48 * 1024) cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-    fn<<<T, 256, smem, stream>>>(p);
     FMB_CHECK_LAUNCH("shard_step_fused_kernel");
     return FMB_OK;
+}
+
+FMB_API int fmb_shard3_step(const int32_t* idsT_all, float* table_local, const float* bias, const float* y,
+                            const uint32_t* posflag, int G, int me, int B, int F, int k, int cap, int loss_kind, float lr,
+                            int mode, void* ws, size_t ws_bytes, void* const* recv_peers, void* const* ctx_peers,
+                            void* const* tflag_peers, const float* recv_local, const float* ctx_local,
+                            const uint32_t* tflags_local, const uint32_t* epoch_dev, int* error_dev, cudaStream_t stream) {
+    return fmb_shard3_step_ex(idsT_all, table_local, bias, y, posflag, G, me, B, F, k, cap, loss_kind, lr, mode, nullptr, ws,
+                              ws_bytes, recv_peers, ctx_peers, tflag_peers, recv_local, ctx_local, tflags_local, epoch_dev,
+                              error_dev, stream);
 }
 
 // the step counter of fmb_shard3_step: +1, on the stream, behind the step

@@ -20,7 +20,8 @@ import torch
 import torch.distributed as dist
 
 from . import _lib
-from ._lib import RunList, check, ptr
+from ._lib import AdagradState, RunList, SparseAdamState, check, ptr
+from .deep import UPDATE_ADAGRAD, UPDATE_SPARSE_ADAM
 
 INT_MAX = 0x7FFFFFFF
 _USE_RUNLIST = os.environ.get("FMB_SHARD_RL", "1") != "0"   # experiment knob: 0 = one warp per 32 sorted positions (round 1)
@@ -100,6 +101,8 @@ class ShardedFM:
         self._slot = 0                     # pipelined mode: which buffer set holds the current batch
         self.launches = 0
         self.overflow = torch.zeros(1, dtype=torch.int32, device=self.device)
+        self._ada = None                   # update mode 3's state (enable_adagrad)
+        self._sa = None                    # update mode 4's state (enable_sparse_adam)
 
     # ---------------------------------------------------------------- parameters (tests)
     def load_full(self, V, w1, bias):
@@ -114,6 +117,79 @@ class ShardedFM:
     def local_params(self):
         t = self.table[:self.R_local].cpu().numpy()
         return t[:, :self.k].copy(), t[:, self.k].copy()
+
+    # ---------------------------------------------------------------- update modes 3 and 4 (state kept across steps)
+    # Row r's state lives beside row r: on rank r % G at local row r // G, in a table with the local table's shape (Adagrad)
+    # or FTRL's [rows][2][rowp] layout (SparseAdam).  Only the owner updates a row, so the state never crosses a link.  The
+    # bias is replicated and every rank runs the same bias step over the global batch, so its state is replicated too.
+    def enable_adagrad(self, eps=1e-10, initial_accumulator_value=0.0):
+        """Switch the step to torch.optim.Adagrad(lr=n, eps=eps, initial_accumulator_value=...) kept across steps: the
+        trajectory of ONE such optimizer over the full tables stepped on the global batch.  Every rank calls it.  Calling it
+        again resets the sums; captured step graphs are dropped (they hold the previous sums' addresses)."""
+        v = float(np.float32(initial_accumulator_value))
+        if v < 0:
+            raise ValueError("initial_accumulator_value must be >= 0")
+        self.update_mode = UPDATE_ADAGRAD
+        self._ada_eps = float(np.float32(eps))
+        self._ada_sums = torch.full((self.R_local + 1, self.rowp), v, dtype=torch.float32, device=self.device)
+        self._ada_bias = torch.full((1,), v, dtype=torch.float32, device=self.device)
+        self._ada = AdagradState(self._ada_sums.data_ptr(), self._ada_bias.data_ptr(), None, self._ada_eps)
+        self._drop_graphs()
+
+    def enable_sparse_adam(self, betas=(0.9, 0.999), eps=1e-8):
+        """Switch the step to torch.optim.SparseAdam(<tables>, lr=n, betas, eps) on the rows each global batch hits and
+        torch.optim.Adam([bias], lr=n, betas, eps), both kept across steps.  Every row hit steps, also with a zero
+        gradient.  Every rank calls it and counts every step.  Calling it again resets the moments and the counter;
+        captured step graphs are dropped, and the step cannot be captured in this mode (a replay would repeat the
+        captured step's bias corrections)."""
+        b1, b2 = (float(b) for b in betas)
+        if not (0.0 <= b1 < 1.0 and 0.0 <= b2 < 1.0) or eps < 0:
+            raise ValueError("need 0 <= beta1, beta2 < 1 and eps >= 0")
+        self.update_mode = UPDATE_SPARSE_ADAM
+        self._sa_mv = torch.zeros((self.R_local + 1, 2, self.rowp), dtype=torch.float32, device=self.device)
+        self._sa_bias = torch.zeros((2,), dtype=torch.float32, device=self.device)
+        self._sa = SparseAdamState(self._sa_mv.data_ptr(), self._sa_bias.data_ptr(), None, b1, b2, float(np.float32(eps)),
+                                   0, 0)
+        self._drop_graphs()
+
+    def local_state(self):
+        """this rank's shard of the update rule's state, in local-row order, and the (replicated) bias state:
+        mode 3 (sums_V [R_local, k], sums_w1 [R_local], bias_sum [1]);
+        mode 4 (m_V, v_V [R_local, k], m_w1, v_w1 [R_local], bias_m, bias_v [1], steps taken)."""
+        k, n = self.k, self.R_local
+        if self.update_mode == UPDATE_ADAGRAD and self._ada is not None:
+            s = self._ada_sums[:n].cpu().numpy()
+            return s[:, :k].copy(), s[:, k].copy(), self._ada_bias.cpu().numpy().copy()
+        if self.update_mode == UPDATE_SPARSE_ADAM and self._sa is not None:
+            mv = self._sa_mv[:n].cpu().numpy()
+            b = self._sa_bias.cpu().numpy()
+            return (mv[:, 0, :k].copy(), mv[:, 1, :k].copy(), mv[:, 0, k].copy(), mv[:, 1, k].copy(), b[:1].copy(),
+                    b[1:].copy(), int(self._sa.step))
+        raise RuntimeError(f"update mode {self.update_mode} keeps no state (enable_adagrad / enable_sparse_adam)")
+
+    def _state_arg(self):
+        """the state slot of the C entry points: fmb_adagrad_t in mode 3, fmb_sparse_adam_t in mode 4, else NULL (a mode
+        3 or 4 step without its state is refused by the library, naming the mode, before any kernel runs)"""
+        if self.update_mode == UPDATE_ADAGRAD and self._ada is not None:
+            return C.byref(self._ada)
+        if self.update_mode == UPDATE_SPARSE_ADAM and self._sa is not None:
+            return C.byref(self._sa)
+        return None
+
+    def _advance(self):
+        """mode 4: one more step on this rank's counter when the step is submitted (the scalars go by value into the
+        launches), so that every rank has the same scalars and host pipelining stays exact"""
+        if self.update_mode == UPDATE_SPARSE_ADAM and self._sa is not None:
+            check(self._lib.fmb_sparse_adam_advance(C.byref(self._sa), self.lr, 0), "fmb_sparse_adam_advance")
+
+    def _drop_graphs(self):
+        for name in ("_graph", "_g_loss", "_pgraphs", "_pg_loss"):
+            self.__dict__.pop(name, None)
+
+    def _refuse_capture(self):
+        if self.update_mode == UPDATE_SPARSE_ADAM:
+            raise RuntimeError("update mode 4 (SparseAdam) cannot be captured into a step graph: a replay would repeat the "
+                               "captured step's bias corrections; run the step eagerly")
 
     # ---------------------------------------------------------------- the step
     def _buf(self, name, shape, dtype=torch.float32):
@@ -201,6 +277,8 @@ class ShardedFM:
         Btot = ctx_all.shape[0]
         N = F * cap
         main = torch.cuda.current_stream()
+        self._advance()
+        state = self._state_arg()
         if join_sort:
             main.wait_stream(self._side)  # sorted keys / permutation are ready (phase_owner_forward put them there)
         wsb = lib.fmb_bwd_workspace_bytes(N, k)
@@ -214,13 +292,13 @@ class ShardedFM:
         with torch.cuda.stream(self._side):
             check(lib.fmb_shard_unpack_ctx(ptr(ctx_all), Btot, k, ptr(delta_all), ptr(lossv_all), _stream()),
                   "fmb_shard_unpack_ctx")
-            check(lib.fmb_finish_step(ptr(delta_all), ptr(lossv_all), Btot, ptr(self.bias), self.lr,
-                                      self.update_mode, ptr(loss), _stream()), "fmb_finish_step")
+            check(lib.fmb_finish_step_ex(ptr(delta_all), ptr(lossv_all), Btot, ptr(self.bias), self.lr,
+                                         self.update_mode, state, ptr(loss), _stream()), "fmb_finish_step")
         self.launches += 9
         rl = C.byref(self._rl[slot]) if (_USE_RUNLIST and slot in self._rl) else None
-        check(lib.fmb_fm_backward_update_rl(ptr(self._ws[f"skeys{slot}"]), ptr(self._ws[f"perm{slot}"]), N, Btot * F, None,
-                                            ptr(self.table), F, k, ptr(ctx_all), self.CW, ptr(gs), self.CW, 1, None,
-                                            INT_MAX, self.lr, self.update_mode, rl, ptr(ws), wsb, st),
+        check(lib.fmb_fm_backward_update_rl_ex(ptr(self._ws[f"skeys{slot}"]), ptr(self._ws[f"perm{slot}"]), N, Btot * F,
+                                               None, ptr(self.table), F, k, ptr(ctx_all), self.CW, ptr(gs), self.CW, 1, None,
+                                               INT_MAX, self.lr, self.update_mode, state, rl, ptr(ws), wsb, st),
               "fmb_fm_backward_update_rl")
         main.wait_stream(self._side)      # join: the step is complete when both branches are
         return loss
@@ -438,10 +516,11 @@ class ShardedFM:
         wsb = lib.fmb_bwd_workspace_bytes(F * cap, k)
         ws = self._buf("bwd_ws", (wsb,), torch.uint8)
         ep = C.c_void_p(pr["epoch"].data_ptr() + 4 * self.CH_TILE)
-        check(lib.fmb_shard3_step(ptr(pr["ids"][p]), ptr(self.table), ptr(self.bias), ptr(y), ptr(pr["posflag"][p]), G,
-                                  self.rank, B, F, k, cap, loss_kind, self.lr, self.update_mode, ptr(ws), wsb,
-                                  pr["ptrs"]["recv"], pr["ptrs"]["ctx"], pr["ptrs"]["tflags"], ptr(pr["recv"]), ptr(pr["ctx"]),
-                                  ptr(pr["tflags"]), ep, ptr(pr["error"]), _stream()), "fmb_shard3_step")
+        self._advance()   # _fused_finish steps the multi-hit rows and the bias with the same scalars
+        check(lib.fmb_shard3_step_ex(ptr(pr["ids"][p]), ptr(self.table), ptr(self.bias), ptr(y), ptr(pr["posflag"][p]), G,
+                                     self.rank, B, F, k, cap, loss_kind, self.lr, self.update_mode, self._state_arg(), ptr(ws),
+                                     wsb, pr["ptrs"]["recv"], pr["ptrs"]["ctx"], pr["ptrs"]["tflags"], ptr(pr["recv"]),
+                                     ptr(pr["ctx"]), ptr(pr["tflags"]), ep, ptr(pr["error"]), _stream()), "fmb_shard3_step")
         check(lib.fmb_shard3_bump(ep, _stream()), "fmb_shard3_bump")
         return ws, wsb
 
@@ -453,15 +532,16 @@ class ShardedFM:
         delta_all = self._buf("delta_all", (Btot,))
         lossv_all = self._buf("lossv_all", (Btot,))
         loss = torch.empty((), device=self.device)
+        state = self._state_arg()
         self._side.wait_stream(main)
         with torch.cuda.stream(self._side):
             check(lib.fmb_shard_unpack_ctx(ptr(pr["ctx"]), Btot, k, ptr(delta_all), ptr(lossv_all), _stream()),
                   "fmb_shard_unpack_ctx")
-            check(lib.fmb_finish_step(ptr(delta_all), ptr(lossv_all), Btot, ptr(self.bias), self.lr,
-                                      self.update_mode, ptr(loss), _stream()), "fmb_finish_step")
+            check(lib.fmb_finish_step_ex(ptr(delta_all), ptr(lossv_all), Btot, ptr(self.bias), self.lr,
+                                         self.update_mode, state, ptr(loss), _stream()), "fmb_finish_step")
         rl = C.byref(self._rl[p]) if (_USE_RUNLIST and p in self._rl) else None
         check(lib.fmb_fm_backward_runs_list(ptr(self._ws[f"skeys{p}"]), F * cap, ptr(self.table), F, k, self.lr,
-                                            self.update_mode, None, rl, ptr(ws), wsb, _stream()),
+                                            self.update_mode, state, rl, ptr(ws), wsb, _stream()),
               "fmb_fm_backward_runs_list")
         self.launches += 6
         main.wait_stream(self._side)
@@ -484,6 +564,7 @@ class ShardedFM:
 
     def capture_fused(self, ids, y, loss_kind=0):
         """capture_peers for the fused step"""
+        self._refuse_capture()
         self._g_ids = ids.clone()
         self._g_y = y.clone()
         side = torch.cuda.Stream()
@@ -519,6 +600,7 @@ class ShardedFM:
 
     def capture_peers(self, ids, y, loss_kind=0):
         """capture_pipelined for the peer-memory step (no collective inside the graphs)."""
+        self._refuse_capture()
         self._g_ids = ids.clone()
         self._g_y = y.clone()
         side = torch.cuda.Stream()
@@ -547,6 +629,7 @@ class ShardedFM:
     def capture(self, ids, y, loss_kind=0):
         """Capture one step (kernels + the three NCCL collectives) into a CUDA graph over static input
         buffers.  `ids`/`y` seed the buffers; two eager warm-up steps run first (they do train)."""
+        self._refuse_capture()
         self._g_ids = ids.clone()
         self._g_y = y.clone()
         side = torch.cuda.Stream()
@@ -575,6 +658,7 @@ class ShardedFM:
     def capture_pipelined(self, ids, y, loss_kind=0):
         """Capture the pipelined step for both buffer-set parities.  `ids`/`y` seed the static buffers; two eager
         warm-up steps run first (they do train).  Afterwards call prepare(first ids), then step_graphed_pipelined."""
+        self._refuse_capture()
         self._g_ids = ids.clone()
         self._g_y = y.clone()
         side = torch.cuda.Stream()

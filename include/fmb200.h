@@ -196,7 +196,8 @@ typedef struct fmb_ftrl_t { float* zn_dev; float* bias_zn_dev; float beta, l1, l
  * bias_sum_dev [1]; mlp_sums_dev [fmb_mlp_numel] (tower fit and fmb_online_deep_run_ex, NULL for FM-only steps).
  * Entry points with a state slot (fmb_fm_step_fused_ex, fmb_fm_backward_runs_ex / _list, fmb_finish_step_ex) take it
  * there in mode 3: pass (const fmb_ftrl_t*)&adagrad.  Algorithmic bytes of the FM step grow by 8F(k+1) per sample.
- * Sharded steps, AFM and fmb_fm_backward_runs_all reject mode 3. */
+ * The row-sharded steps take each rank's shard of the sums (fmb_shard3_step_ex); the shard2 path, AFM and
+ * fmb_fm_backward_runs_all reject mode 3. */
 typedef struct fmb_adagrad_t { float* sums_dev; float* bias_sum_dev; float* mlp_sums_dev; float eps; } fmb_adagrad_t;
 /* update mode 4: torch.optim.SparseAdam(betas, eps, lr = the step's lr) on the embedding tables -- only the rows a batch
  * hits update their moments and weights, a zero gradient of such a row included -- and torch.optim.Adam(betas, eps) on the
@@ -210,7 +211,8 @@ typedef struct fmb_adagrad_t { float* sums_dev; float* bias_sum_dev; float* mlp_
  * bias_mv_dev [2]; mlp_mv_dev [2][fmb_mlp_numel] (m, then v) or NULL.  Zero-fill the moments and counters to start.
  * The entry points with a state slot take it there (pass (const fmb_ftrl_t*)&sa), advanced to the step being run by
  * fmb_sparse_adam_advance; a session step advances it itself (fmb_session_set_sparse_adam).  Algorithmic bytes of the FM
- * step grow by 16F(k+1) per sample.  Sharded steps, AFM and fmb_fm_backward_runs_all reject mode 4. */
+ * step grow by 16F(k+1) per sample.  The row-sharded steps take each rank's shard of the moments (fmb_shard3_step_ex);
+ * the shard2 path, AFM and fmb_fm_backward_runs_all reject mode 4. */
 typedef struct fmb_adam_step_t { float emb_step, bias_step, bias_bc2s, mlp_step, mlp_bc2s; } fmb_adam_step_t;
 typedef struct fmb_sparse_adam_t {
     float* mv_dev; float* bias_mv_dev; float* mlp_mv_dev;
@@ -392,6 +394,17 @@ int fmb_shard3_step(const int32_t* idsT_all_dev, float* table_local_dev, const f
                     void* ws_dev, size_t ws_bytes, void* const* recv_peers, void* const* ctx_peers, void* const* tflag_peers,
                     const float* recv_local_dev, const float* ctx_local_dev, const uint32_t* tflags_local_dev,
                     const uint32_t* epoch_dev, int* error_dev, fmb_stream_t stream);
+/* _ex: with the update rule's state (NULL in modes 0 and 1).  Mode 3: an fmb_adagrad_t whose sums_dev is this rank's
+ * [R_local + 1][rowp] shard (local row r / G of row r, the local table's layout) and bias_sum_dev the replicated [1];
+ * mode 4: an fmb_sparse_adam_t whose mv_dev is this rank's [R_local + 1][2][rowp] shard and bias_mv_dev the replicated
+ * [2], advanced to this step by fmb_sparse_adam_advance (once per step on every rank).  Pass the same state to the
+ * fmb_fm_backward_runs_list and fmb_finish_step_ex calls that follow.  Mode 3 or 4 without its state is refused. */
+int fmb_shard3_step_ex(const int32_t* idsT_all_dev, float* table_local_dev, const float* bias_dev, const float* y_dev,
+                       const uint32_t* posflag_dev, int G, int me, int B, int F, int k, int cap, int loss_kind, float lr,
+                       int mode, const void* state, void* ws_dev, size_t ws_bytes, void* const* recv_peers,
+                       void* const* ctx_peers, void* const* tflag_peers, const float* recv_local_dev,
+                       const float* ctx_local_dev, const uint32_t* tflags_local_dev, const uint32_t* epoch_dev,
+                       int* error_dev, fmb_stream_t stream);
 int fmb_shard3_bump(uint32_t* epoch_dev, fmb_stream_t stream);
 
 /* ---- A4/A5: MLP tower on the Bi-Interaction vector (deepfm_adam.py:79-89, nfm_adam.py:78-88,
